@@ -490,6 +490,32 @@ def mutate_batch(ctx, pkg, ell, pre, post, proofs, proof_size, first_index, ever
     return pre_m, post_m, proofs_m, want_ok, want_st
 
 
+DUMP_SAMPLE = 256  # instances whose post-trackers and proofs are written: about 17 MB as float32 at n = 128
+
+
+def dump_outputs(out_dir: str, B: int, post, proofs, status, ok, st, ell: int = ELL, proof_size: int = 4576):
+    """What the round trips of one step return to their caller, as float32 .npy files, so that two builds
+    can be compared output for output: post-trackers and proofs (one byte per element) of a fixed, seeded
+    sample of the batch, the sampled indices, and every instance's generation status, verdict and
+    validation status."""
+    import numpy as np
+
+    idx = np.arange(B)
+    if B > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_SAMPLE, replace=False))
+    arrays = {
+        "sample_index": idx,
+        "post_trackers": np.frombuffer(post, np.uint8).reshape(B, ell * 96)[idx],
+        "proofs": np.frombuffer(proofs, np.uint8).reshape(B, proof_size)[idx],
+        "generate_status": status,
+        "valid": ok,
+        "validate_status": st,
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
+
+
 def gpu_main(args):
     import torch
     import torch.distributed as dist
@@ -541,10 +567,10 @@ def gpu_main(args):
         rands = all_rands[s]
         post, proofs, status = ctx.whisk_generate_shuffle_proof_batch(crs, pre, rands)
         ok, st = ctx.whisk_is_valid_shuffle_proof_batch(crs, pre, post, proofs, rands)
-        return status, ok, st
+        return post, proofs, status, ok, st
 
     for _ in range(args.warmup):
-        status, ok, st = step()
+        _, _, status, ok, st = step()
         assert status == [0] * B and ok == [1] * B and st == [0] * B, "warm-up round trip failed"
 
     def barrier():
@@ -565,7 +591,7 @@ def gpu_main(args):
     barrier()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        status, ok, st = step()
+        post, proofs, status, ok, st = step()
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
     barrier()
@@ -576,6 +602,8 @@ def gpu_main(args):
     launches = ctx.launch_count() - l0
     busy_ms = ctx.engine_busy_ms()
     wall_max, dev_max = max_over_ranks(wall), max_over_ranks(busy_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, B, post, proofs, status, ok, st)
 
     # roofline pass: the same step with ONE lane, so that the CUDA-event interval of a kernel is its own
     # duration (with several lanes the streams share the GPU and every interval also contains the other
@@ -583,7 +611,7 @@ def gpu_main(args):
     ctx.set_lanes(1)
     step()
     ctx.engine_stats(reset=True)
-    status, ok, st = step()
+    _, _, status, ok, st = step()
     torch.cuda.synchronize()
     assert status == [0] * B and ok == [1] * B and st == [0] * B, "roofline-pass round trip failed"
     stats = ctx.engine_stats()
@@ -798,7 +826,13 @@ def main():
     ap.add_argument("--no-config4", action="store_true", help="skip the sharded batched-verification pass")
     ap.add_argument("--no-n512", action="store_true", help="skip the n=512 throughput line")
     ap.add_argument("--msm-sizes", default="", help="comma separated log2 sizes for the MSM sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's post-trackers, proofs and verdicts (rank 0's batch) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.lanes < 0:
         world_ = max(1, int(os.environ.get("WORLD_SIZE", "1")))
         args.lanes = 6 if (os.cpu_count() or 1) // world_ >= 8 else 8
