@@ -10,21 +10,25 @@
 
 #include "../../include/curdle_b200.h"
 #include "context.cuh"
+#include "host/engine.hpp"
 #include "launch.h"
 
 using namespace cdl;
-
-namespace cdl {
-static __global__ void k_iota(uint32_t* out, uint32_t n) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = i;
-}
-}  // namespace cdl
 
 static_assert(sizeof(Fp) == sizeof(cdl_fp), "fp layout");
 static_assert(sizeof(Fr) == sizeof(cdl_fr), "fr layout");
 static_assert(sizeof(G1Affine) == sizeof(cdl_g1_affine), "affine layout");
 static_assert(sizeof(G1Jac) == sizeof(cdl_g1_jac), "jac layout");
+
+// the MSM stage's tasks for offsets[0..k], result j to pool slot j; false when the offsets are not monotone
+static bool msm_tasks(const uint32_t* offsets, size_t k, std::vector<MsmTask>& tasks) {
+  tasks.resize(k);
+  for (size_t j = 0; j < k; j++) {
+    if (offsets[j + 1] < offsets[j]) return false;
+    tasks[j] = MsmTask{offsets[j], offsets[j + 1] - offsets[j], (uint32_t)j, 0};
+  }
+  return true;
+}
 
 extern "C" {
 
@@ -117,54 +121,29 @@ int32_t cdl_device_info(cdl_ctx* c, int32_t* sm_count, int32_t* clock_khz, char*
 }
 
 // --------------------------------------------------------------------- MSM
+// The batched MSMs run as one MSM stage of the context's engine (Engine::run_msm picks the kernels and
+// the chunking); MSM j of a call writes its result to engine-pool slot j.
 int32_t cdl_g1_msm_batch(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars,
                          const uint32_t* offsets, size_t k, cdl_g1_affine* out) {
   if (!c || !offsets || !out || (k && offsets[k] && (!points || !scalars))) return CDL_ERR_INVALID_ARG;
   if (k == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
+  const size_t total = offsets[k];
+  cdlh::MsmStage st;
+  if (!msm_tasks(offsets, k, st.tasks)) return c->fail(CDL_ERR_INVALID_ARG, "msm_batch: offsets not monotone");
+  // the bases go to pool slots [k, k + total); pool indices are 30 bits (bit 31 negates, bit 30 is the kernels' flag)
+  if (k + total >= (1u << 30))
+    return c->fail(CDL_ERR_INVALID_ARG, "msm_batch: %zu MSMs of %zu terms exceed the 2^30-point pool", k, total);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  size_t total = offsets[k];
-  size_t max_terms = 0;
-  std::vector<MsmTask> tasks(k);
-  for (size_t j = 0; j < k; j++) {
-    if (offsets[j + 1] < offsets[j]) return c->fail(CDL_ERR_INVALID_ARG, "msm_batch: offsets not monotone");
-    tasks[j].term_off = offsets[j];
-    tasks[j].term_cnt = offsets[j + 1] - offsets[j];
-    tasks[j].out_idx = (uint32_t)j;
-    tasks[j].pad = 0;
-    if (tasks[j].term_cnt > max_terms) max_terms = tasks[j].term_cnt;
-  }
-  G1Affine* d_pts = (G1Affine*)c->buf(0, (total + 1) * sizeof(G1Affine));
-  Fr* d_sc = (Fr*)c->buf(1, (total + 1) * sizeof(Fr));
-  uint32_t* d_idx = (uint32_t*)c->buf(2, (total + 1) * sizeof(uint32_t));
-  MsmTask* d_tasks = (MsmTask*)c->buf(3, k * sizeof(MsmTask));
-  G1Affine* d_out = (G1Affine*)c->buf(4, k * sizeof(G1Affine));
-  if (!d_pts || !d_sc || !d_idx || !d_tasks || !d_out) return c->fail(CDL_ERR_CUDA, "device allocation failed");
-  if (total) {
-    CDL_CUDA(c, cudaMemcpyAsync(d_pts, points, total * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
-    CDL_CUDA(c, cudaMemcpyAsync(d_sc, scalars, total * sizeof(Fr), cudaMemcpyHostToDevice, c->stream));
-    k_iota<<<(unsigned)((total + 255) / 256), 256, 0, c->stream>>>(d_idx, (uint32_t)total);
-  }
-  CDL_CUDA(c, cudaMemcpyAsync(d_tasks, tasks.data(), k * sizeof(MsmTask), cudaMemcpyHostToDevice, c->stream));
-  if ((int)k >= kMsmSplitThreshold || max_terms > kMsmSplitTerms) {
-    std::vector<MsmSub> subs;
-    std::vector<MsmTask2> tasks2;
-    msm_build_subs(tasks.data(), k, msm_tp_pick_chunk(total, c->sm_count), subs, tasks2);
-    MsmSub* d_subs = (MsmSub*)c->buf(5, subs.size() * sizeof(MsmSub));
-    MsmTask2* d_t2 = (MsmTask2*)c->buf(6, tasks2.size() * sizeof(MsmTask2));
-    void* d_scr = c->buf(7, msm_tp_scratch_bytes(total, subs.size(), k));
-    if (!d_subs || !d_t2 || !d_scr) return c->fail(CDL_ERR_CUDA, "device allocation failed");
-    CDL_CUDA(c, cudaMemcpyAsync(d_subs, subs.data(), subs.size() * sizeof(MsmSub), cudaMemcpyHostToDevice, c->stream));
-    CDL_CUDA(c, cudaMemcpyAsync(d_t2, tasks2.data(), tasks2.size() * sizeof(MsmTask2), cudaMemcpyHostToDevice, c->stream));
-    CDL_CUDA(c, cudaStreamSynchronize(c->stream));  // subs/tasks2 are pageable host vectors
-    launch_msm_tp(d_pts, d_idx, d_sc, (int)total, d_subs, (int)subs.size(), d_t2, (int)k, d_out, nullptr, d_scr, c->stream);
-  } else {
-    launch_msm_small(d_pts, d_idx, d_sc, d_tasks, (int)k, max_terms, d_out, nullptr, c->stream);
-  }
-  CDL_CUDA(c, cudaGetLastError());
-  CDL_CUDA(c, cudaMemcpyAsync(out, d_out, k * sizeof(G1Affine), cudaMemcpyDeviceToHost, c->stream));
-  CDL_CUDA(c, cudaStreamSynchronize(c->stream));
-  return CDL_OK;
+  c->spin_wait = true;  // latency regime, as for small protocol batches: see cdl_ctx::sync_stream
+  cdlh::Engine* E = cdlh::engine_of(c);
+  st.idx.resize(total);
+  for (size_t t = 0; t < total; t++) st.idx[t] = (uint32_t)(k + t);
+  st.sc.assign(reinterpret_cast<const cdlh::Fr*>(scalars), reinterpret_cast<const cdlh::Fr*>(scalars) + total);
+  int32_t rc;
+  if ((rc = E->ensure_pool(k + total)) || (rc = E->upload_points((uint32_t)k, points, total)) || (rc = E->run_msm(st)))
+    return rc;
+  return E->download_points(0, out, k);
 }
 
 // Batched MSM over a DEVICE-RESIDENT pool of bases: term t of MSM j is scalars[t] * d_pool[idx[t]]
@@ -180,58 +159,27 @@ int32_t cdl_g1_msm_batch_device(cdl_ctx* c, cdl_g1_affine* d_pool, const uint32_
   if (!c || !d_pool || !offsets || (k && offsets[k] && (!idx || !scalars))) return CDL_ERR_INVALID_ARG;
   if (k == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
-  CDL_CUDA(c, cudaSetDevice(c->device));
   const size_t total = offsets[k];
-  size_t max_terms = 0;
-  std::vector<MsmTask> tasks(k);
-  for (size_t j = 0; j < k; j++) {
-    if (offsets[j + 1] < offsets[j]) return c->fail(CDL_ERR_INVALID_ARG, "msm_batch_device: offsets not monotone");
-    tasks[j].term_off = offsets[j];
-    tasks[j].term_cnt = offsets[j + 1] - offsets[j];
-    tasks[j].out_idx = (uint32_t)j;
-    tasks[j].pad = 0;
-    if (tasks[j].term_cnt > max_terms) max_terms = tasks[j].term_cnt;
-  }
+  cdlh::MsmStage st;
+  if (!msm_tasks(offsets, k, st.tasks)) return c->fail(CDL_ERR_INVALID_ARG, "msm_batch_device: offsets not monotone");
   // pool indices are 30 bits: bit 31 negates, bit 30 is the kernels' own flag
   for (size_t t = 0; t < total; t++)
     if (idx[t] & 0x40000000u) return c->fail(CDL_ERR_INVALID_ARG, "msm_batch_device: pool index of term %zu exceeds 2^30 - 1", t);
-  Fr* d_sc = (Fr*)c->buf(1, (total + 1) * sizeof(Fr));
-  uint32_t* d_idx = (uint32_t*)c->buf(2, (total + 1) * sizeof(uint32_t));
-  MsmTask* d_tasks = (MsmTask*)c->buf(3, k * sizeof(MsmTask));
-  G1Affine* d_out = (G1Affine*)c->buf(4, k * sizeof(G1Affine));
-  uint8_t* d_c48 = (uint8_t*)c->buf(0, k * 48);
-  if (!d_sc || !d_idx || !d_tasks || !d_out || !d_c48) return c->fail(CDL_ERR_CUDA, "device allocation failed");
-  if (total) {
-    CDL_CUDA(c, cudaMemcpyAsync(d_sc, scalars, total * sizeof(Fr), cudaMemcpyHostToDevice, c->stream));
-    CDL_CUDA(c, cudaMemcpyAsync(d_idx, idx, total * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
-  }
-  CDL_CUDA(c, cudaMemcpyAsync(d_tasks, tasks.data(), k * sizeof(MsmTask), cudaMemcpyHostToDevice, c->stream));
-  const G1Affine* pool = reinterpret_cast<const G1Affine*>(d_pool);
-  if ((int)k >= kMsmSplitThreshold || max_terms > kMsmSplitTerms) {
-    std::vector<MsmSub> subs;
-    std::vector<MsmTask2> tasks2;
-    msm_build_subs(tasks.data(), k, msm_tp_pick_chunk(total, c->sm_count), subs, tasks2);
-    MsmSub* d_subs = (MsmSub*)c->buf(5, subs.size() * sizeof(MsmSub));
-    MsmTask2* d_t2 = (MsmTask2*)c->buf(6, tasks2.size() * sizeof(MsmTask2));
-    void* d_scr = c->buf(7, msm_tp_scratch_bytes(total, subs.size(), k));
-    if (!d_subs || !d_t2 || !d_scr) return c->fail(CDL_ERR_CUDA, "device allocation failed");
-    CDL_CUDA(c, cudaMemcpyAsync(d_subs, subs.data(), subs.size() * sizeof(MsmSub), cudaMemcpyHostToDevice, c->stream));
-    CDL_CUDA(c, cudaMemcpyAsync(d_t2, tasks2.data(), tasks2.size() * sizeof(MsmTask2), cudaMemcpyHostToDevice, c->stream));
-    CDL_CUDA(c, cudaStreamSynchronize(c->stream));  // subs/tasks2 are pageable host vectors
-    launch_msm_tp(pool, d_idx, d_sc, (int)total, d_subs, (int)subs.size(), d_t2, (int)k, d_out, d_c48, d_scr, c->stream);
-  } else {
-    if (max_terms > kMsmMaxTerms) return c->fail(CDL_ERR_TOO_LARGE, "msm of %zu terms exceeds the small-MSM limit", max_terms);
-    launch_msm_small(pool, d_idx, d_sc, d_tasks, (int)k, max_terms, d_out, d_c48, c->stream);
-  }
-  CDL_CUDA(c, cudaGetLastError());
+  CDL_CUDA(c, cudaSetDevice(c->device));
+  c->spin_wait = true;  // latency regime, as for small protocol batches: see cdl_ctx::sync_stream
+  cdlh::Engine* E = cdlh::engine_of(c);
+  st.idx.assign(idx, idx + total);
+  st.sc.assign(reinterpret_cast<const cdlh::Fr*>(scalars), reinterpret_cast<const cdlh::Fr*>(scalars) + total);
+  int32_t rc;
+  if ((rc = E->ensure_pool(k)) || (rc = E->run_msm(st, nullptr, reinterpret_cast<const G1Affine*>(d_pool)))) return rc;
+  if (out48) memcpy(out48, st.out48.data(), k * 48);
   if (out_slot) {  // scatter the results into their pool slots (k small copies on the stream)
     for (size_t j = 0; j < k; j++)
-      CDL_CUDA(c, cudaMemcpyAsync(reinterpret_cast<G1Affine*>(d_pool) + out_slot[j], d_out + j, sizeof(G1Affine),
+      CDL_CUDA(c, cudaMemcpyAsync(reinterpret_cast<G1Affine*>(d_pool) + out_slot[j], E->d_pool() + j, sizeof(G1Affine),
                                   cudaMemcpyDeviceToDevice, c->stream));
   }
-  if (out) CDL_CUDA(c, cudaMemcpyAsync(out, d_out, k * sizeof(G1Affine), cudaMemcpyDeviceToHost, c->stream));
-  if (out48) CDL_CUDA(c, cudaMemcpyAsync(out48, d_c48, k * 48, cudaMemcpyDeviceToHost, c->stream));
-  CDL_CUDA(c, cudaStreamSynchronize(c->stream));
+  if (out) return E->download_points(0, out, k);  // its wait covers the scatter
+  CDL_CUDA(c, c->sync_stream());
   return CDL_OK;
 }
 
@@ -246,31 +194,17 @@ int32_t cdl_g1_msm(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalar
   cdl_g1_affine a;
   int32_t rc = cdl_g1_msm_batch(c, points, scalars, offs, 1, &a);
   if (rc != CDL_OK) return rc;
-  // lift to gnark's G1Jac: (x, y, 1) or (1, 1, 0) for infinity
-  bool inf = true;
-  for (int i = 0; i < 6; i++) inf = inf && a.x.l[i] == 0 && a.y.l[i] == 0;
-  static const uint64_t one[6] = {0x760900000002fffdull, 0xebf4000bc40c0002ull, 0x5f48985753c758baull,
-                                  0x77ce585370525745ull, 0x5c071a97a256ec6dull, 0x15f65ec3fa80e493ull};
-  if (inf) {
-    memcpy(out->x.l, one, 48);
-    memcpy(out->y.l, one, 48);
-    memset(out->z.l, 0, 48);
-  } else {
-    out->x = a.x;
-    out->y = a.y;
-    memcpy(out->z.l, one, 48);
-  }
+  cdlh::affine_to_jac(out, a);
   return CDL_OK;
 }
 
 int32_t cdl_g1_sum_affine(cdl_ctx* c, const cdl_g1_affine* in, size_t n, cdl_g1_affine* out) {
   if (!c || !out || (n && !in)) return CDL_ERR_INVALID_ARG;
-  static const uint64_t fr_one[4] = {0x00000001fffffffeull, 0x5884b7fa00034802ull, 0x998c4fefecbc4ff5ull, 0x1824b159acc5056full};
-  std::vector<cdl_fr> ones(n);
-  for (size_t i = 0; i < n; i++) memcpy(ones[i].l, fr_one, 32);
+  const std::vector<cdlh::Fr> one_v(n, cdlh::FR_ONE);
+  const cdl_fr* ones = reinterpret_cast<const cdl_fr*>(one_v.data());
   if (n > kBigMsmThreshold) {
     cdl_g1_jac j;
-    int32_t rc = cdl_g1_msm(c, in, ones.data(), n, &j);
+    int32_t rc = cdl_g1_msm(c, in, ones, n, &j);
     if (rc != CDL_OK) return rc;
     bool inf = true;
     for (int i = 0; i < 6; i++) inf = inf && j.z.l[i] == 0;
@@ -279,7 +213,7 @@ int32_t cdl_g1_sum_affine(cdl_ctx* c, const cdl_g1_affine* in, size_t n, cdl_g1_
     return CDL_OK;
   }
   uint32_t offs[2] = {0, (uint32_t)n};
-  return cdl_g1_msm_batch(c, in, ones.data(), offs, 1, out);
+  return cdl_g1_msm_batch(c, in, ones, offs, 1, out);
 }
 
 // --------------------------------------------------------------------- elementwise

@@ -10,7 +10,9 @@
 
 #include "host/engine.hpp"
 
+using cdlh::affine_to_jac;
 using cdlh::Engine;
+using cdlh::engine_of;
 using cdlh::Fr;
 using cdlh::Layout;
 
@@ -28,14 +30,16 @@ const uint32_t kGenY[12] = {0x0ce72271u, 0xbaac93d5u, 0x7918fd8eu, 0x8c22631au, 
 const uint64_t kFpOne[6] = {0x760900000002fffdull, 0xebf4000bc40c0002ull, 0x5f48985753c758baull,
                             0x77ce585370525745ull, 0x5c071a97a256ec6dull, 0x15f65ec3fa80e493ull};
 
-Engine* engine_of(cdl_ctx* c) {
+}  // namespace
+
+Engine* cdlh::engine_of(cdl_ctx* c) {
   if (!c->engine) c->engine = new Engine(c);
   Engine* E = static_cast<Engine*>(c->engine);
   E->clear_fixed();  // begin_call selects the tables of its CRS; every other call runs without
   return E;
 }
 
-void affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a) {
+void cdlh::affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a) {
   bool inf = true;
   for (int i = 0; i < 6; i++) inf = inf && a.x.l[i] == 0 && a.y.l[i] == 0;
   if (inf) {
@@ -48,6 +52,8 @@ void affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a) {
     memcpy(out->z.l, kFpOne, 48);
   }
 }
+
+namespace {
 
 // n draws a_i from r, points a_i * G (rand.go:72-95), written to pool[dst..]
 int32_t rand_points_to_pool(Engine* E, cdl_rand* r, uint32_t gen_slot, uint32_t dst, size_t n) {

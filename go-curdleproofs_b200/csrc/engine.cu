@@ -282,17 +282,21 @@ int32_t Engine::decompress(const uint8_t* enc48, const std::vector<uint32_t>& ds
 
 static constexpr uint32_t kFixedMinTerms = 16;
 
-int32_t Engine::run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before) {
+int32_t Engine::run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before,
+                        const G1Affine* points) {
   ProfScope ps(prof.gpu);
   size_t nt = st.tasks.size(), nterm = st.idx.size();
   st.out48.resize(nt * 48);
   if (!nt) return CDL_OK;
+  if (!points) points = d_pool_;
   size_t max_terms = 0;
   for (auto& t : st.tasks) max_terms = std::max<size_t>(max_terms, t.term_cnt);
   int32_t rc;
   if ((rc = reserve(s_idx_, (nterm + 1) * 4)) || (rc = reserve(s_sc_, (nterm + 1) * 32)) ||
       (rc = reserve(s_task_, nt * sizeof(MsmTask))) || (rc = reserve(s_out_, nt * 48)))
     return rc;
+  // the latency kernel stages a task's terms in shared memory: every task it gets must fit
+  static_assert(cdl::kMsmSplitTerms <= cdl::kMsmMaxTerms, "small-MSM tasks must fit the kernel's staging");
   const bool throughput = (int)nt >= cdl::kMsmSplitThreshold || max_terms > cdl::kMsmSplitTerms;
   std::vector<uint32_t> fixed_tasks;  // tasks whose CRS terms go through the fixed-base tables
   {
@@ -355,16 +359,14 @@ int32_t Engine::run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_sca
     CDL_CUDA(ctx_, cudaMemcpyAsync(s_sub_.d, s_sub_.h, subs.size() * sizeof(cdl::MsmSub), cudaMemcpyHostToDevice, ctx_->stream));
     CDL_CUDA(ctx_, cudaMemcpyAsync(s_t2_.d, s_t2_.h, tasks2.size() * sizeof(cdl::MsmTask2), cudaMemcpyHostToDevice, ctx_->stream));
     tick();
-    cdl::launch_msm_tp(d_pool_, (const uint32_t*)s_idx_.d, (const cdl::Fr*)s_sc_.d, (int)nterm, (const cdl::MsmSub*)s_sub_.d,
+    cdl::launch_msm_tp(points, (const uint32_t*)s_idx_.d, (const cdl::Fr*)s_sc_.d, (int)nterm, (const cdl::MsmSub*)s_sub_.d,
                        (int)subs.size(), (const cdl::MsmTask2*)s_t2_.d, (int)nt, d_pool_, (uint8_t*)s_out_.d, d_win_,
                        ctx_->stream, fixed_, fsubs.empty() ? nullptr : (const uint32_t*)s_fsub_.d, (int)fsubs.size());
     tock(0, alg, 128.0 * nterm);
     launches += fsubs.empty() ? 3 : 4;  // recode, bucket warps, chunk sums (+ fixed-base warps); tock counted the combine
   } else {
-    if (max_terms > cdl::kMsmMaxTerms)
-      return ctx_->fail(CDL_ERR_TOO_LARGE, "msm of %zu terms exceeds the small-MSM limit %zu", max_terms, (size_t)cdl::kMsmMaxTerms);
     tick();
-    cdl::launch_msm_small(d_pool_, (const uint32_t*)s_idx_.d, (const cdl::Fr*)s_sc_.d, (const MsmTask*)s_task_.d, (int)nt,
+    cdl::launch_msm_small(points, (const uint32_t*)s_idx_.d, (const cdl::Fr*)s_sc_.d, (const MsmTask*)s_task_.d, (int)nt,
                           max_terms, d_pool_, (uint8_t*)s_out_.d, ctx_->stream);
     tock(0, alg, 128.0 * nterm);
   }

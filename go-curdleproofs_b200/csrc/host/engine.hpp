@@ -145,11 +145,15 @@ class Engine {
   int32_t compress(const std::vector<uint32_t>& src, std::vector<uint8_t>& out48);
   int32_t decompress(const uint8_t* enc48, const std::vector<uint32_t>& dst, std::vector<uint8_t>& status);
   // `before` (optional) runs on the stream after the stage's indices / scalars reached the device and before
-  // the MSM kernels: the verifier's scalar pipeline fills part of the scalar array there (d_scalars)
-  int32_t run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before = nullptr);
+  // the MSM kernels: the verifier's scalar pipeline fills part of the scalar array there (d_scalars).
+  // `points` (optional) is a device array the stage's indices refer to instead of the pool; results always
+  // go to pool[task.out_idx].
+  int32_t run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before = nullptr,
+                  const cdl::G1Affine* points = nullptr);
   int32_t run_elem(const std::vector<cdl::ElemOp>& ops, const std::vector<Fr>& sc);
 
   cdl_ctx* ctx() { return ctx_; }
+  cdl::G1Affine* d_pool() { return d_pool_; }
   ThreadPool& threads() { return pool_; }
   // instrumentation for bench.py: per kernel class (0 msm, 1 elementwise, 2 decompress,
   // 3 compress / normalise): launches, CUDA-event time on the launching stream,
@@ -222,5 +226,11 @@ struct WireProof {
 };
 // returns empty string on success, else the decode error
 std::string parse_wire_proof(const uint8_t* buf, size_t len, bool with_m, WireProof& out, size_t* used);
+
+// C ABI helpers (capi_protocol.cu).  The context's engine, created on first use; its fixed-base tables are
+// cleared (only a protocol call selects those of its CRS).
+Engine* engine_of(cdl_ctx* c);
+// gnark's G1Jac of an affine point: (x, y, 1), or (1, 1, 0) for infinity
+void affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a);
 
 }  // namespace cdlh

@@ -736,13 +736,9 @@ static uint32_t ba_grid(uint64_t npairs, int sm_count) {
     while (h) { uint32_t t = g % h; g = h; h = t; }
     return a / g * b;  // lcm
   }();
-  static const uint32_t target = [] {
-    const char* e = getenv("CDL_BA_BPT");
-    return e ? (uint32_t)atoi(e) : kBaTargetPairs;
-  }();
   const uint64_t wave = (uint64_t)per_sm * (uint64_t)sm_count;
   if (npairs < wave * kBaThreads * 2) return (uint32_t)((npairs + 2 * kBaThreads - 1) / (2 * kBaThreads));
-  uint64_t m = (npairs + wave * kBaThreads * target / 2) / (wave * kBaThreads * target);
+  uint64_t m = (npairs + wave * kBaThreads * kBaTargetPairs / 2) / (wave * kBaThreads * kBaTargetPairs);
   if (m < 1) m = 1;
   return (uint32_t)(m * wave);
 }
@@ -848,11 +844,8 @@ cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigM
       const uint32_t ntot = nblk * (uint32_t)kBaThreads;
       // totals per inverting thread: one field inversion costs ~ 85 products, so as few threads as keep
       // every scheduler busy (kBaInvThreadsPerSm per SM) share the totals among them
-      static const uint32_t inv_tpsm = [] {
-        const char* e = getenv("CDL_BA_INV_TPSM");
-        return e ? (uint32_t)atoi(e) : 256u;
-      }();
-      int G = (int)(ntot / ((uint32_t)sm_count * inv_tpsm));
+      constexpr uint32_t kBaInvThreadsPerSm = 256;
+      int G = (int)(ntot / ((uint32_t)sm_count * kBaInvThreadsPerSm));
       G = G < 1 ? 1 : G > 256 ? 256 : G;
       G1Affine* dst = work[(r - 1) & 1];
       if (r == 1) k_ba_fwd<false><<<nblk, kBaThreads, 0, st>>>(src, offsets + nb, r - 1, pre, totals);

@@ -19,7 +19,6 @@
 //                   chain is serial per MSM but runs at full lane efficiency across thousands of
 //                   MSMs, and overlaps the other lanes' kernels in a batched call.
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #define CDL_FP_MUL_CALL 1
@@ -186,7 +185,7 @@ k_msm_warp_gmem(const G1Affine* __restrict__ points, const MsmRec* __restrict__ 
 // whole L2) releases it, the next batched launch takes it back.
 struct L2Persist {
   int sms = 0;
-  size_t bytes = 0;       // carve-out this path asks for (0: unsupported / disabled)
+  size_t bytes = 0;       // carve-out this path asks for (0: unsupported)
   int max_window = 0;
   bool queried = false, on = false;
 };
@@ -202,7 +201,7 @@ static L2Persist& l2_state(int dev) {  // g_l2_mu held
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, dev) == cudaSuccess) {
       const size_t hot = (size_t)g.sms * kCtasPerSm * kWarpsPerCta * kWarpBucketBytes;
-      if (prop.persistingL2CacheMaxSize > 0 && !getenv("CDL_NO_L2_PERSIST"))
+      if (prop.persistingL2CacheMaxSize > 0)
         g.bytes = std::min<size_t>((size_t)prop.persistingL2CacheMaxSize, hot);
       cudaDeviceGetAttribute(&g.max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev);
     }
@@ -377,14 +376,8 @@ size_t msm_tp_scratch_bytes(size_t nterm, size_t nsub, size_t ntasks) {
 // additions against 2 mixed additions per term); shorter ones give more warps and a shorter tail.
 // Measured on B200 with batches of 2 048 Whisk round trips (MSM class per step): 64 terms 377 ms,
 // 128: 378, 160: 374, 256: 384, 512: 404, 1 024: 427; batched verification alone (one 712-term MSM
-// per proof) gains 5-12 % from 64-128 over 256.  CDL_MSM_CHUNK overrides the default of 128.
+// per proof) gains 5-12 % from 64-128 over 256.
 uint32_t msm_tp_pick_chunk(size_t nterm, int sm_count) {
-  static const uint32_t forced = [] {
-    const char* e = getenv("CDL_MSM_CHUNK");
-    int v = e ? atoi(e) : 0;
-    return (uint32_t)(v >= 8 && v <= 4096 ? v : 0);
-  }();
-  if (forced) return forced;
   // latency regime (a handful of large MSMs, e.g. the verifier's 5*ell + 8 terms for one proof):
   // too few 128-term chunks to occupy the machine, so cut finer and shorten each warp's serial walk
   if (nterm / kMsmChunk < (size_t)2 * sm_count) return 32;
@@ -433,12 +426,8 @@ void launch_msm_tp(const G1Affine* points, const uint32_t* idx, const Fr* scalar
     k_msm_warp_gmem<<<ctas, 32 * kWarpsPerCta, 0, st>>>(points, rec, subs, nsub, win, buckets, next);
   }
   k_msm_chunk_sum<<<(ntasks * nrows + 127) / 128, 128, 0, st>>>(win, tasks, ntasks, nsub, nrows, wsum);
-  static const int quad_max = [] {
-    const char* e = getenv("CDL_COMBINE_QUAD_MAX");
-    return e ? atoi(e) : kCombineQuadMaxTasks;
-  }();
   const int fs = fixed ? 1 : 0;
-  if (ntasks <= quad_max) k_msm_combine_quad<<<(ntasks + 7) / 8, 32, 0, st>>>(wsum, tasks, ntasks, fs, out_aff, out_c48);
+  if (ntasks <= kCombineQuadMaxTasks) k_msm_combine_quad<<<(ntasks + 7) / 8, 32, 0, st>>>(wsum, tasks, ntasks, fs, out_aff, out_c48);
   else k_msm_combine_tp<<<(ntasks + 63) / 64, 64, 0, st>>>(wsum, tasks, ntasks, fs, out_aff, out_c48);
 }
 

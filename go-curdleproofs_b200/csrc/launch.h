@@ -100,7 +100,7 @@ inline void msm_build_subs(const MsmTask* tasks, size_t ntasks, uint32_t chunk, 
 cudaError_t launch_exclusive_scan(uint32_t* counts, uint32_t n, uint32_t* bsum, uint32_t* offsets, cudaStream_t st,
                                   uint32_t pad = 0);
 
-// Latency path (k_msm.cu): one CTA per task.  Callers switch to the throughput path at
+// Latency path (k_msm.cu): one CTA per task.  Engine::run_msm switches to the throughput path at
 // kMsmSplitThreshold tasks per launch.
 constexpr int kMsmSplitThreshold = 96;
 // ... or when one task is long enough that a single CTA's thread-per-bucket walk is the slower choice

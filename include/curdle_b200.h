@@ -211,7 +211,8 @@ int32_t cdl_host_selftest(uint8_t* out32, const cdl_fr* a, const cdl_fr* b, cdl_
  * challenges.  Returns CDL_OK when both runs agree byte for byte; *used_x8 tells whether the
  * eight-way path was available on this host (0: both runs were scalar). */
 int32_t cdl_host_selftest_fibers(uint32_t n, uint32_t rounds, uint8_t* digest32, int32_t* used_x8);
-/* Per kernel class statistics of the protocol-level calls since the last reset
+/* Per kernel class statistics of the protocol-level calls and of the batched MSMs
+ * (cdl_g1_msm_batch, cdl_g1_msm_batch_device, cdl_g1_msm up to 1 024 terms) since the last reset
  * (class 0 small-MSM, 1 elementwise scalar-mul/fold, 2 decompress, 3 compress /
  * normalise): launches, CUDA-event milliseconds on the launching stream,
  * algorithmic modmul (SURVEY.md §8d conventions) and algorithmic bytes.
@@ -226,7 +227,7 @@ int32_t cdl_engine_busy_ms(cdl_ctx* ctx, double* busy_ms);
  * and host threads: one lane's host-side transcript work overlaps the other
  * lanes' kernels.  Results do not depend on it.  Also environment CDL_LANES. */
 int32_t cdl_set_lanes(cdl_ctx* ctx, int32_t lanes);
-/* Number of GPU kernels launched by protocol-level calls on this context so far. */
+/* Number of GPU kernels launched by protocol-level calls and batched MSMs on this context so far. */
 uint64_t cdl_launch_count(cdl_ctx* ctx);
 
 /* ---- large MSM, device-resident vectors, multi-GPU ----------------------

@@ -276,3 +276,40 @@ def test_msm_batch_over_device_resident_pool(ctx, pkg):
     assert affs_dec(aff3) == [None, None] and enc3 == (bytes([0xC0]) + bytes(47)) * 2
     for d in (pool, dx, L, Rr):
         d.close()
+
+
+def test_msm_calls_share_the_engine_pool_with_protocol_calls(ctx, pkg, pts):
+    """The batched-MSM entry points run on the context's engine and overwrite the start of the point pool
+    that the protocol calls keep their CRS image and instances in.  A batch of 32 Whisk round trips runs on
+    that same (root) engine; MSM calls between two runs with the same seeds must give the oracle's results
+    and leave the second run byte-identical to the first."""
+    ell, B = 12, 32
+    crs = ctx.generate_crs(ell, pkg.Rand(0))
+    r = pkg.Rand(1000)
+    rs, ks = r.get_frs(ell), r.get_frs(ell)
+    rG = ctx.g1_scalar_mul_affine(aff_enc(b.G1_GEN) * ell, rs, broadcast=False)
+    e1, e2 = ctx.g1_compress(rG), ctx.g1_compress(ctx.g1_scalar_mul_affine(rG, ks, broadcast=False))
+    pre = b"".join(e1[48 * j:48 * j + 48] + e2[48 * j:48 * j + 48] for j in range(ell)) * B
+
+    def round_trip():
+        post, proofs, status = ctx.whisk_generate_shuffle_proof_batch(crs, pre, [pkg.Rand(3000 + i) for i in range(B)])
+        ok, st = ctx.whisk_is_valid_shuffle_proof_batch(crs, pre, post, proofs, [pkg.Rand(2000 + i) for i in range(B)])
+        assert status == [0] * B and st == [0] * B and ok == [1] * B
+        return bytes(post), bytes(proofs)
+
+    first = round_trip()
+    random.seed(31)
+    offs = [0, 5, 5, 45, 46]
+    ps = [pts[random.randrange(len(pts))] for _ in range(offs[-1])]
+    sc = [random.randrange(R) for _ in range(offs[-1])]
+    got = affs_dec(ctx.g1_msm_batch(affs_enc(ps), frs_enc(sc), offs))
+    assert got == [b.g1_msm_naive(ps[offs[i]:offs[i + 1]], sc[offs[i]:offs[i + 1]]) for i in range(len(offs) - 1)]
+    pool = ctx.dev_buffer(96 * 10)
+    pool.upload(affs_enc(pts[:8]) + bytes(96 * 2))
+    sc = [random.randrange(R) for _ in range(8)]
+    aff, enc = ctx.g1_msm_batch_device(pool, list(range(8)), frs_enc(sc), [0, 3, 8], out_slot=[9, 8])
+    want = [b.g1_msm(pts[:3], sc[:3]), b.g1_msm(pts[3:8], sc[3:])]
+    assert affs_dec(aff) == want and enc == b"".join(b.g1_compress(p) for p in want)
+    assert affs_dec(pool.download(96 * 2, 96 * 8)) == want[::-1]
+    pool.close()
+    assert round_trip() == first
