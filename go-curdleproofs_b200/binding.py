@@ -91,6 +91,7 @@ def load_library():
     lib.cdl_whisk_is_valid_shuffle_proof_batch.argtypes = [vp, vp, sz, vp, vp, vp, sz, C.POINTER(vp), i32p, i32p]
     lib.cdl_whisk_generate_tracker_proof_batch.argtypes = [vp, sz, vp, vp, C.POINTER(vp), vp, i32p]
     lib.cdl_whisk_is_valid_tracker_proof_batch.argtypes = [vp, sz, vp, vp, vp, i32p, i32p]
+    lib.cdl_whisk_match_trackers.argtypes = [vp, sz, vp, sz, vp, i32p, i32p]
     lib.cdl_host_selftest.argtypes = [vp, vp, vp, vp]
     lib.cdl_host_selftest_fibers.argtypes = [C.c_uint32, C.c_uint32, vp, C.POINTER(C.c_int32)]
     lib.cdl_engine_stats.argtypes = [vp, vp, vp, vp, vp, C.c_int]
@@ -534,6 +535,17 @@ def _ctx_whisk_is_valid_tracker_proof_batch(self, trackers: bytes, k_comms: byte
     return list(ok), list(status)
 
 
+def _ctx_whisk_match_trackers(self, trackers: bytes, ks: bytes):
+    """Which of the V secrets in ks (V x 32 bytes, gnark fr.Element) own which of the T trackers
+    (T x 96 bytes) -> (owner list, status list); owner[t] is the smallest owning key index or -1."""
+    T = len(trackers) // 96
+    V = len(ks) // 32
+    owner = (C.c_int32 * max(T, 1))()
+    status = (C.c_int32 * max(T, 1))()
+    self._chk(self.lib.cdl_whisk_match_trackers(self.h, T, _inbuf(trackers), V, _inbuf(ks), owner, status))
+    return list(owner)[:T], list(status)[:T]
+
+
 def _ctx_engine_stats(self, reset: bool = False):
     """Per kernel class (msm, elem, decompress, compress): launches, event ms, algorithmic modmul / bytes."""
     n = (C.c_uint64 * 4)()
@@ -584,6 +596,7 @@ Context.whisk_generate_shuffle_proof_batch = _ctx_whisk_generate_batch
 Context.whisk_is_valid_shuffle_proof_batch = _ctx_whisk_is_valid_batch
 Context.whisk_generate_tracker_proof_batch = _ctx_whisk_generate_tracker_proof_batch
 Context.whisk_is_valid_tracker_proof_batch = _ctx_whisk_is_valid_tracker_proof_batch
+Context.whisk_match_trackers = _ctx_whisk_match_trackers
 Context.launch_count = _ctx_launch_count
 Context.engine_busy_ms = _ctx_engine_busy_ms
 Context.set_lanes = _ctx_set_lanes

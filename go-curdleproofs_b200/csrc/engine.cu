@@ -67,6 +67,7 @@ Engine::~Engine() {
   cudaSetDevice(ctx_->device);
   if (d_pool_) cudaFree(d_pool_);
   if (d_win_) cudaFree(d_win_);
+  if (d_match_) cudaFree(d_match_);
   for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_}) {
     if (s->h) cudaFreeHost(s->h);
     if (s->d) cudaFree(s->d);

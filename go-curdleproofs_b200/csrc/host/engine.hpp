@@ -151,6 +151,9 @@ class Engine {
   int32_t run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before = nullptr,
                   const cdl::G1Affine* points = nullptr);
   int32_t run_elem(const std::vector<cdl::ElemOp>& ops, const std::vector<Fr>& sc);
+  // Whisk tracker matching (capi_whisk_match.cu) on decoded trackers pool[t] = rG_t, pool[T + t] = krG_t:
+  // owner[t] = the smallest v with ks[v] * rG_t == krG_t, else INT32_MAX.  ks: V gnark fr.Element (Montgomery)
+  int32_t match_trackers(uint32_t T, const Fr* ks, uint32_t V, int32_t* owner);
 
   cdl_ctx* ctx() { return ctx_; }
   cdl::G1Affine* d_pool() { return d_pool_; }
@@ -203,6 +206,9 @@ class Engine {
   size_t pool_cap_ = 0;
   void* d_win_ = nullptr;  // window sums of the two-kernel MSM path
   size_t win_cap_ = 0;
+  void* d_match_ = nullptr;  // tables and window bases of one tile of trackers (match_scratch)
+  size_t match_cap_ = 0;
+  bool match_scratch(uint32_t tile);
   // pinned host staging + device scratch, grow-only
   struct Staging {
     void* h = nullptr;

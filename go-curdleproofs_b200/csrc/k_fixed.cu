@@ -1,33 +1,43 @@
-// Builds the fixed-base tables of a CRS (fixed_base.cuh) on the device.
+// Builds fixed-base tables (fixed_base.cuh) on the device: those of a CRS (width 12) and the per-tracker
+// tables of Whisk tracker matching (width kMatchC, k_match.cu).
 #define CDL_FP_MUL_CALL 1
 #include "fixed_base.cuh"
 #include "launch.h"
 
 namespace cdl {
 
-constexpr int kFbSeg = 8;                  // a (base, window) row is built by 8 threads, 256 entries each
-constexpr int kFbSegLen = kFbM / kFbSeg;
-constexpr int kFbNorm = 8;                 // entries normalised with one inversion
+constexpr int kFbSeg = 8;   // a (base, window) row is built by 8 threads, M / 8 entries each
+constexpr int kFbNorm = 8;  // entries normalised with one inversion (CRS tables)
 
-// thread (b, w, s): Q = 2^(12 w) P_b, then the entries (256 s + 1) Q .. (256 s + 256) Q by repeated addition
-// of Q; every 8 consecutive entries share one inversion (Montgomery's trick)
+// thread (b, w, s): Q = 2^(C w) P_b, then the entries (M/8 s + 1) Q .. (M/8 s + M/8) Q by repeated addition
+// of Q; consecutive entries share one inversion (Montgomery's trick).
+// Width 12 (CRS tables, built once per CRS): bases[b] = P_b, each thread doubles its way to Q; groups of 8.
+// Width kMatchC (tracker tables, built on every matching call): bases[b W + w] = 2^(C w) P_b is given
+// (launch_match_windows), and a thread's 16 entries share one inversion.
+template <int C>
 __global__ void __launch_bounds__(64)
 k_fixed_build(const G1Affine* __restrict__ bases, uint32_t nbase, G1Affine* __restrict__ tab) {
+  constexpr int W = fb_windows(C), M = fb_entries(C), kFbSegLen = M / kFbSeg;
+  constexpr bool kRowBases = C != kFbC;
+  constexpr int kNorm = kRowBases ? kFbSegLen : kFbNorm;
+  static_assert(kFbSegLen % kNorm == 0, "segment length");
   const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= nbase * (uint32_t)(kFbW * kFbSeg)) return;
-  const uint32_t b = t / (kFbW * kFbSeg), r = t - b * (kFbW * kFbSeg);
+  if (t >= nbase * (uint32_t)(W * kFbSeg)) return;
+  const uint32_t b = t / (W * kFbSeg), r = t - b * (W * kFbSeg);
   const int w = (int)(r / kFbSeg), s = (int)(r - (uint32_t)w * kFbSeg);
-  G1Affine* row = tab + ((size_t)b * kFbW + w) * kFbM + (size_t)s * kFbSegLen;
-  const G1Affine p = bases[b];
+  G1Affine* row = tab + ((size_t)b * W + w) * M + (size_t)s * kFbSegLen;
   G1Affine q;
-  {
+  if constexpr (kRowBases) {
+    q = bases[(size_t)b * W + w];
+  } else {
+    const G1Affine p = bases[b];
     G1Jac j;
     jac_from_affine(j, p);
 #pragma unroll 1
-    for (int i = 0; i < w * kFbC; i++) jac_dbl(j, j);
+    for (int i = 0; i < w * C; i++) jac_dbl(j, j);
     jac_to_affine(q, j);  // infinity stays infinity: the whole row is infinity then
   }
-  // acc = (256 s) Q
+  // acc = (M/8 s) Q
   G1Xyzz acc;
   xyzz_set_inf(acc);
   {
@@ -41,14 +51,14 @@ k_fixed_build(const G1Affine* __restrict__ bases, uint32_t nbase, G1Affine* __re
       }
     }
   }
-  G1Xyzz pend[kFbNorm];
-  Fp pre[kFbNorm];
+  G1Xyzz pend[kNorm];
+  Fp pre[kNorm];
 #pragma unroll 1
-  for (int base = 0; base < kFbSegLen; base += kFbNorm) {
+  for (int base = 0; base < kFbSegLen; base += kNorm) {
     Fp run;
     FpM::set_one(run);
 #pragma unroll 1
-    for (int e = 0; e < kFbNorm; e++) {
+    for (int e = 0; e < kNorm; e++) {
       xyzz_add_mixed(acc, acc, q);
       if (!xyzz_is_inf(acc)) FpM::mul(run, run, acc.zzz);
       pend[e] = acc;
@@ -57,7 +67,7 @@ k_fixed_build(const G1Affine* __restrict__ bases, uint32_t nbase, G1Affine* __re
     Fp inv;
     fp_inv(inv, run);
 #pragma unroll 1
-    for (int e = kFbNorm - 1; e >= 0; e--) {
+    for (int e = kNorm - 1; e >= 0; e--) {
       const G1Xyzz v = pend[e];
       G1Affine a;
       if (xyzz_is_inf(v)) {
@@ -78,11 +88,20 @@ k_fixed_build(const G1Affine* __restrict__ bases, uint32_t nbase, G1Affine* __re
   }
 }
 
-size_t fixed_table_bytes(uint32_t nbase) { return (size_t)nbase * kFbW * kFbM * sizeof(G1Affine); }
-
-void launch_fixed_build(const G1Affine* bases, uint32_t nbase, G1Affine* tab, cudaStream_t st) {
-  const uint32_t threads = nbase * (uint32_t)(kFbW * kFbSeg);
-  if (threads) k_fixed_build<<<(threads + 63) / 64, 64, 0, st>>>(bases, nbase, tab);
+template <int C>
+size_t fixed_table_bytes(uint32_t nbase) {
+  return (size_t)nbase * fb_windows(C) * fb_entries(C) * sizeof(G1Affine);
 }
+
+template <int C>
+void launch_fixed_build(const G1Affine* bases, uint32_t nbase, G1Affine* tab, cudaStream_t st) {
+  const uint32_t threads = nbase * (uint32_t)(fb_windows(C) * kFbSeg);
+  if (threads) k_fixed_build<C><<<(threads + 63) / 64, 64, 0, st>>>(bases, nbase, tab);
+}
+
+template size_t fixed_table_bytes<kFbC>(uint32_t);
+template void launch_fixed_build<kFbC>(const G1Affine*, uint32_t, G1Affine*, cudaStream_t);
+template size_t fixed_table_bytes<kMatchC>(uint32_t);
+template void launch_fixed_build<kMatchC>(const G1Affine*, uint32_t, G1Affine*, cudaStream_t);
 
 }  // namespace cdl

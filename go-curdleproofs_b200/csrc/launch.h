@@ -40,7 +40,25 @@ void launch_jac_to_affine(const G1Jac* in, G1Affine* out, int n, cudaStream_t st
 // double-and-add (the thread-per-op kernel only; small launches take the quad kernel)
 void launch_elem_ops(G1Affine* pool, const ElemOp* ops, const Fr* scalars, int n, cudaStream_t st,
                      FixedTable ft = FixedTable());
+// --- Whisk tracker matching (k_match.cu): owner[t] = min { v : ks[v] * rg[t] == krg[t] }, INT32_MAX if none.
+// launch_match_prep converts ks (device, Montgomery) to canonical form in place and resets owner[0 .. T).
+constexpr int kMatchC = 8;              // window width of the per-tracker tables: 32 windows x 128 entries, 384 KiB
+// Trackers whose tables are built, then used, together: bounds the table memory (96 MiB).  The resident warps of
+// k_match_table walk the keys of a few trackers at a time, so the tile's tables need not stay in the L2.
+constexpr uint32_t kMatchTile = 256;
+void launch_match_prep(Fr* ks, uint32_t V, int32_t* owner, uint32_t T, cudaStream_t st);
+void launch_match_shared(const G1Affine* rg, const G1Affine* krg, uint32_t T, const Fr* ks, uint32_t V,
+                         int32_t* owner, cudaStream_t st);
+// out[b W + w] = 2^(kMatchC w) rg[b], w < W = fb_windows(kMatchC), Jacobian (normalise with launch_jac_to_affine)
+void launch_match_windows(const G1Affine* rg, uint32_t nt, G1Jac* out, cudaStream_t st);
+// trackers t0 .. t0 + nt - 1 against every key; tab = launch_fixed_build<kMatchC>(window bases of rg + t0, nt, ..)
+void launch_match_table(const G1Affine* tab, const G1Affine* krg, uint32_t t0, uint32_t nt, const Fr* ks,
+                        uint32_t V, int32_t* owner, cudaStream_t st);
+// fixed-base tables of window width C for nbase points: C = 12 the CRS tables, bases = the points; C = kMatchC
+// the tracker tables, bases = their fb_windows(C) window bases each (launch_match_windows)
+template <int C = kFbC>
 size_t fixed_table_bytes(uint32_t nbase);
+template <int C = kFbC>
 void launch_fixed_build(const G1Affine* bases, uint32_t nbase, G1Affine* tab, cudaStream_t st);
 void launch_copy_ranges(G1Affine* pool, const CopyRange* ranges, int n, cudaStream_t st);
 // verifier scalar pipeline on the device (k_verify_scalars.cu): per-proof inputs, all Montgomery fr.Element

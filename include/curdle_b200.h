@@ -199,6 +199,18 @@ int32_t cdl_whisk_generate_tracker_proof_batch(cdl_ctx* ctx, size_t B, const uin
  * ok[b] is the reference's bool, status[b] its error (CDL_ERR_DECODE for malformed proof / points). */
 int32_t cdl_whisk_is_valid_tracker_proof_batch(cdl_ctx* ctx, size_t B, const uint8_t* trackers, const uint8_t* k_comms,
                                                const uint8_t* proofs, int32_t* ok, int32_t* status);
+/* Which of the caller's Whisk secrets own which trackers.  trackers: T x 96 bytes {rG, krG} as in
+ * cdl_whisk_generate_tracker_proof_batch; ks: V secrets (gnark fr.Element, Montgomery).
+ * owner[t] = the smallest v with ks[v] * rG_t == krG_t (equal as group elements), else -1.
+ * status[t] = CDL_OK, CDL_ERR_DECODE when either point fails SetBytes (flags, curve, subgroup),
+ * or CDL_ERR_PROTOCOL when rG_t is the point at infinity (such a tracker identifies nobody).
+ * owner[t] = -1 whenever status[t] != CDL_OK.  Returns CDL_OK when the arguments are valid,
+ * whatever the per-tracker statuses; CDL_ERR_INVALID_ARG for a null pointer, T == 0 or V == 0;
+ * CDL_ERR_TOO_LARGE when T or V exceeds CDL_WHISK_MATCH_MAX (2^24).  The reference leaves this
+ * check (k * rG == krG, one ScalarMultiplication per pair) to its caller. */
+#define CDL_WHISK_MATCH_MAX (1u << 24)
+int32_t cdl_whisk_match_trackers(cdl_ctx* ctx, size_t T, const uint8_t* trackers,
+                                 size_t V, const cdl_fr* ks, int32_t* owner, int32_t* status);
 
 /* Host-side self test (no GPU needed): out32 receives Merlin's published
  * "test protocol" challenge computed by the library's transcript code;
@@ -211,11 +223,12 @@ int32_t cdl_host_selftest(uint8_t* out32, const cdl_fr* a, const cdl_fr* b, cdl_
  * challenges.  Returns CDL_OK when both runs agree byte for byte; *used_x8 tells whether the
  * eight-way path was available on this host (0: both runs were scalar). */
 int32_t cdl_host_selftest_fibers(uint32_t n, uint32_t rounds, uint8_t* digest32, int32_t* used_x8);
-/* Per kernel class statistics of the protocol-level calls and of the batched MSMs
- * (cdl_g1_msm_batch, cdl_g1_msm_batch_device, cdl_g1_msm up to 1 024 terms) since the last reset
- * (class 0 small-MSM, 1 elementwise scalar-mul/fold, 2 decompress, 3 compress /
- * normalise): launches, CUDA-event milliseconds on the launching stream,
- * algorithmic modmul (SURVEY.md §8d conventions) and algorithmic bytes.
+/* Per kernel class statistics of the protocol-level calls, of the batched MSMs
+ * (cdl_g1_msm_batch, cdl_g1_msm_batch_device, cdl_g1_msm up to 1 024 terms) and of
+ * cdl_whisk_match_trackers since the last reset (class 0 small-MSM, 1 elementwise
+ * scalar-mul/fold and tracker matching, 2 decompress, 3 compress / normalise): launches,
+ * CUDA-event milliseconds on the launching stream, algorithmic modmul (SURVEY.md §8d
+ * conventions; 3 193 per matched (key, tracker) pair) and algorithmic bytes.
  * Each output array has 4 entries. */
 int32_t cdl_engine_stats(cdl_ctx* ctx, uint64_t* launches, double* ms, double* modmul, double* bytes, int reset);
 /* Device busy time since the last cdl_engine_stats(.., reset = 1): the length of
@@ -227,7 +240,8 @@ int32_t cdl_engine_busy_ms(cdl_ctx* ctx, double* busy_ms);
  * and host threads: one lane's host-side transcript work overlaps the other
  * lanes' kernels.  Results do not depend on it.  Also environment CDL_LANES. */
 int32_t cdl_set_lanes(cdl_ctx* ctx, int32_t lanes);
-/* Number of GPU kernels launched by protocol-level calls and batched MSMs on this context so far. */
+/* Number of GPU kernels launched by protocol-level calls, batched MSMs and tracker matching on this
+ * context so far. */
 uint64_t cdl_launch_count(cdl_ctx* ctx);
 
 /* ---- large MSM, device-resident vectors, multi-GPU ----------------------

@@ -163,3 +163,22 @@ func (c *Context) IsValidWhiskShuffleProofs(crs *CRS, pre, post, proofs []byte, 
 	}
 	return
 }
+
+// MatchWhiskTrackers finds which of the secrets ks own which of the trackers (96 bytes each): owner[t] is
+// the smallest v with ks[v]·rG_t == krG_t, else -1; status[t] != 0 when tracker t does not decode
+// (CDL_ERR_DECODE) or its rG is the point at infinity (CDL_ERR_PROTOCOL).  The reference leaves this
+// check to the caller, one ScalarMultiplication per (key, tracker) pair.
+func (c *Context) MatchWhiskTrackers(trackers []byte, ks []fr.Element) (owner, status []int32, err error) {
+	if len(trackers) == 0 || len(trackers)%TrackerSize != 0 || len(ks) == 0 {
+		return nil, nil, errStatus(C.int32_t(C.CDL_ERR_INVALID_ARG))
+	}
+	T := len(trackers) / TrackerSize
+	owner = make([]int32, T)
+	status = make([]int32, T)
+	rc := C.cdl_whisk_match_trackers(c.h, C.size_t(T), (*C.uint8_t)(unsafe.Pointer(&trackers[0])), C.size_t(len(ks)),
+		frPtr(ks), (*C.int32_t)(unsafe.Pointer(&owner[0])), (*C.int32_t)(unsafe.Pointer(&status[0])))
+	if rc != 0 {
+		return nil, nil, c.err(rc)
+	}
+	return owner, status, nil
+}
