@@ -110,6 +110,7 @@ def load_library():
     lib.cdl_set_msm_window.argtypes = [vp, i32]
     lib.cdl_set_msm_batch_affine.argtypes = [vp, i32]
     lib.cdl_set_fixed_base_min_batch.argtypes = [vp, i32]
+    lib.cdl_set_batch_verify_min.argtypes = [vp, i32]
     lib.cdl_comm_unique_id.argtypes = [vp]
     lib.cdl_comm_init.argtypes = [vp, vp, i32, i32]
     lib.cdl_comm_destroy.argtypes = [vp]
@@ -326,6 +327,10 @@ def _ctx_set_msm_window(self, bits: int):
 
 def _ctx_set_fixed_base_min_batch(self, instances: int):
     self._chk(self.lib.cdl_set_fixed_base_min_batch(self.h, instances))
+
+
+def _ctx_set_batch_verify_min(self, proofs: int):
+    self._chk(self.lib.cdl_set_batch_verify_min(self.h, proofs))
 
 
 def _ctx_set_msm_batch_affine(self, rounds: int):
@@ -580,6 +585,7 @@ Context.g1_msm_device = _ctx_g1_msm_device
 Context.set_msm_window = _ctx_set_msm_window
 Context.set_msm_batch_affine = _ctx_set_msm_batch_affine
 Context.set_fixed_base_min_batch = _ctx_set_fixed_base_min_batch
+Context.set_batch_verify_min = _ctx_set_batch_verify_min
 Context.comm_init = _ctx_comm_init
 Context.comm_destroy = _ctx_comm_destroy
 Context.g1_msm_sharded_device = _ctx_g1_msm_sharded_device

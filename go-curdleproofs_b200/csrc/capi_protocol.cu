@@ -334,6 +334,13 @@ int32_t cdl_set_fixed_base_min_batch(cdl_ctx* c, int32_t instances) {
   return CDL_OK;
 }
 
+int32_t cdl_set_batch_verify_min(cdl_ctx* c, int32_t proofs) {
+  if (!c || proofs < -1) return CDL_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lk(c->mu);
+  c->root()->batch_verify_min = proofs;
+  return CDL_OK;
+}
+
 void cdl_crs_free(cdl_crs* crs) {
   if (!crs) return;
   if (crs->d_points) { cudaSetDevice(crs->ctx->device); cudaFree(crs->d_points); }

@@ -38,6 +38,7 @@ struct cdl_ctx {
   int comm_rank = 0, comm_world = 1;
   int msm_c_override = 0;  // CDL_MSM_C / cdl_set_msm_window: 0 = pick by size
   int fixed_min_batch = -1;  // cdl_set_fixed_base_min_batch: instances per (lane) call from which the CRS fixed-base tables are used; -1 = CDL_FIXED_BASE_MINB or 64, 0 = never
+  int batch_verify_min = -1;  // cdl_set_batch_verify_min: proofs per (lane) verification from which one combined MSM checks the batch first; -1 = default, 0 = never
   int msm_ba_override = -1;  // cdl_set_msm_batch_affine: batch-affine rounds of the large MSM, -1 = pick by bucket load
   // Batched protocol calls are cut into up to n_lanes sub-batches that advance
   // concurrently, each on its own lane context (same device, own stream, engine,

@@ -68,7 +68,8 @@ Engine::~Engine() {
   if (d_pool_) cudaFree(d_pool_);
   if (d_win_) cudaFree(d_win_);
   if (d_match_) cudaFree(d_match_);
-  for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_}) {
+  if (d_bv_) cudaFree(d_bv_);
+  for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_, &s_bv_}) {
     if (s->h) cudaFreeHost(s->h);
     if (s->d) cudaFree(s->d);
   }
@@ -283,8 +284,7 @@ int32_t Engine::decompress(const uint8_t* enc48, const std::vector<uint32_t>& ds
 
 static constexpr uint32_t kFixedMinTerms = 16;
 
-int32_t Engine::run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before,
-                        const G1Affine* points) {
+int32_t Engine::run_msm(MsmStage& st, const MsmBefore& before, const G1Affine* points) {
   ProfScope ps(prof.gpu);
   size_t nt = st.tasks.size(), nterm = st.idx.size();
   st.out48.resize(nt * 48);
@@ -324,8 +324,13 @@ int32_t Engine::run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_sca
   CDL_CUDA(ctx_, cudaMemcpyAsync(s_sc_.d, s_sc_.h, nterm * 32, cudaMemcpyHostToDevice, ctx_->stream));
   CDL_CUDA(ctx_, cudaMemcpyAsync(s_task_.d, s_task_.h, nt * sizeof(MsmTask), cudaMemcpyHostToDevice, ctx_->stream));
   if (before) {
-    int32_t brc = before((cdl::Fr*)s_sc_.d);
+    bool done = false;
+    int32_t brc = before((const uint32_t*)s_idx_.d, (cdl::Fr*)s_sc_.d, (const MsmTask*)s_task_.d, done);
     if (brc) return brc;
+    if (done) {
+      std::fill(st.out48.begin(), st.out48.end(), 0);
+      return CDL_OK;
+    }
   }
   double alg = 0;
   // credited per task at the reference's term count (a base expanded into several CRS terms counts once)

@@ -145,11 +145,13 @@ class Engine {
   int32_t compress(const std::vector<uint32_t>& src, std::vector<uint8_t>& out48);
   int32_t decompress(const uint8_t* enc48, const std::vector<uint32_t>& dst, std::vector<uint8_t>& status);
   // `before` (optional) runs on the stream after the stage's indices / scalars reached the device and before
-  // the MSM kernels: the verifier's scalar pipeline fills part of the scalar array there (d_scalars).
+  // the MSM kernels: the verifier's scalar pipeline fills part of the scalar array there (d_scalars), and its
+  // combined check reads the stage (d_idx: host indices plus kMsmIdxFixed flags; d_tasks).  Setting `done`
+  // skips the MSM kernels: out48 is then left zero.
   // `points` (optional) is a device array the stage's indices refer to instead of the pool; results always
   // go to pool[task.out_idx].
-  int32_t run_msm(MsmStage& st, const std::function<int32_t(cdl::Fr* d_scalars)>& before = nullptr,
-                  const cdl::G1Affine* points = nullptr);
+  using MsmBefore = std::function<int32_t(const uint32_t* d_idx, cdl::Fr* d_scalars, const cdl::MsmTask* d_tasks, bool& done)>;
+  int32_t run_msm(MsmStage& st, const MsmBefore& before = nullptr, const cdl::G1Affine* points = nullptr);
   int32_t run_elem(const std::vector<cdl::ElemOp>& ops, const std::vector<Fr>& sc);
   // Whisk tracker matching (capi_whisk_match.cu) on decoded trackers pool[t] = rG_t, pool[T + t] = krG_t:
   // owner[t] = the smallest v with ks[v] * rG_t == krG_t, else INT32_MAX.  ks: V gnark fr.Element (Montgomery)
@@ -209,13 +211,20 @@ class Engine {
   void* d_match_ = nullptr;  // tables and window bases of one tile of trackers (match_scratch)
   size_t match_cap_ = 0;
   bool match_scratch(uint32_t tile);
+  void* d_bv_ = nullptr;  // combined verifier check: term list, large-MSM scratch, result (batch_check)
+  size_t bv_cap_ = 0;
+  // The verifier's second MSM stage `st`, uploaded (d_idx, d_sc, d_tasks), as one large MSM with the weight
+  // rho[t] (Montgomery) on task t and the CRS bases (pool indices < crs_size) merged: *all_inf = whether it
+  // is the point at infinity.
+  int32_t batch_check(const MsmStage& st, const std::vector<Fr>& rho, uint32_t crs_size, const uint32_t* d_idx,
+                      const cdl::Fr* d_sc, const cdl::MsmTask* d_tasks, bool* all_inf);
   // pinned host staging + device scratch, grow-only
   struct Staging {
     void* h = nullptr;
     void* d = nullptr;
     size_t cap = 0;
   };
-  Staging s_idx_, s_sc_, s_task_, s_out_, s_ops_, s_enc_, s_st_, s_jac_, s_sub_, s_t2_, s_cr_, s_fsub_, s_vs_, s_as_;
+  Staging s_idx_, s_sc_, s_task_, s_out_, s_ops_, s_enc_, s_st_, s_jac_, s_sub_, s_t2_, s_cr_, s_fsub_, s_vs_, s_as_, s_bv_;
   int32_t reserve(Staging& s, size_t bytes);
   void tick();                                   // event before a kernel
   void tock(int cls, double modmul, double bytes);  // event after; call finish_timing() after the sync

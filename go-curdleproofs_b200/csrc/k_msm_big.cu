@@ -117,10 +117,10 @@ __device__ __forceinline__ uint32_t big_raw_digit(const uint32_t* k6, int w, int
 }
 
 __global__ void __launch_bounds__(256)
-k_big_tables(const G1Affine* __restrict__ points, int n, BigPoint* __restrict__ tab) {
+k_big_tables(const G1Affine* __restrict__ points, const uint32_t* __restrict__ idx, int n, BigPoint* __restrict__ tab) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const G1Affine p = points[i];
+  const G1Affine p = points[idx ? idx[i] : (uint32_t)i];
   Fp beta, bx;
   fp_set_beta(beta);
   FpM::mul(bx, p.x, beta);  // infinity (0, 0) stays (0, 0)
@@ -791,8 +791,9 @@ size_t big_msm_scratch_bytes(const BigMsmDims& d) { return big_layout(d).total; 
 
 // All launches go to `st`; nothing synchronises.  d_out receives one G1Jac.
 cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigMsmDims& d, int normalize,
-                           void* scratch, int sm_count, G1Jac* d_out, cudaStream_t st) {
-  msm_l2_carveout(false);  // the point gathers want the whole L2
+                           void* scratch, int sm_count, G1Jac* d_out, cudaStream_t st, const uint32_t* idx,
+                           bool release_l2, int* nkernels) {
+  if (release_l2) msm_l2_carveout(false);  // the point gathers want the whole L2
   uint8_t* base = (uint8_t*)scratch;
   BigLayout L = big_layout(d);
   uint32_t* counts = (uint32_t*)(base + L.counts);
@@ -816,6 +817,7 @@ cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigM
     BigMsmDims e = d;
     e.nlocal = 1; e.wfirst = 0; e.wstep = 1; e.c = 0;
     k_big_horner<<<1, 32, 0, st>>>(one, e, normalize, d_out);
+    if (nkernels) *nkernels = 1;
     return cudaGetLastError();
   }
   const uint32_t nb = d.nb;
@@ -824,7 +826,7 @@ cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigM
   cudaMemsetAsync(counts, 0, ((size_t)nb + 1) * 4, st);
   cudaMemsetAsync(meta, 0, 256, st);
   const int gd = (d.n + 255) / 256;
-  k_big_tables<<<gd, 256, 0, st>>>(points, d.n, tab);
+  k_big_tables<<<gd, 256, 0, st>>>(points, idx, d.n, tab);
   k_big_digits<0><<<gd, 256, 0, st>>>(scalars, d.n, d, counts, nullptr, nullptr);
   cudaError_t se = launch_exclusive_scan(counts, nb, bsum, offsets, st, (1u << R) - 1u);
   if (se != cudaSuccess) return se;
@@ -878,8 +880,9 @@ cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigM
   int total = d.nlocal * per;
   if (total <= kBigQuadMaxOutputs) k_big_reduce1_quad<<<(4 * total + 127) / 128, 128, 0, st>>>(buckets, d.M, Lc, total, red[0]);
   else k_big_reduce1<<<(total + 127) / 128, 128, 0, st>>>(buckets, d.M, Lc, total, red[0]);
-  int cur = 0;
+  int cur = 0, nsum = 0;
   while (per > 1) {
+    nsum++;
     int G = per > 256 ? 16 : (per > 16 ? 8 : per);
     int pout = (per + G - 1) / G;
     int tot = d.nlocal * pout;
@@ -889,6 +892,8 @@ cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigM
     per = pout;
   }
   k_big_horner<<<1, 32, 0, st>>>(red[cur], d, normalize, d_out);
+  // tables, 2 digits, 2 x 3 scan, 2 size sort, mark, accum, slice, finish, reduce1, horner: 17; 3 per round
+  if (nkernels) *nkernels = 17 + 3 * R + nsum;
   return cudaGetLastError();
 }
 

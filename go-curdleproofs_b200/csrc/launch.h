@@ -72,6 +72,14 @@ struct VsParams {
 };
 void launch_verify_scalars(const VsParams* params, const Fr* as, Fr* sc, uint32_t nproofs, uint32_t ell, uint32_t n,
                            uint32_t m, cudaStream_t st);
+// combined verifier check (k_batch_verify.cu), all scalars Montgomery: term j < nterm of the stage becomes
+// (idx[j] without flags, sc[j] * rho[task of j]); then for each CRS base b < ncrs the weighted scalars of its
+// terms (stage positions crs_pos[crs_off[b] .. crs_off[b + 1])) are summed into term nterm + b and zeroed in place
+void launch_bv_assemble(const uint32_t* idx, const Fr* sc, const MsmTask* tasks, uint32_t ntask, const Fr* rho,
+                        uint32_t nterm, const uint32_t* crs_off, const uint32_t* crs_pos, uint32_t ncrs, uint32_t* cidx,
+                        Fr* csc, cudaStream_t st);
+// flag[0] = 1 if r[0] is the point at infinity, else 0
+void launch_bv_is_inf(const G1Jac* r, uint32_t* flag, cudaStream_t st);
 // indexed codecs on a pool: enc[i] <- pool[src[i]] ; pool[dst[i]] <- enc[i]
 void launch_compress_idx(const G1Affine* pool, const uint32_t* src, uint8_t* out48, int n, cudaStream_t s);
 void launch_decompress_idx(const uint8_t* in48, G1Affine* pool, const uint32_t* dst, uint8_t* status, int n,
@@ -147,8 +155,12 @@ size_t big_msm_scratch_bytes(const BigMsmDims& d);
 inline uint64_t big_msm_entries(const BigMsmDims& d) {
   return 2ull * (uint64_t)d.n * (uint64_t)d.nlocal + (uint64_t)d.nb * (((uint64_t)1 << d.R) - 1);
 }
+// idx (optional): term i's base is points[idx[i]].  release_l2: drop the persisting-L2 window of the batched
+// small-MSM path first (a process-wide limit; a caller whose other streams run that path keeps it).
+// nkernels (optional) receives the number of kernels launched.
 cudaError_t launch_big_msm(const G1Affine* points, const Fr* scalars, const BigMsmDims& d, int normalize,
-                           void* scratch, int sm_count, G1Jac* d_out, cudaStream_t st);
+                           void* scratch, int sm_count, G1Jac* d_out, cudaStream_t st, const uint32_t* idx = nullptr,
+                           bool release_l2 = true, int* nkernels = nullptr);
 void launch_big_combine(const G1Jac* in, int n, G1Jac* out, cudaStream_t st);
 
 }  // namespace cdl

@@ -146,6 +146,12 @@ size_t cdl_crs_ell(const cdl_crs* crs);
  * object) instead of running buckets / double-and-add over them.  -1 = default (environment
  * CDL_FIXED_BASE_MINB, else 64), 0 = never.  Tuning aid; results do not depend on it. */
 int32_t cdl_set_fixed_base_min_batch(cdl_ctx* ctx, int32_t instances);
+/* Batched Whisk shuffle-proof verification (cdl_whisk_is_valid_shuffle_proof_batch): a lane of at least
+ * `proofs` proofs first checks all of its proofs' final verifier equations at once, as one large MSM over a
+ * random linear combination of them (128-bit weights derived from the batch; a false pass has probability
+ * at most 2^-128).  When that sum is not the point at infinity, the proofs are checked one by one as
+ * without it.  -1 = default (64), 0 = never.  Tuning aid; results do not depend on it. */
+int32_t cdl_set_batch_verify_min(cdl_ctx* ctx, int32_t proofs);
 void cdl_crs_free(cdl_crs* crs);
 
 /* common.ShufflePermuteCommit (common/util.go:45-88): Ts = perm(k*Rs), Us = perm(k*Ss),

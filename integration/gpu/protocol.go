@@ -106,6 +106,15 @@ func (c *Context) Prove(crs *CRS, Rs, Ss, Ts, Us []bls12381.G1Affine, M *bls1238
 	return buf[:n], nil
 }
 
+// SetBatchVerifyMin is cdl_set_batch_verify_min: lanes of at least proofs proofs check their whole batch
+// with one combined MSM first (-1 = default, 0 = never).  Results do not depend on it.
+func (c *Context) SetBatchVerifyMin(proofs int) error {
+	if rc := C.cdl_set_batch_verify_min(c.h, C.int32_t(proofs)); rc != 0 {
+		return c.err(rc)
+	}
+	return nil
+}
+
 // Verify is Proof.FromReader + curdleproof.Verify (curdleproof.go:199-318): (bool, error) as in the
 // reference — (false, nil) for an invalid proof, (false, err) for malformed input.
 func (c *Context) Verify(crs *CRS, proof []byte, Rs, Ss, Ts, Us []bls12381.G1Affine, M *bls12381.G1Jac, r *Rand) (bool, error) {
