@@ -85,6 +85,10 @@ def load_library():
     lib.cdl_shuffle_permute_commit.argtypes = [vp, vp, vp, vp, u32p, vp, vp, vp, vp, vp, vp]
     lib.cdl_prove.argtypes = [vp, vp, vp, vp, vp, vp, vp, u32p, vp, vp, vp, vp, sz, C.POINTER(sz)]
     lib.cdl_verify.argtypes = [vp, vp, vp, sz, vp, vp, vp, vp, vp, vp, i32p]
+    szp = C.POINTER(sz)
+    lib.cdl_shuffle_permute_commit_batch.argtypes = [vp, vp, sz, vp, vp, u32p, vp, C.POINTER(vp), vp, vp, vp, vp, i32p]
+    lib.cdl_prove_batch.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp, u32p, vp, vp, C.POINTER(vp), vp, sz, szp, i32p]
+    lib.cdl_verify_batch.argtypes = [vp, vp, sz, vp, sz, szp, vp, vp, vp, vp, vp, C.POINTER(vp), i32p, i32p]
     lib.cdl_whisk_generate_shuffle_proof.argtypes = [vp, vp, vp, vp, vp, vp, sz]
     lib.cdl_whisk_is_valid_shuffle_proof.argtypes = [vp, vp, vp, vp, sz, sz, vp, sz, vp, i32p]
     lib.cdl_whisk_generate_shuffle_proof_batch.argtypes = [vp, vp, sz, vp, C.POINTER(vp), vp, vp, sz, i32p]
@@ -458,7 +462,7 @@ def _ctx_shuffle_permute_commit(self, crs: CRS, Rs: bytes, Ss: bytes, perm, k: b
 def _ctx_prove(self, crs: CRS, Rs, Ss, Ts, Us, M, perm, k, rs_m, rand: Rand) -> bytes:
     """curdleproof.Prove + Proof.Serialize."""
     ell = crs.ell
-    cap = 48 * (18 + 10 * 32) + 32 * 7 + 40
+    cap = PROOF_CAP
     out = C.create_string_buffer(cap)
     n = C.c_size_t()
     p = (C.c_uint32 * ell)(*perm)
@@ -471,6 +475,69 @@ def _ctx_verify(self, crs: CRS, proof: bytes, Rs, Ss, Ts, Us, M, rand: Rand) -> 
     ok = C.c_int32()
     self._chk(self.lib.cdl_verify(self.h, crs.h, proof, len(proof), Rs, Ss, Ts, Us, M, rand.h, C.byref(ok)))
     return bool(ok.value)
+
+
+PROOF_CAP = 48 * (18 + 10 * 32) + 32 * 7 + 40  # the largest proof Prove serializes (lg n < 32)
+
+
+def _split(buf, n: int, size: int):
+    return [bytes(buf[i * size:(i + 1) * size]) for i in range(n)]
+
+
+def _perms(perms, B: int, ell: int):
+    flat = [p for perm in perms for p in perm]
+    if len(perms) != B or len(flat) != B * ell:
+        raise CdlError(-3, "every instance needs a permutation of ell entries")
+    return (C.c_uint32 * (B * ell))(*flat)
+
+
+def _ctx_shuffle_permute_commit_batch(self, crs: CRS, Rs, Ss, perms, ks, rands):
+    """common.ShufflePermuteCommit for B = len(rands) instances.  Rs, Ss and ks are lists of per-instance
+    byte strings (ell affine points, one fr.Element), perms a list of permutations.  Returns per-instance
+    lists (Ts, Us, M jac, rs_m, status); an instance whose status is not 0 has zero-filled outputs."""
+    B, ell = len(rands), crs.ell
+    pb = ell * G1_AFFINE_BYTES
+    Ts, Us = bytearray(B * pb), bytearray(B * pb)
+    M, rs_m = bytearray(B * G1_JAC_BYTES), bytearray(B * 4 * FR_BYTES)
+    status = (C.c_int32 * max(1, B))()
+    rh = (C.c_void_p * max(1, B))(*[r.h for r in rands])
+    self._chk(self.lib.cdl_shuffle_permute_commit_batch(
+        self.h, crs.h, B, b"".join(Rs), b"".join(Ss), _perms(perms, B, ell), b"".join(ks), rh, _inbuf(Ts), _inbuf(Us),
+        _inbuf(M), _inbuf(rs_m), status))
+    return (_split(Ts, B, pb), _split(Us, B, pb), _split(M, B, G1_JAC_BYTES), _split(rs_m, B, 4 * FR_BYTES),
+            list(status)[:B])
+
+
+def _ctx_prove_batch(self, crs: CRS, Rs, Ss, Ts, Us, Ms, perms, ks, rs_ms, rands, proof_cap: int = PROOF_CAP):
+    """curdleproof.Prove + Proof.Serialize for B = len(rands) instances (lists of per-instance byte strings as
+    in shuffle_permute_commit_batch).  Returns (proofs, proof lengths, status): proofs[b] is b"" unless
+    status[b] == 0; the length is also reported when the proof did not fit proof_cap."""
+    B, ell = len(rands), crs.ell
+    out = bytearray(max(1, B) * proof_cap)
+    lens = (C.c_size_t * max(1, B))()
+    status = (C.c_int32 * max(1, B))()
+    rh = (C.c_void_p * max(1, B))(*[r.h for r in rands])
+    self._chk(self.lib.cdl_prove_batch(
+        self.h, crs.h, B, b"".join(Rs), b"".join(Ss), b"".join(Ts), b"".join(Us), b"".join(Ms), _perms(perms, B, ell),
+        b"".join(ks), b"".join(rs_ms), rh, _inbuf(out), proof_cap, lens, status))
+    proofs = [bytes(out[b * proof_cap:b * proof_cap + lens[b]]) if status[b] == 0 else b"" for b in range(B)]
+    return proofs, list(lens)[:B], list(status)[:B]
+
+
+def _ctx_verify_batch(self, crs: CRS, proofs, Rs, Ss, Ts, Us, Ms, rands):
+    """Proof.FromReader + curdleproof.Verify for B = len(rands) instances: proofs is a list of proof byte
+    strings, the instance arguments lists as in prove_batch.  Returns (ok, status) lists; status[b] is
+    what cdl_verify would have returned for instance b."""
+    B = len(rands)
+    stride = max([len(p) for p in proofs] + [1])
+    buf = b"".join(p.ljust(stride, b"\0") for p in proofs)
+    lens = (C.c_size_t * max(1, B))(*[len(p) for p in proofs])
+    ok = (C.c_int32 * max(1, B))()
+    status = (C.c_int32 * max(1, B))()
+    rh = (C.c_void_p * max(1, B))(*[r.h for r in rands])
+    self._chk(self.lib.cdl_verify_batch(self.h, crs.h, B, buf, stride, lens, b"".join(Rs), b"".join(Ss), b"".join(Ts),
+                                        b"".join(Us), b"".join(Ms), rh, ok, status))
+    return list(ok)[:B], list(status)[:B]
 
 
 def _ctx_whisk_generate(self, crs: CRS, pre: bytes, rand: Rand, proof_size: int = 4576):
@@ -596,6 +663,9 @@ Context.crs_from_points = _ctx_crs_from_points
 Context.shuffle_permute_commit = _ctx_shuffle_permute_commit
 Context.prove = _ctx_prove
 Context.verify = _ctx_verify
+Context.shuffle_permute_commit_batch = _ctx_shuffle_permute_commit_batch
+Context.prove_batch = _ctx_prove_batch
+Context.verify_batch = _ctx_verify_batch
 Context.whisk_generate_shuffle_proof = _ctx_whisk_generate
 Context.whisk_is_valid_shuffle_proof = _ctx_whisk_is_valid
 Context.whisk_generate_shuffle_proof_batch = _ctx_whisk_generate_batch

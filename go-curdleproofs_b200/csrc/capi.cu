@@ -32,7 +32,7 @@ static bool msm_tasks(const uint32_t* offsets, size_t k, std::vector<MsmTask>& t
 
 extern "C" {
 
-uint32_t cdl_abi_version(void) { return (1u << 16) | 6u; }
+uint32_t cdl_abi_version(void) { return (1u << 16) | 7u; }
 
 int32_t cdl_create(int device, cdl_ctx** out) {
   if (!out) return CDL_ERR_INVALID_ARG;

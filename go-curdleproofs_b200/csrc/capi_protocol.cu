@@ -99,14 +99,20 @@ struct Prep {
   Layout L;
 };
 
-// common prologue of the protocol calls
-int32_t begin_call(cdl_ctx* c, const cdl_crs* crs, size_t B, Engine** E, Layout* L) {
+constexpr size_t kPoolIndexLimit = (size_t)1 << 30;  // MSM term indices carry flags in bits 30 and 31
+
+// common prologue of the protocol calls; `intake`: room behind the instance regions for Engine::load_instances
+int32_t begin_call(cdl_ctx* c, const cdl_crs* crs, size_t B, Engine** E, Layout* L, bool intake = false) {
   if (crs->ctx != c->root()) return c->fail(CDL_ERR_INVALID_ARG, "crs belongs to another context");
+  *L = Layout(crs->ell);
+  const size_t need = (size_t)L->crs_size + B * (size_t)L->inst_size + (intake ? Engine::intake_points(*L, B) : 0);
+  if (need >= kPoolIndexLimit)
+    return c->fail(CDL_ERR_TOO_LARGE, "%zu instances of ell = %u need %zu pool points; pool indices are below 2^30", B,
+                   L->ell, need);
   CDL_CUDA(c, cudaSetDevice(c->device));
   *E = engine_of(c);
-  *L = Layout(crs->ell);
   c->spin_wait = B < 8 && c->parent == nullptr;  // latency regime: see cdl_ctx::sync_stream
-  int32_t rc = (*E)->ensure_pool((size_t)L->crs_size + B * (size_t)L->inst_size);
+  int32_t rc = (*E)->ensure_pool(need);
   if (rc) return rc;
   (*E)->select_fixed(*L, crs, B);
   return (*E)->load_crs(*L, crs);
@@ -348,70 +354,167 @@ void cdl_crs_free(cdl_crs* crs) {
   delete crs;
 }
 
-// ------------------------------------------------------------------ ShufflePermuteCommit
-int32_t cdl_shuffle_permute_commit(cdl_ctx* c, const cdl_crs* crs, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
-                                   const uint32_t* perm, const cdl_fr* k, cdl_rand* r, cdl_g1_affine* Ts,
-                                   cdl_g1_affine* Us, cdl_g1_jac* M, cdl_fr* rs_m) {
-  if (!c || !crs || !Rs || !Ss || !perm || !k || !r || !Ts || !Us || !M || !rs_m) return CDL_ERR_INVALID_ARG;
+}  // extern "C"
+
+// ------------------------------------------------------------------ ShufflePermuteCommit / Prove / Verify
+// The batched forms take B caller-supplied instances (instance-major arrays) and give every instance what
+// the single call gives it; the single calls are their B = 1 front ends.
+namespace {
+
+bool rands_present(cdl_rand* const* rands, size_t B) {
+  for (size_t b = 0; b < B; b++)
+    if (!rands[b]) return false;
+  return true;
+}
+
+// the instances whose permutation is in range; the others fail with CDL_ERR_INVALID_ARG before any draw
+std::vector<uint32_t> valid_instances(cdl_ctx* c, uint32_t ell, size_t B, const uint32_t* perms, int32_t* status) {
+  std::vector<uint32_t> sel;
+  sel.reserve(B);
+  for (size_t b = 0; b < B; b++) {
+    const uint32_t* p = perms + b * ell;
+    status[b] = CDL_OK;
+    for (uint32_t i = 0; i < ell && status[b] == CDL_OK; i++)
+      if (p[i] >= ell) status[b] = c->fail(CDL_ERR_INVALID_ARG, "permutation entry out of range");
+    if (status[b] == CDL_OK) sel.push_back((uint32_t)b);
+  }
+  return sel;
+}
+
+}  // namespace
+
+extern "C" {
+
+int32_t cdl_shuffle_permute_commit_batch(cdl_ctx* c, const cdl_crs* crs, size_t B, const cdl_g1_affine* Rs,
+                                         const cdl_g1_affine* Ss, const uint32_t* perms, const cdl_fr* ks,
+                                         cdl_rand* const* rands, cdl_g1_affine* Ts, cdl_g1_affine* Us, cdl_g1_jac* M,
+                                         cdl_fr* rs_m, int32_t* status) {
+  if (!c || !crs || B == 0 || !Rs || !Ss || !perms || !ks || !rands || !Ts || !Us || !M || !rs_m || !status ||
+      !rands_present(rands, B))
+    return CDL_ERR_INVALID_ARG;
+  if (size_t G = lanes_for(c, B); G > 1) {
+    const size_t e = crs->ell;
+    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_shuffle_permute_commit_batch(lane, crs, hi - lo, Rs + lo * e, Ss + lo * e, perms + lo * e, ks + lo,
+                                              rands + lo, Ts + lo * e, Us + lo * e, M + lo, rs_m + 4 * lo, status + lo);
+    });
+  }
   std::lock_guard<std::mutex> lk(c->mu);
   Engine* E;
   Layout L(1);
-  int32_t rc = begin_call(c, crs, 1, &E, &L);
+  int32_t rc = begin_call(c, crs, B, &E, &L, true);
   if (rc) return rc;
-  const uint32_t ell = L.ell, base = L.base(0);
-  for (uint32_t i = 0; i < ell; i++)
-    if (perm[i] >= ell) return c->fail(CDL_ERR_INVALID_ARG, "permutation entry out of range");
-  if ((rc = E->upload_points(base + L.Rs, Rs, ell)) || (rc = E->upload_points(base + L.Ss, Ss, ell))) return rc;
-  std::vector<std::vector<uint32_t>> perms(1, std::vector<uint32_t>(perm, perm + ell));
-  std::vector<Fr> ks(1);
-  memcpy(&ks[0], k, 32);
-  std::vector<cdl_rand*> rands(1, r);
+  const uint32_t ell = L.ell;
+  const std::vector<uint32_t> sel = valid_instances(c, ell, B, perms, status);
+  const uint32_t Bn = (uint32_t)sel.size();
+  if (!Bn) return CDL_OK;
+  const cdl_g1_affine* in[2] = {Rs, Ss};
+  if ((rc = E->load_instances(L, sel, in, 2, nullptr))) return rc;
+  std::vector<std::vector<uint32_t>> pv(Bn);
+  std::vector<Fr> kv(Bn);
+  std::vector<cdl_rand*> rv(Bn);
+  for (uint32_t j = 0; j < Bn; j++) {
+    pv[j].assign(perms + (size_t)sel[j] * ell, perms + ((size_t)sel[j] + 1) * ell);
+    memcpy(&kv[j], ks + sel[j], 32);
+    rv[j] = rands[sel[j]];
+  }
   std::vector<std::vector<Fr>> rsm;
-  if ((rc = E->shuffle_permute_commit(L, 1, perms, ks, rands, rsm))) return rc;
-  cdl_g1_affine m_aff;
-  if ((rc = E->download_points(base + L.Ts, Ts, ell)) || (rc = E->download_points(base + L.Us, Us, ell)) ||
-      (rc = E->download_points(base + L.M, &m_aff, 1)))
-    return rc;
-  affine_to_jac(M, m_aff);
-  memcpy(rs_m, rsm[0].data(), 4 * 32);
+  if ((rc = E->shuffle_permute_commit(L, Bn, pv, kv, rv, rsm))) return rc;
+  // Ts | Us | M of every instance, gathered behind the instance regions and downloaded in one copy
+  const uint32_t tail = L.base(Bn), per = 2 * ell + 1;
+  std::vector<cdl::CopyRange> ranges;
+  for (uint32_t j = 0; j < Bn; j++) {
+    ranges.push_back(cdl::CopyRange{L.base(j) + L.Ts, tail + j * per, 2 * ell, 0});
+    ranges.push_back(cdl::CopyRange{L.base(j) + L.M, tail + j * per + 2 * ell, 1, 0});
+  }
+  std::vector<cdl_g1_affine> out((size_t)Bn * per);
+  if ((rc = E->copy_ranges(ranges)) || (rc = E->download_points(tail, out.data(), out.size()))) return rc;
+  for (uint32_t j = 0; j < Bn; j++) {
+    const size_t b = sel[j];
+    const cdl_g1_affine* o = out.data() + (size_t)j * per;
+    memcpy(Ts + b * ell, o, (size_t)ell * sizeof(cdl_g1_affine));
+    memcpy(Us + b * ell, o + ell, (size_t)ell * sizeof(cdl_g1_affine));
+    affine_to_jac(M + b, o[2 * ell]);
+    memcpy(rs_m + 4 * b, rsm[j].data(), 4 * 32);
+  }
   return CDL_OK;
 }
 
-// ------------------------------------------------------------------ Prove
+int32_t cdl_shuffle_permute_commit(cdl_ctx* c, const cdl_crs* crs, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
+                                   const uint32_t* perm, const cdl_fr* k, cdl_rand* r, cdl_g1_affine* Ts,
+                                   cdl_g1_affine* Us, cdl_g1_jac* M, cdl_fr* rs_m) {
+  int32_t status = CDL_OK;
+  cdl_rand* rr[1] = {r};
+  int32_t rc = cdl_shuffle_permute_commit_batch(c, crs, 1, Rs, Ss, perm, k, rr, Ts, Us, M, rs_m, &status);
+  return rc ? rc : status;
+}
+
+int32_t cdl_prove_batch(cdl_ctx* c, const cdl_crs* crs, size_t B, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
+                        const cdl_g1_affine* Ts, const cdl_g1_affine* Us, const cdl_g1_jac* M, const uint32_t* perms,
+                        const cdl_fr* ks, const cdl_fr* rs_m, cdl_rand* const* rands, uint8_t* proofs,
+                        size_t proof_cap, size_t* proof_lens, int32_t* status) {
+  if (!c || !crs || B == 0 || !Rs || !Ss || !Ts || !Us || !M || !perms || !ks || !rs_m || !rands || !proofs ||
+      !proof_lens || !status || !rands_present(rands, B))
+    return CDL_ERR_INVALID_ARG;
+  if (size_t G = lanes_for(c, B); G > 1) {
+    const size_t e = crs->ell;
+    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_prove_batch(lane, crs, hi - lo, Rs + lo * e, Ss + lo * e, Ts + lo * e, Us + lo * e, M + lo,
+                             perms + lo * e, ks + lo, rs_m + 4 * lo, rands + lo, proofs + lo * proof_cap, proof_cap,
+                             proof_lens + lo, status + lo);
+    });
+  }
+  std::lock_guard<std::mutex> lk(c->mu);
+  Engine* E;
+  Layout L(1);
+  int32_t rc = begin_call(c, crs, B, &E, &L, true);
+  if (rc) return rc;
+  const uint32_t ell = L.ell;
+  const std::vector<uint32_t> sel = valid_instances(c, ell, B, perms, status);
+  const uint32_t Bn = (uint32_t)sel.size();
+  if (!Bn) return CDL_OK;
+  const cdl_g1_affine* in[4] = {Rs, Ss, Ts, Us};
+  if ((rc = E->load_instances(L, sel, in, 4, M))) return rc;
+  std::vector<std::vector<uint32_t>> pv(Bn);
+  std::vector<Fr> kv(Bn);
+  std::vector<std::vector<Fr>> rsm(Bn, std::vector<Fr>(4));
+  std::vector<cdl_rand*> rv(Bn);
+  for (uint32_t j = 0; j < Bn; j++) {
+    pv[j].assign(perms + (size_t)sel[j] * ell, perms + ((size_t)sel[j] + 1) * ell);
+    memcpy(&kv[j], ks + sel[j], 32);
+    memcpy(rsm[j].data(), rs_m + 4 * (size_t)sel[j], 4 * 32);
+    rv[j] = rands[sel[j]];
+  }
+  std::vector<std::vector<uint8_t>> out;
+  std::vector<int32_t> st;
+  std::vector<std::string> errs;
+  std::vector<uint8_t> inst_enc;
+  if (L.n != (1u << L.m)) {  // Engine::prove refuses the whole call; here it is every instance's error
+    for (uint32_t b : sel) status[b] = c->fail(CDL_ERR_PROTOCOL, "cs and ds are not a power of two (ell + 4 = %u)", L.n);
+    return CDL_OK;
+  }
+  if ((rc = E->prove(L, Bn, crs, pv, kv, rsm, rv, out, st, errs, inst_enc, false))) return rc;
+  for (uint32_t j = 0; j < Bn; j++) {
+    const size_t b = sel[j];
+    if (st[j] != CDL_OK) { status[b] = c->fail(st[j], "%s", errs[j].c_str()); continue; }
+    proof_lens[b] = out[j].size();
+    if (out[j].size() > proof_cap) {
+      status[b] = c->fail(CDL_ERR_INVALID_ARG, "proof buffer too small: need %zu bytes", out[j].size());
+      continue;
+    }
+    memcpy(proofs + b * proof_cap, out[j].data(), out[j].size());
+  }
+  return CDL_OK;
+}
+
 int32_t cdl_prove(cdl_ctx* c, const cdl_crs* crs, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
                   const cdl_g1_affine* Ts, const cdl_g1_affine* Us, const cdl_g1_jac* M, const uint32_t* perm,
                   const cdl_fr* k, const cdl_fr* rs_m, cdl_rand* r, uint8_t* proof, size_t proof_cap,
                   size_t* proof_len) {
-  if (!c || !crs || !Rs || !Ss || !Ts || !Us || !M || !perm || !k || !rs_m || !r || !proof || !proof_len)
-    return CDL_ERR_INVALID_ARG;
-  std::lock_guard<std::mutex> lk(c->mu);
-  Engine* E;
-  Layout L(1);
-  int32_t rc = begin_call(c, crs, 1, &E, &L);
-  if (rc) return rc;
-  const uint32_t ell = L.ell, base = L.base(0);
-  for (uint32_t i = 0; i < ell; i++)
-    if (perm[i] >= ell) return c->fail(CDL_ERR_INVALID_ARG, "permutation entry out of range");
-  if ((rc = E->upload_points(base + L.Rs, Rs, ell)) || (rc = E->upload_points(base + L.Ss, Ss, ell)) ||
-      (rc = E->upload_points(base + L.Ts, Ts, ell)) || (rc = E->upload_points(base + L.Us, Us, ell)) ||
-      (rc = E->upload_jac(base + L.M, M, 1)))
-    return rc;
-  std::vector<std::vector<uint32_t>> perms(1, std::vector<uint32_t>(perm, perm + ell));
-  std::vector<Fr> ks(1);
-  memcpy(&ks[0], k, 32);
-  std::vector<std::vector<Fr>> rsm(1, std::vector<Fr>(4));
-  memcpy(rsm[0].data(), rs_m, 4 * 32);
-  std::vector<cdl_rand*> rands(1, r);
-  std::vector<std::vector<uint8_t>> proofs;
-  std::vector<int32_t> status;
-  std::vector<std::string> errs;
-  std::vector<uint8_t> inst_enc;
-  if ((rc = E->prove(L, 1, crs, perms, ks, rsm, rands, proofs, status, errs, inst_enc, false))) return rc;
-  if (status[0] != CDL_OK) return c->fail(status[0], "%s", errs[0].c_str());
-  *proof_len = proofs[0].size();
-  if (proofs[0].size() > proof_cap) return c->fail(CDL_ERR_INVALID_ARG, "proof buffer too small: need %zu bytes", proofs[0].size());
-  memcpy(proof, proofs[0].data(), proofs[0].size());
-  return CDL_OK;
+  int32_t status = CDL_OK;
+  cdl_rand* rr[1] = {r};
+  int32_t rc = cdl_prove_batch(c, crs, 1, Rs, Ss, Ts, Us, M, perm, k, rs_m, rr, proof, proof_cap, proof_len, &status);
+  return rc ? rc : status;
 }
 
 }  // extern "C"
@@ -477,38 +580,76 @@ int32_t load_proofs(Engine* E, const Layout& L, uint32_t B, const uint8_t* const
 
 extern "C" {
 
-int32_t cdl_verify(cdl_ctx* c, const cdl_crs* crs, const uint8_t* proof, size_t proof_len,
-                   const cdl_g1_affine* Rs, const cdl_g1_affine* Ss, const cdl_g1_affine* Ts,
-                   const cdl_g1_affine* Us, const cdl_g1_jac* M, cdl_rand* r, int32_t* ok) {
-  if (!c || !crs || !proof || !Rs || !Ss || !Ts || !Us || !M || !r || !ok) return CDL_ERR_INVALID_ARG;
-  *ok = 0;
+int32_t cdl_verify_batch(cdl_ctx* c, const cdl_crs* crs, size_t B, const uint8_t* proofs, size_t proof_stride,
+                         const size_t* proof_lens, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
+                         const cdl_g1_affine* Ts, const cdl_g1_affine* Us, const cdl_g1_jac* M,
+                         cdl_rand* const* rands, int32_t* ok, int32_t* status) {
+  if (!c || !crs || B == 0 || !proofs || !proof_lens || !Rs || !Ss || !Ts || !Us || !M || !rands || !ok || !status ||
+      !rands_present(rands, B))
+    return CDL_ERR_INVALID_ARG;
+  for (size_t b = 0; b < B; b++) {
+    if (proof_lens[b] > proof_stride) return c->fail(CDL_ERR_INVALID_ARG, "proof %zu is longer than the proof stride", b);
+    ok[b] = 0;
+  }
+  if (size_t G = lanes_for(c, B); G > 1) {
+    const size_t e = crs->ell;
+    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_verify_batch(lane, crs, hi - lo, proofs + lo * proof_stride, proof_stride, proof_lens + lo,
+                              Rs + lo * e, Ss + lo * e, Ts + lo * e, Us + lo * e, M + lo, rands + lo, ok + lo,
+                              status + lo);
+    });
+  }
   std::lock_guard<std::mutex> lk(c->mu);
   Engine* E;
   Layout L(1);
-  int32_t rc = begin_call(c, crs, 1, &E, &L);
+  int32_t rc = begin_call(c, crs, B, &E, &L, true);
   if (rc) return rc;
-  const uint32_t ell = L.ell, base = L.base(0);
-  if ((rc = E->upload_points(base + L.Rs, Rs, ell)) || (rc = E->upload_points(base + L.Ss, Ss, ell)) ||
-      (rc = E->upload_points(base + L.Ts, Ts, ell)) || (rc = E->upload_points(base + L.Us, Us, ell)) ||
-      (rc = E->upload_jac(base + L.M, M, 1)))
-    return rc;
-  std::vector<uint32_t> src(4 * ell + 1);
-  for (uint32_t i = 0; i < 4 * ell; i++) src[i] = base + L.Rs + i;
-  src[4 * ell] = base + L.M;
+  const uint32_t ell = L.ell;
+  std::vector<uint32_t> sel(B);
+  for (size_t b = 0; b < B; b++) sel[b] = (uint32_t)b;
+  const cdl_g1_affine* in[4] = {Rs, Ss, Ts, Us};
+  if ((rc = E->load_instances(L, sel, in, 4, M))) return rc;
+  // transcript encodings Rs | Ss | Ts | Us | M of every instance, in one launch
+  const size_t per = (size_t)4 * ell + 1;
+  std::vector<uint32_t> src(B * per);
+  for (size_t b = 0; b < B; b++) {
+    const uint32_t base = L.base((uint32_t)b);
+    for (uint32_t i = 0; i < 4 * ell; i++) src[b * per + i] = base + L.Rs + i;
+    src[b * per + 4 * ell] = base + L.M;
+  }
   std::vector<uint8_t> inst;
   if ((rc = E->compress(src, inst))) return rc;
-  const uint8_t* m_enc = inst.data() + (size_t)4 * ell * 48;
-  std::vector<const uint8_t*> inst_ptr(1, inst.data());
+  std::vector<const uint8_t*> inst_ptr(B), m_enc(B), proof_ptr(B);
+  for (size_t b = 0; b < B; b++) {
+    inst_ptr[b] = inst.data() + b * per * 48;
+    m_enc[b] = inst_ptr[b] + (size_t)4 * ell * 48;
+    proof_ptr[b] = proofs + b * proof_stride;
+  }
   std::vector<Engine::ParsedProof> pp;
-  if ((rc = load_proofs(E, L, 1, &proof, &proof_len, false, &m_enc, inst_ptr, false, pp))) return rc;
-  if (!pp[0].ok) return c->fail(CDL_ERR_DECODE, "%s", pp[0].err.c_str());
-  std::vector<cdl_rand*> rands(1, r);
-  std::vector<int32_t> verdict, status;
+  if ((rc = load_proofs(E, L, (uint32_t)B, proof_ptr.data(), proof_lens, false, m_enc.data(), inst_ptr, false, pp)))
+    return rc;
+  // a proof that fails to decode is the reference's decode error: Engine::verify makes no draws for it
+  std::vector<uint8_t> decode_failed(B);
+  for (size_t b = 0; b < B; b++) decode_failed[b] = !pp[b].ok;
+  std::vector<cdl_rand*> rv(rands, rands + B);
+  std::vector<int32_t> verdict, st;
   std::vector<std::string> errs;
-  if ((rc = E->verify(L, 1, crs, pp, rands, verdict, status, errs))) return rc;
-  if (status[0] != CDL_OK) return c->fail(status[0], "%s", errs[0].c_str());
-  *ok = verdict[0];
+  if ((rc = E->verify(L, (uint32_t)B, crs, pp, rv, verdict, st, errs))) return rc;
+  for (size_t b = 0; b < B; b++) {
+    status[b] = decode_failed[b] ? CDL_ERR_DECODE : st[b];
+    if (status[b] != CDL_OK) c->fail(status[b], "%s", errs[b].c_str());
+    else ok[b] = verdict[b];
+  }
   return CDL_OK;
+}
+
+int32_t cdl_verify(cdl_ctx* c, const cdl_crs* crs, const uint8_t* proof, size_t proof_len,
+                   const cdl_g1_affine* Rs, const cdl_g1_affine* Ss, const cdl_g1_affine* Ts,
+                   const cdl_g1_affine* Us, const cdl_g1_jac* M, cdl_rand* r, int32_t* ok) {
+  int32_t status = CDL_OK;
+  cdl_rand* rr[1] = {r};
+  int32_t rc = cdl_verify_batch(c, crs, 1, proof, proof_len, &proof_len, Rs, Ss, Ts, Us, M, rr, ok, &status);
+  return rc ? rc : status;
 }
 
 // ------------------------------------------------------------------ Whisk

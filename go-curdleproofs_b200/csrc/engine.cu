@@ -69,7 +69,8 @@ Engine::~Engine() {
   if (d_win_) cudaFree(d_win_);
   if (d_match_) cudaFree(d_match_);
   if (d_bv_) cudaFree(d_bv_);
-  for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_, &s_bv_}) {
+  for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_, &s_bv_,
+                     &s_in_}) {
     if (s->h) cudaFreeHost(s->h);
     if (s->d) cudaFree(s->d);
   }
@@ -180,21 +181,6 @@ int32_t Engine::upload_points(uint32_t dst, const void* host_affine, size_t coun
   return CDL_OK;
 }
 
-int32_t Engine::upload_jac(uint32_t dst, const void* host_jac, size_t count) {
-  if (!count) return CDL_OK;
-  int32_t rc = reserve(s_jac_, count * sizeof(cdl::G1Jac));
-  if (rc) return rc;
-  memcpy(s_jac_.h, host_jac, count * sizeof(cdl::G1Jac));
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_jac_.d, s_jac_.h, count * sizeof(cdl::G1Jac), cudaMemcpyHostToDevice, ctx_->stream));
-  tick();
-  cdl::launch_jac_to_affine((const cdl::G1Jac*)s_jac_.d, d_pool_ + dst, (int)count, ctx_->stream);
-  tock(3, 0, 240.0 * count);
-  CDL_CUDA(ctx_, cudaGetLastError());
-  CDL_CUDA(ctx_, ctx_->sync_stream());
-  finish_timing();
-  return CDL_OK;
-}
-
 int32_t Engine::download_points(uint32_t src, void* host_affine, size_t count) {
   if (!count) return CDL_OK;
   CDL_CUDA(ctx_, cudaMemcpyAsync(host_affine, d_pool_ + src, count * sizeof(G1Affine), cudaMemcpyDeviceToHost, ctx_->stream));
@@ -238,6 +224,47 @@ struct ProfScope {
   ~ProfScope() { acc += Engine::now() - t0; }
 };
 }  // namespace
+
+int32_t Engine::load_instances(const Layout& L, const std::vector<uint32_t>& sel, const cdl_g1_affine* const* pts,
+                               uint32_t npts, const cdl_g1_jac* M) {
+  ProfScope ps(prof.gpu);
+  const size_t B = sel.size(), per = (size_t)npts * L.ell;
+  if (!B) return CDL_OK;
+  const uint32_t tail = L.base((uint32_t)B), tail_m = tail + (uint32_t)(B * per);
+  int32_t rc;
+  if ((rc = reserve(s_in_, B * per * sizeof(G1Affine))) || (M && (rc = reserve(s_jac_, B * sizeof(cdl::G1Jac)))))
+    return rc;
+  {
+    ProfScope pc(prof.copy);
+    G1Affine* h = (G1Affine*)s_in_.h;
+    pool_.parallel_for(B, std::function<void(size_t)>([&](size_t j) {
+      for (uint32_t a = 0; a < npts; a++)
+        memcpy(h + j * per + (size_t)a * L.ell, pts[a] + (size_t)sel[j] * L.ell, (size_t)L.ell * sizeof(G1Affine));
+    }));
+    if (M)
+      for (size_t j = 0; j < B; j++) memcpy((cdl::G1Jac*)s_jac_.h + j, M + sel[j], sizeof(cdl::G1Jac));
+  }
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_ + tail, s_in_.h, B * per * sizeof(G1Affine), cudaMemcpyHostToDevice, ctx_->stream));
+  if (M) {
+    CDL_CUDA(ctx_, cudaMemcpyAsync(s_jac_.d, s_jac_.h, B * sizeof(cdl::G1Jac), cudaMemcpyHostToDevice, ctx_->stream));
+    tick();
+    cdl::launch_jac_to_affine((const cdl::G1Jac*)s_jac_.d, d_pool_ + tail_m, (int)B, ctx_->stream);
+    tock(3, 0, 240.0 * B);
+    CDL_CUDA(ctx_, cudaGetLastError());
+  }
+  std::vector<cdl::CopyRange> ranges;
+  ranges.reserve(M ? 2 * B : B);
+  for (size_t j = 0; j < B; j++) {
+    const uint32_t base = L.base((uint32_t)j);
+    ranges.push_back(cdl::CopyRange{tail + (uint32_t)(j * per), base + L.Rs, (uint32_t)per, 0});
+    if (M) ranges.push_back(cdl::CopyRange{tail_m + (uint32_t)j, base + L.M, 1, 0});
+  }
+  // copy_ranges waits for the stream before it refills its descriptors, so the staging buffers are free and
+  // the normalisation's events complete when it returns; the copy itself is ordered before the next stage
+  if ((rc = copy_ranges(ranges))) return rc;
+  finish_timing();
+  return CDL_OK;
+}
 
 int32_t Engine::compress(const std::vector<uint32_t>& src, std::vector<uint8_t>& out48) {
   ProfScope ps(prof.gpu);

@@ -137,11 +137,18 @@ class Engine {
   void select_fixed(const Layout& L, const cdl_crs* crs, size_t B);
   void clear_fixed() { fixed_ = cdl::FixedTable(); }  // calls whose pool does not start with a CRS image
   int32_t upload_points(uint32_t dst, const void* host_affine, size_t count);
-  int32_t upload_jac(uint32_t dst, const void* host_jac, size_t count);  // normalises to affine on the device
   int32_t download_points(uint32_t src, void* host_affine, size_t count);
   int32_t copy_points(uint32_t dst, uint32_t src, size_t count);
   int32_t set_infinity(uint32_t dst, size_t count);
   int32_t copy_ranges(const std::vector<cdl::CopyRange>& ranges);  // many pool-to-pool copies in one launch
+  // Instance intake of the batched C ABI calls: instance j of the engine call is the caller's instance sel[j].
+  // pts[a] + sel[j] * ell (a < npts: Rs, Ss[, Ts, Us]) go to pool[base(j) + a * ell ..) and, when M is given,
+  // M[sel[j]] (gnark G1Jac) to pool[base(j) + M].  One pinned host-to-device copy into the pool behind the
+  // instance regions, one normalisation of every M and one copy_ranges launch, so the pool must hold
+  // base(sel.size()) + intake_points(L, sel.size()) points.
+  int32_t load_instances(const Layout& L, const std::vector<uint32_t>& sel, const cdl_g1_affine* const* pts,
+                         uint32_t npts, const cdl_g1_jac* M);
+  static size_t intake_points(const Layout& L, size_t B) { return B * ((size_t)4 * L.ell + 1); }
   int32_t compress(const std::vector<uint32_t>& src, std::vector<uint8_t>& out48);
   int32_t decompress(const uint8_t* enc48, const std::vector<uint32_t>& dst, std::vector<uint8_t>& status);
   // `before` (optional) runs on the stream after the stage's indices / scalars reached the device and before
@@ -224,7 +231,8 @@ class Engine {
     void* d = nullptr;
     size_t cap = 0;
   };
-  Staging s_idx_, s_sc_, s_task_, s_out_, s_ops_, s_enc_, s_st_, s_jac_, s_sub_, s_t2_, s_cr_, s_fsub_, s_vs_, s_as_, s_bv_;
+  Staging s_idx_, s_sc_, s_task_, s_out_, s_ops_, s_enc_, s_st_, s_jac_, s_sub_, s_t2_, s_cr_, s_fsub_, s_vs_, s_as_, s_bv_,
+      s_in_;
   int32_t reserve(Staging& s, size_t bytes);
   void tick();                                   // event before a kernel
   void tock(int cls, double modmul, double bytes);  // event after; call finish_timing() after the sync

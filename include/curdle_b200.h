@@ -174,6 +174,31 @@ int32_t cdl_verify(cdl_ctx* ctx, const cdl_crs* crs, const uint8_t* proof, size_
                    const cdl_g1_affine* Rs, const cdl_g1_affine* Ss, const cdl_g1_affine* Ts,
                    const cdl_g1_affine* Us, const cdl_g1_jac* M, cdl_rand* r, int32_t* ok);
 
+/* Batched forms of the three calls above: B caller-supplied instances in lock step, one GPU launch per
+ * protocol stage for the whole batch, cut into lanes (cdl_set_lanes) as the Whisk batch calls are.
+ * Arrays are instance-major: Rs, Ss, Ts, Us and perms hold B x ell entries; ks, M, rands, status, ok and
+ * proof_lens B entries; rs_m B x 4.  Proof b is at proofs + b * proof_cap (proof_stride for verification,
+ * where proof_lens[b] <= proof_stride).  For every instance b the batch gives what the single call gives on
+ * the same inputs: the same outputs, status[b] equal to the single call's return code and the same position
+ * of rands[b] afterwards.  An instance whose status is not CDL_OK leaves its outputs as they were, except
+ * proof_lens[b] when the proof did not fit proof_cap; an instance with a permutation entry >= ell or a
+ * proof that fails to decode draws nothing from its Rand.  Returns CDL_OK when the arguments are valid,
+ * whatever the per-instance statuses (cdl_last_error then holds a failing instance's message);
+ * CDL_ERR_INVALID_ARG for a null pointer, B == 0 or a CRS of another context; CDL_ERR_TOO_LARGE when one
+ * lane's instances would need 2^30 or more pool points (about 150 000 instances at ell = 508). */
+int32_t cdl_shuffle_permute_commit_batch(cdl_ctx* ctx, const cdl_crs* crs, size_t B, const cdl_g1_affine* Rs,
+                                         const cdl_g1_affine* Ss, const uint32_t* perms, const cdl_fr* ks,
+                                         cdl_rand* const* rands, cdl_g1_affine* Ts, cdl_g1_affine* Us, cdl_g1_jac* M,
+                                         cdl_fr* rs_m, int32_t* status);
+int32_t cdl_prove_batch(cdl_ctx* ctx, const cdl_crs* crs, size_t B, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
+                        const cdl_g1_affine* Ts, const cdl_g1_affine* Us, const cdl_g1_jac* M, const uint32_t* perms,
+                        const cdl_fr* ks, const cdl_fr* rs_m, cdl_rand* const* rands, uint8_t* proofs,
+                        size_t proof_cap, size_t* proof_lens, int32_t* status);
+int32_t cdl_verify_batch(cdl_ctx* ctx, const cdl_crs* crs, size_t B, const uint8_t* proofs, size_t proof_stride,
+                         const size_t* proof_lens, const cdl_g1_affine* Rs, const cdl_g1_affine* Ss,
+                         const cdl_g1_affine* Ts, const cdl_g1_affine* Us, const cdl_g1_jac* M,
+                         cdl_rand* const* rands, int32_t* ok, int32_t* status);
+
 /* whisk.GenerateWhiskShuffleProof (whisk/whisk.go:63-114).  Trackers are
  * 96-byte {rG, krG} pairs; crs ell trackers in, ell out; proof is zero padded
  * to proof_cap (4576 for the reference's N = 128). */

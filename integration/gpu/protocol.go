@@ -191,3 +191,97 @@ func (c *Context) MatchWhiskTrackers(trackers []byte, ks []fr.Element) (owner, s
 	}
 	return owner, status, nil
 }
+
+func randHandles(rands []*Rand) **C.cdl_rand {
+	hs := make([]*C.cdl_rand, len(rands))
+	for i, r := range rands {
+		hs[i] = r.h
+	}
+	return (**C.cdl_rand)(unsafe.Pointer(&hs[0]))
+}
+
+// ShufflePermuteCommitBatch is common.ShufflePermuteCommit (common/util.go:45-88) for B = len(rands) caller
+// instances in lock step: Rs, Ss and perms hold B*ell entries (instance-major), ks one scalar per instance.
+// status[b] is what the single call would return for instance b (CDL_ERR_INVALID_ARG for a permutation
+// entry out of range, in which case rands[b] draws nothing).
+func (c *Context) ShufflePermuteCommitBatch(crs *CRS, Rs, Ss []bls12381.G1Affine, perms []uint32, ks []fr.Element,
+	rands []*Rand) (Ts, Us []bls12381.G1Affine, M []bls12381.G1Jac, rsM []fr.Element, status []int32, err error) {
+	B := len(rands)
+	if B == 0 || len(Rs) != B*crs.Ell || len(Ss) != B*crs.Ell || len(perms) != B*crs.Ell || len(ks) != B {
+		return nil, nil, nil, nil, nil, errStatus(C.int32_t(C.CDL_ERR_INVALID_ARG))
+	}
+	Ts = make([]bls12381.G1Affine, len(Rs))
+	Us = make([]bls12381.G1Affine, len(Rs))
+	M = make([]bls12381.G1Jac, B)
+	rsM = make([]fr.Element, 4*B)
+	status = make([]int32, B)
+	rc := C.cdl_shuffle_permute_commit_batch(c.h, crs.h, C.size_t(B), affPtr(Rs), affPtr(Ss),
+		(*C.uint32_t)(unsafe.Pointer(&perms[0])), frPtr(ks), randHandles(rands), affPtr(Ts), affPtr(Us),
+		(*C.cdl_g1_jac)(unsafe.Pointer(&M[0])), frPtr(rsM), (*C.int32_t)(unsafe.Pointer(&status[0])))
+	if rc != 0 {
+		return nil, nil, nil, nil, nil, c.err(rc)
+	}
+	return
+}
+
+// ProveBatch is curdleproof.Prove + Proof.Serialize for B = len(rands) caller instances in lock step (arrays
+// as in ShufflePermuteCommitBatch, rsM 4 per instance).  proofs[b] is nil unless status[b] == 0.
+func (c *Context) ProveBatch(crs *CRS, Rs, Ss, Ts, Us []bls12381.G1Affine, M []bls12381.G1Jac, perms []uint32,
+	ks, rsM []fr.Element, rands []*Rand) (proofs [][]byte, status []int32, err error) {
+	B := len(rands)
+	n := B * crs.Ell
+	if B == 0 || len(Rs) != n || len(Ss) != n || len(Ts) != n || len(Us) != n || len(M) != B || len(perms) != n ||
+		len(ks) != B || len(rsM) != 4*B {
+		return nil, nil, errStatus(C.int32_t(C.CDL_ERR_INVALID_ARG))
+	}
+	const proofCap = 48*(18+10*32) + 32*7 + 40
+	buf := make([]byte, B*proofCap)
+	lens := make([]C.size_t, B)
+	status = make([]int32, B)
+	rc := C.cdl_prove_batch(c.h, crs.h, C.size_t(B), affPtr(Rs), affPtr(Ss), affPtr(Ts), affPtr(Us),
+		(*C.cdl_g1_jac)(unsafe.Pointer(&M[0])), (*C.uint32_t)(unsafe.Pointer(&perms[0])), frPtr(ks), frPtr(rsM),
+		randHandles(rands), (*C.uint8_t)(unsafe.Pointer(&buf[0])), C.size_t(proofCap), &lens[0],
+		(*C.int32_t)(unsafe.Pointer(&status[0])))
+	if rc != 0 {
+		return nil, nil, c.err(rc)
+	}
+	proofs = make([][]byte, B)
+	for b := range proofs {
+		if status[b] == 0 {
+			proofs[b] = buf[b*proofCap : b*proofCap+int(lens[b])]
+		}
+	}
+	return proofs, status, nil
+}
+
+// VerifyBatch is Proof.FromReader + curdleproof.Verify for B = len(rands) caller instances in lock step:
+// ok[b] is the reference's bool and status[b] its error (what Verify would return for instance b).
+func (c *Context) VerifyBatch(crs *CRS, proofs [][]byte, Rs, Ss, Ts, Us []bls12381.G1Affine, M []bls12381.G1Jac,
+	rands []*Rand) (ok, status []int32, err error) {
+	B := len(rands)
+	n := B * crs.Ell
+	if B == 0 || len(proofs) != B || len(Rs) != n || len(Ss) != n || len(Ts) != n || len(Us) != n || len(M) != B {
+		return nil, nil, errStatus(C.int32_t(C.CDL_ERR_INVALID_ARG))
+	}
+	stride := 1
+	for _, p := range proofs {
+		if len(p) > stride {
+			stride = len(p)
+		}
+	}
+	buf := make([]byte, B*stride)
+	lens := make([]C.size_t, B)
+	for b, p := range proofs {
+		copy(buf[b*stride:], p)
+		lens[b] = C.size_t(len(p))
+	}
+	ok = make([]int32, B)
+	status = make([]int32, B)
+	rc := C.cdl_verify_batch(c.h, crs.h, C.size_t(B), (*C.uint8_t)(unsafe.Pointer(&buf[0])), C.size_t(stride), &lens[0],
+		affPtr(Rs), affPtr(Ss), affPtr(Ts), affPtr(Us), (*C.cdl_g1_jac)(unsafe.Pointer(&M[0])), randHandles(rands),
+		(*C.int32_t)(unsafe.Pointer(&ok[0])), (*C.int32_t)(unsafe.Pointer(&status[0])))
+	if rc != 0 {
+		return nil, nil, c.err(rc)
+	}
+	return ok, status, nil
+}
