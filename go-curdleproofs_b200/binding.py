@@ -51,6 +51,8 @@ def load_library():
     vp, sz, i32, u32p = C.c_void_p, C.c_size_t, C.c_int32, C.POINTER(C.c_uint32)
     lib.cdl_abi_version.restype = C.c_uint32
     lib.cdl_create.argtypes = [C.c_int, C.POINTER(vp)]
+    lib.cdl_create_devices.argtypes = [C.POINTER(C.c_int32), sz, C.POINTER(vp)]
+    lib.cdl_context_devices.argtypes = [vp, C.POINTER(C.c_int32), sz, C.POINTER(sz)]
     lib.cdl_destroy.argtypes = [vp]
     lib.cdl_destroy.restype = None
     lib.cdl_last_error.argtypes = [vp]
@@ -100,6 +102,7 @@ def load_library():
     lib.cdl_host_selftest_fibers.argtypes = [C.c_uint32, C.c_uint32, vp, C.POINTER(C.c_int32)]
     lib.cdl_engine_stats.argtypes = [vp, vp, vp, vp, vp, C.c_int]
     lib.cdl_engine_busy_ms.argtypes = [vp, C.POINTER(C.c_double)]
+    lib.cdl_engine_busy_ms_device.argtypes = [vp, sz, C.POINTER(C.c_double)]
     lib.cdl_set_lanes.argtypes = [vp, i32]
     lib.cdl_launch_count.argtypes = [vp]
     lib.cdl_launch_count.restype = u64
@@ -133,12 +136,17 @@ def load_library():
 
 
 class Context:
-    """One CUDA device; mirrors cdl_ctx."""
+    """One CUDA device, or with `devices` a list of them whose batched calls are split over the GPUs
+    (cdl_create_devices); mirrors cdl_ctx."""
 
-    def __init__(self, device: int = 0):
+    def __init__(self, device: int = 0, devices=None):
         self.lib = load_library()
         h = C.c_void_p()
-        rc = self.lib.cdl_create(device, C.byref(h))
+        if devices is None:
+            rc = self.lib.cdl_create(device, C.byref(h))
+        else:
+            devs = list(devices)
+            rc = self.lib.cdl_create_devices((C.c_int32 * max(1, len(devs)))(*devs), len(devs), C.byref(h))
         if rc != 0:
             raise CdlError(rc, "cdl_create failed (no CUDA device? this library has no CPU fallback)")
         self.h = h
@@ -635,6 +643,22 @@ def _ctx_engine_busy_ms(self) -> float:
     return v.value
 
 
+def _ctx_engine_busy_ms_device(self, slot: int) -> float:
+    """Busy time of device slot `slot` since the last stats reset."""
+    v = C.c_double()
+    self._chk(self.lib.cdl_engine_busy_ms_device(self.h, slot, C.byref(v)))
+    return v.value
+
+
+def _ctx_devices(self):
+    """The context's device list (one entry per device slot)."""
+    n = C.c_size_t()
+    self._chk(self.lib.cdl_context_devices(self.h, None, 0, C.byref(n)))
+    out = (C.c_int32 * max(1, n.value))()
+    self._chk(self.lib.cdl_context_devices(self.h, out, n.value, C.byref(n)))
+    return list(out)[:n.value]
+
+
 def _ctx_set_lanes(self, lanes: int):
     self._chk(self.lib.cdl_set_lanes(self.h, lanes))
 
@@ -675,5 +699,7 @@ Context.whisk_is_valid_tracker_proof_batch = _ctx_whisk_is_valid_tracker_proof_b
 Context.whisk_match_trackers = _ctx_whisk_match_trackers
 Context.launch_count = _ctx_launch_count
 Context.engine_busy_ms = _ctx_engine_busy_ms
+Context.engine_busy_ms_device = _ctx_engine_busy_ms_device
+Context.devices = _ctx_devices
 Context.set_lanes = _ctx_set_lanes
 Context.engine_stats = _ctx_engine_stats

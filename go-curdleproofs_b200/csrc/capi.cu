@@ -32,15 +32,20 @@ static bool msm_tasks(const uint32_t* offsets, size_t k, std::vector<MsmTask>& t
 
 extern "C" {
 
-uint32_t cdl_abi_version(void) { return (1u << 16) | 7u; }
+uint32_t cdl_abi_version(void) { return (1u << 16) | 8u; }
 
-int32_t cdl_create(int device, cdl_ctx** out) {
+void cdl_destroy(cdl_ctx* c);
+
+int32_t cdl_create_devices(const int32_t* devices, size_t n, cdl_ctx** out) {
   if (!out) return CDL_ERR_INVALID_ARG;
   *out = nullptr;
+  if (!devices || n == 0 || n > 16) return CDL_ERR_INVALID_ARG;
   int count = 0;
   cudaError_t e = cudaGetDeviceCount(&count);
   if (e != cudaSuccess || count == 0) return CDL_ERR_NO_DEVICE;
-  if (device < 0 || device >= count) return CDL_ERR_INVALID_ARG;
+  for (size_t s = 0; s < n; s++)
+    if (devices[s] < 0 || devices[s] >= count) return CDL_ERR_INVALID_ARG;
+  const int device = devices[0];
   cdl_ctx* c = new cdl_ctx();
   c->device = device;
   if (cudaSetDevice(device) != cudaSuccess || cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) {
@@ -54,34 +59,63 @@ int32_t cdl_create(int device, cdl_ctx** out) {
   c->name = prop.name;
   cudaEventCreate(&c->ev0);
   cudaEventCreate(&c->ev1);
-  cudaEventCreate(&c->base_ev);
-  cudaEventRecord(c->base_ev, c->stream);
-  cudaStreamSynchronize(c->stream);
-  // the small-MSM kernel stages up to ~6000 terms in shared memory
-  msm_small_init();
+  c->slots.resize(n);
+  for (size_t s = 0; s < n; s++) {
+    cdl_ctx::Slot& sl = c->slots[s];
+    sl.device = devices[s];
+    if (cudaSetDevice(sl.device) != cudaSuccess || cudaEventCreate(&sl.base_ev) != cudaSuccess) {
+      cdl_destroy(c);
+      return CDL_ERR_CUDA;
+    }
+    // slot 0's timeline starts on the root stream; the others on their device's default stream
+    cudaEventRecord(sl.base_ev, s == 0 ? c->stream : 0);
+    cudaEventSynchronize(sl.base_ev);
+    // the small-MSM kernel stages up to ~6000 terms in shared memory (a per-device kernel attribute)
+    msm_small_init();
+  }
+  cudaSetDevice(device);
   if (const char* e = getenv("CDL_MSM_C")) c->msm_c_override = atoi(e);
   if (const char* e = getenv("CDL_LANES")) { int v = atoi(e); if (v >= 1 && v <= 16) c->n_lanes = v; }
   *out = c;
   return CDL_OK;
 }
 
-// lane context `i` of a root context (created on first use; caller holds the root's mutex)
-cdl_ctx* cdl_lane_(cdl_ctx* root, size_t i) {
-  while (root->lanes.size() <= i) {
+int32_t cdl_create(int device, cdl_ctx** out) {
+  const int32_t d = device;
+  return cdl_create_devices(&d, 1, out);
+}
+
+int32_t cdl_context_devices(cdl_ctx* c, int32_t* devices, size_t cap, size_t* n) {
+  if (!c || !n || (cap && !devices)) return CDL_ERR_INVALID_ARG;
+  const std::vector<cdl_ctx::Slot>& sl = c->root()->slots;
+  *n = sl.size();
+  for (size_t s = 0; s < sl.size() && s < cap; s++) devices[s] = sl[s].device;
+  return CDL_OK;
+}
+
+// lane context `i` of slot `slot` of a root context (created on first use; caller holds the root's mutex)
+cdl_ctx* cdl_lane_(cdl_ctx* root, size_t slot, size_t i) {
+  cdl_ctx::Slot& sl = root->slots[slot];
+  while (sl.lanes.size() <= i) {
     cdl_ctx* l = new cdl_ctx();
-    l->device = root->device;
-    l->sm_count = root->sm_count;
+    l->device = sl.device;
+    l->dev_slot = slot;
     l->clock_khz = root->clock_khz;
     l->name = root->name;
     l->parent = root;
     l->n_lanes = 1;
     l->msm_c_override = root->msm_c_override;
-    if (cudaStreamCreateWithFlags(&l->stream, cudaStreamNonBlocking) != cudaSuccess) { delete l; return nullptr; }
+    cudaDeviceGetAttribute(&l->sm_count, cudaDevAttrMultiProcessorCount, l->device);
+    if (cudaSetDevice(l->device) != cudaSuccess ||
+        cudaStreamCreateWithFlags(&l->stream, cudaStreamNonBlocking) != cudaSuccess) {
+      delete l;
+      return nullptr;
+    }
     cudaEventCreate(&l->ev0);
     cudaEventCreate(&l->ev1);
-    root->lanes.push_back(l);
+    sl.lanes.push_back(l);
   }
-  return root->lanes[i];
+  return sl.lanes[i];
 }
 
 int32_t cdl_set_lanes(cdl_ctx* c, int32_t lanes) {
@@ -98,13 +132,17 @@ void cdl_destroy(cdl_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   cdl_comm_destroy(c);
-  for (cdl_ctx* l : c->lanes) cdl_destroy(l);
-  c->lanes.clear();
+  for (cdl_ctx::Slot& sl : c->slots) {
+    for (cdl_ctx* l : sl.lanes) cdl_destroy(l);
+    sl.lanes.clear();
+    cudaSetDevice(sl.device);
+    if (sl.base_ev) cudaEventDestroy(sl.base_ev);
+  }
+  cudaSetDevice(c->device);
   if (c->engine) cdl_engine_free_(c->engine);
   c->free_all();
   cudaEventDestroy(c->ev0);
   cudaEventDestroy(c->ev1);
-  if (c->base_ev) cudaEventDestroy(c->base_ev);
   if (c->ev_sync) cudaEventDestroy(c->ev_sync);
   cudaStreamDestroy(c->stream);
   delete c;

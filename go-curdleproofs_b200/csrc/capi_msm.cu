@@ -220,8 +220,12 @@ int32_t cdl_comm_unique_id(uint8_t* id128) {
 
 int32_t cdl_comm_init(cdl_ctx* c, const uint8_t* id128, int32_t rank, int32_t world) {
   if (!c || !id128 || world < 1 || rank < 0 || rank >= world) return CDL_ERR_INVALID_ARG;
-  NcclApi* a = nccl_api();
   std::lock_guard<std::mutex> lk(c->mu);
+  // the sharded MSM runs one process (one single-device context) per GPU
+  if (c->root()->slots.size() > 1)
+    return c->fail(CDL_ERR_INVALID_ARG, "comm_init: a context with %zu device slots cannot join a communicator",
+                   c->root()->slots.size());
+  NcclApi* a = nccl_api();
   if (!a->err.empty()) return c->fail(CDL_ERR_NO_DEVICE, "NCCL unavailable: %s", a->err.c_str());
   CDL_CUDA(c, cudaSetDevice(c->device));
   if (c->nccl_comm) { a->CommDestroy((ncclComm_t)c->nccl_comm); c->nccl_comm = nullptr; }

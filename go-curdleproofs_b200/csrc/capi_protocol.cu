@@ -15,10 +15,12 @@ using cdlh::Engine;
 using cdlh::engine_of;
 using cdlh::Fr;
 using cdlh::Layout;
+using cdlh::run_split;
+using cdlh::slots_for;
 
 static_assert(sizeof(Fr) == sizeof(cdl_fr), "host fr layout");
 
-extern "C" cdl_ctx* cdl_lane_(cdl_ctx* root, size_t i);  // capi.cu
+extern "C" cdl_ctx* cdl_lane_(cdl_ctx* root, size_t slot, size_t i);  // capi.cu
 
 namespace {
 
@@ -37,6 +39,22 @@ Engine* cdlh::engine_of(cdl_ctx* c) {
   Engine* E = static_cast<Engine*>(c->engine);
   E->clear_fixed();  // begin_call selects the tables of its CRS; every other call runs without
   return E;
+}
+
+const cdl::G1Affine* cdl_crs::points_on(size_t s) const {
+  Replica& r = rep[s];
+  if (r.d_points) return r.d_points;
+  const size_t bytes = host.size() * sizeof(cdl::G1Affine);
+  if (cudaMalloc(&r.d_points, bytes) != cudaSuccess) {
+    cudaGetLastError();
+    r.d_points = nullptr;
+    return nullptr;
+  }
+  if (cudaMemcpy(r.d_points, host.data(), bytes, cudaMemcpyHostToDevice) != cudaSuccess) {
+    cudaFree(r.d_points);
+    r.d_points = nullptr;
+  }
+  return r.d_points;
 }
 
 void cdlh::affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a) {
@@ -72,24 +90,21 @@ int32_t put_generator(Engine* E, uint32_t slot) {
   return E->upload_points(slot, &g, 1);
 }
 
-// finish a CRS object from pool[0 .. ell+9): copies the image to its own device buffer, caches encodings
+// finish a CRS object from pool[0 .. ell+9): keeps the host image, copies it to slot 0's device buffer (the
+// other slots upload theirs on first use), caches encodings
 int32_t crs_finish(cdl_ctx* c, Engine* E, const Layout& L, cdl_crs** out) {
   std::unique_ptr<cdl_crs> crs(new cdl_crs());
   crs->ctx = c;
   crs->ell = L.ell;
+  crs->rep.resize(c->slots.size());
   int32_t rc = E->set_infinity(L.INF, 1);
   if (rc) return rc;
-  if (cudaMalloc(&crs->d_points, (size_t)L.crs_size * sizeof(cdl::G1Affine)) != cudaSuccess)
-    return c->fail(CDL_ERR_CUDA, "crs allocation failed");
   std::vector<uint32_t> src(L.crs_size);
   for (uint32_t i = 0; i < L.crs_size; i++) src[i] = i;
-  if ((rc = E->compress(src, crs->enc))) { cudaFree(crs->d_points); return rc; }
-  std::vector<cdl_g1_affine> tmp(L.crs_size);
-  if ((rc = E->download_points(0, tmp.data(), L.crs_size))) { cudaFree(crs->d_points); return rc; }
-  if (cudaMemcpy(crs->d_points, tmp.data(), (size_t)L.crs_size * sizeof(cdl::G1Affine), cudaMemcpyHostToDevice) != cudaSuccess) {
-    cudaFree(crs->d_points);
-    return c->fail(CDL_ERR_CUDA, "crs upload failed");
-  }
+  if ((rc = E->compress(src, crs->enc))) return rc;
+  crs->host.resize(L.crs_size);
+  if ((rc = E->download_points(0, crs->host.data(), L.crs_size))) return rc;
+  if (!crs->points_on(0)) return c->fail(CDL_ERR_CUDA, "crs upload failed");
   *out = crs.release();
   return CDL_OK;
 }
@@ -120,36 +135,86 @@ int32_t begin_call(cdl_ctx* c, const cdl_crs* crs, size_t B, Engine** E, Layout*
 
 constexpr size_t kMinLaneBatch = 32;  // below this a sub-batch no longer fills its launches
 
-// number of lanes a batch of B instances is cut into
-size_t lanes_for(cdl_ctx* c, size_t B) {
-  if (c->parent || c->n_lanes <= 1) return 1;
-  return std::max<size_t>(1, std::min<size_t>((size_t)c->n_lanes, B / kMinLaneBatch));
+// number of lanes a slot's block of n instances is cut into
+size_t lanes_for(cdl_ctx* c, size_t n) {
+  if (c->n_lanes <= 1) return 1;
+  return std::max<size_t>(1, std::min<size_t>((size_t)c->n_lanes, n / kMinLaneBatch));
 }
 
-// runs fn(lane ctx, lo, hi) for contiguous sub-batches [lo, hi) concurrently, one host thread per lane
-int32_t run_lanes(cdl_ctx* c, size_t B, size_t G, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn) {
+}  // namespace
+
+size_t cdlh::slots_for(cdl_ctx* c, size_t B) {
+  if (c->parent) return 1;
+  return std::max<size_t>(1, std::min<size_t>(c->slots.size(), B / kMinLaneBatch));
+}
+
+// first unit of block s when B units are dealt to D slots in contiguous blocks (sharding.shard_bounds)
+static size_t shard_lo(size_t B, size_t D, size_t s) { return s * (B / D) + std::min(s, B % D); }
+
+int32_t cdlh::run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes,
+                        size_t align) {
   std::lock_guard<std::mutex> lk(c->mu);
-  CDL_CUDA(c, cudaSetDevice(c->device));
-  std::vector<cdl_ctx*> lane(G);
-  for (size_t g = 0; g < G; g++)
-    if (!(lane[g] = cdl_lane_(c, g))) return c->fail(CDL_ERR_CUDA, "lane context creation failed");
-  std::vector<int32_t> rc(G, CDL_OK);
-  std::vector<std::thread> th;
-  for (size_t g = 0; g < G; g++) {
-    size_t lo = B * g / G, hi = B * (g + 1) / G;
-    th.emplace_back([&, g, lo, hi] { rc[g] = fn(lane[g], lo, hi); });
+  struct Piece { cdl_ctx* ctx; size_t lo, hi; };
+  std::vector<Piece> pieces;
+  const size_t D = slots_for(c, B);
+  auto bound = [&](size_t s) {
+    if (s == D) return B;
+    return std::min(B, (shard_lo(B, D, s) + align / 2) / align * align);
+  };
+  for (size_t s = 0; s < D; s++) {
+    const size_t lo = bound(s), n = bound(s + 1) - lo;
+    if (!n) continue;
+    const size_t G = lanes ? lanes_for(c, n) : 1;
+    for (size_t g = 0; g < G; g++) {
+      cdl_ctx* l = cdl_lane_(c, s, g);
+      if (!l) return c->fail(CDL_ERR_CUDA, "lane context creation failed");
+      pieces.push_back(Piece{l, lo + n * g / G, lo + n * (g + 1) / G});
+    }
   }
+  CDL_CUDA(c, cudaSetDevice(c->device));
+  std::vector<int32_t> rc(pieces.size(), CDL_OK);
+  std::vector<std::thread> th;
+  for (size_t i = 0; i < pieces.size(); i++)
+    th.emplace_back([&, i] { rc[i] = fn(pieces[i].ctx, pieces[i].lo, pieces[i].hi); });
   for (auto& t : th) t.join();
-  for (size_t g = 0; g < G; g++)
-    if (rc[g] != CDL_OK) return c->fail(rc[g], "%s", lane[g]->err.c_str());
+  for (size_t i = 0; i < pieces.size(); i++)
+    if (rc[i] != CDL_OK) return c->fail(rc[i], "%s", pieces[i].ctx->err.c_str());
   return CDL_OK;
 }
 
+namespace {
+
+// whether a batched protocol call of B instances on c is cut into pieces (run_split) rather than run on c itself
+bool split_lanes(cdl_ctx* c, size_t B) { return !c->parent && (cdlh::slots_for(c, B) > 1 || lanes_for(c, B) > 1); }
+
+// f(engine, slot) for every engine of a root context: its own (slot 0) and its lanes'
 template <class F>
 void for_each_engine(cdl_ctx* c, F f) {
-  if (c->engine) f(static_cast<Engine*>(c->engine));
-  for (cdl_ctx* l : c->lanes)
-    if (l->engine) f(static_cast<Engine*>(l->engine));
+  if (c->engine) f(static_cast<Engine*>(c->engine), (size_t)0);
+  for (size_t s = 0; s < c->slots.size(); s++)
+    for (cdl_ctx* l : c->slots[s].lanes)
+      if (l->engine) f(static_cast<Engine*>(l->engine), s);
+}
+
+// length of the union of the kernel intervals of slot s's engines
+double slot_busy_ms(cdl_ctx* c, size_t s) {
+  std::vector<std::pair<float, float>> iv;
+  for_each_engine(c, [&](Engine* E, size_t es) {
+    if (es == s) iv.insert(iv.end(), E->intervals.begin(), E->intervals.end());
+  });
+  std::sort(iv.begin(), iv.end());
+  double busy = 0, cur_lo = 0, cur_hi = -1;
+  for (auto& p : iv) {
+    if (cur_hi < 0 || p.first > cur_hi) {
+      if (cur_hi >= 0) busy += cur_hi - cur_lo;
+      cur_lo = p.first;
+      cur_hi = p.second;
+    } else if (p.second > cur_hi) {
+      cur_hi = p.second;
+    }
+  }
+  if (cur_hi >= 0) busy += cur_hi - cur_lo;
+  return busy;
 }
 
 }  // namespace
@@ -162,7 +227,7 @@ uint64_t cdl_launch_count(cdl_ctx* c) {
   if (!c) return 0;
   std::lock_guard<std::mutex> lk(c->mu);
   uint64_t n = 0;
-  for_each_engine(c, [&](Engine* E) { n += E->launches; });
+  for_each_engine(c, [&](Engine* E, size_t) { n += E->launches; });
   return n;
 }
 
@@ -175,7 +240,7 @@ int32_t cdl_engine_stats(cdl_ctx* c, uint64_t* launches, double* ms, double* mod
     if (modmul) modmul[i] = 0;
     if (bytes) bytes[i] = 0;
   }
-  for_each_engine(c, [&](Engine* E) {
+  for_each_engine(c, [&](Engine* E, size_t) {
     for (int i = 0; i < 4; i++) {
       if (launches) launches[i] += E->stats.n[i];
       if (ms) ms[i] += E->stats.ms[i];
@@ -190,21 +255,16 @@ int32_t cdl_engine_stats(cdl_ctx* c, uint64_t* launches, double* ms, double* mod
 int32_t cdl_engine_busy_ms(cdl_ctx* c, double* busy_ms) {
   if (!c || !busy_ms) return CDL_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lk(c->mu);
-  std::vector<std::pair<float, float>> iv;
-  for_each_engine(c, [&](Engine* E) { iv.insert(iv.end(), E->intervals.begin(), E->intervals.end()); });
-  std::sort(iv.begin(), iv.end());
-  double busy = 0, cur_lo = 0, cur_hi = -1;
-  for (auto& p : iv) {
-    if (cur_hi < 0 || p.first > cur_hi) {
-      if (cur_hi >= 0) busy += cur_hi - cur_lo;
-      cur_lo = p.first;
-      cur_hi = p.second;
-    } else if (p.second > cur_hi) {
-      cur_hi = p.second;
-    }
-  }
-  if (cur_hi >= 0) busy += cur_hi - cur_lo;
+  double busy = 0;
+  for (size_t s = 0; s < c->slots.size(); s++) busy = std::max(busy, slot_busy_ms(c, s));
   *busy_ms = busy;
+  return CDL_OK;
+}
+
+int32_t cdl_engine_busy_ms_device(cdl_ctx* c, size_t slot, double* busy_ms) {
+  if (!c || !busy_ms || slot >= c->slots.size()) return CDL_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lk(c->mu);
+  *busy_ms = slot_busy_ms(c, slot);
   return CDL_OK;
 }
 
@@ -327,7 +387,7 @@ int32_t cdl_crs_export(cdl_ctx* c, const cdl_crs* crs, cdl_g1_affine* points) {
   if (!c || !crs || !points) return CDL_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  CDL_CUDA(c, cudaMemcpy(points, crs->d_points, (size_t)(crs->ell + 9) * sizeof(cdl::G1Affine), cudaMemcpyDeviceToHost));
+  CDL_CUDA(c, cudaMemcpy(points, crs->rep[0].d_points, (size_t)(crs->ell + 9) * sizeof(cdl::G1Affine), cudaMemcpyDeviceToHost));
   return CDL_OK;
 }
 
@@ -349,8 +409,12 @@ int32_t cdl_set_batch_verify_min(cdl_ctx* c, int32_t proofs) {
 
 void cdl_crs_free(cdl_crs* crs) {
   if (!crs) return;
-  if (crs->d_points) { cudaSetDevice(crs->ctx->device); cudaFree(crs->d_points); }
-  if (crs->d_fixed) { cudaSetDevice(crs->ctx->device); cudaFree(crs->d_fixed); }
+  for (size_t s = 0; s < crs->rep.size(); s++) {
+    const cdl_crs::Replica& r = crs->rep[s];
+    cudaSetDevice(crs->ctx->slots[s].device);
+    if (r.d_points) cudaFree(r.d_points);
+    if (r.d_fixed) cudaFree(r.d_fixed);
+  }
   delete crs;
 }
 
@@ -392,9 +456,9 @@ int32_t cdl_shuffle_permute_commit_batch(cdl_ctx* c, const cdl_crs* crs, size_t 
   if (!c || !crs || B == 0 || !Rs || !Ss || !perms || !ks || !rands || !Ts || !Us || !M || !rs_m || !status ||
       !rands_present(rands, B))
     return CDL_ERR_INVALID_ARG;
-  if (size_t G = lanes_for(c, B); G > 1) {
+  if (split_lanes(c, B)) {
     const size_t e = crs->ell;
-    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
       return cdl_shuffle_permute_commit_batch(lane, crs, hi - lo, Rs + lo * e, Ss + lo * e, perms + lo * e, ks + lo,
                                               rands + lo, Ts + lo * e, Us + lo * e, M + lo, rs_m + 4 * lo, status + lo);
     });
@@ -456,9 +520,9 @@ int32_t cdl_prove_batch(cdl_ctx* c, const cdl_crs* crs, size_t B, const cdl_g1_a
   if (!c || !crs || B == 0 || !Rs || !Ss || !Ts || !Us || !M || !perms || !ks || !rs_m || !rands || !proofs ||
       !proof_lens || !status || !rands_present(rands, B))
     return CDL_ERR_INVALID_ARG;
-  if (size_t G = lanes_for(c, B); G > 1) {
+  if (split_lanes(c, B)) {
     const size_t e = crs->ell;
-    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
       return cdl_prove_batch(lane, crs, hi - lo, Rs + lo * e, Ss + lo * e, Ts + lo * e, Us + lo * e, M + lo,
                              perms + lo * e, ks + lo, rs_m + 4 * lo, rands + lo, proofs + lo * proof_cap, proof_cap,
                              proof_lens + lo, status + lo);
@@ -591,9 +655,9 @@ int32_t cdl_verify_batch(cdl_ctx* c, const cdl_crs* crs, size_t B, const uint8_t
     if (proof_lens[b] > proof_stride) return c->fail(CDL_ERR_INVALID_ARG, "proof %zu is longer than the proof stride", b);
     ok[b] = 0;
   }
-  if (size_t G = lanes_for(c, B); G > 1) {
+  if (split_lanes(c, B)) {
     const size_t e = crs->ell;
-    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
       return cdl_verify_batch(lane, crs, hi - lo, proofs + lo * proof_stride, proof_stride, proof_lens + lo,
                               Rs + lo * e, Ss + lo * e, Ts + lo * e, Us + lo * e, M + lo, rands + lo, ok + lo,
                               status + lo);
@@ -658,9 +722,9 @@ int32_t cdl_whisk_generate_shuffle_proof_batch(cdl_ctx* c, const cdl_crs* crs, s
                                                size_t proof_cap, int32_t* status_out) {
   if (!c || !crs || !pre_trackers || !rands_in || !post_trackers || !proofs_out || !status_out || B == 0)
     return CDL_ERR_INVALID_ARG;
-  if (size_t G = lanes_for(c, B); G > 1) {
+  if (split_lanes(c, B)) {
     const size_t tb = (size_t)crs->ell * 96;
-    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
       return cdl_whisk_generate_shuffle_proof_batch(lane, crs, hi - lo, pre_trackers + lo * tb, rands_in + lo,
                                                     post_trackers + lo * tb, proofs_out + lo * proof_cap, proof_cap,
                                                     status_out + lo);
@@ -738,9 +802,9 @@ int32_t cdl_whisk_is_valid_shuffle_proof_batch(cdl_ctx* c, const cdl_crs* crs, s
                                                cdl_rand* const* rands_in, int32_t* ok, int32_t* status_out) {
   if (!c || !crs || !pre_trackers || !post_trackers || !proofs || !rands_in || !ok || !status_out || B == 0)
     return CDL_ERR_INVALID_ARG;
-  if (size_t G = lanes_for(c, B); G > 1) {
+  if (split_lanes(c, B)) {
     const size_t tb = (size_t)crs->ell * 96;
-    return run_lanes(c, B, G, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
       return cdl_whisk_is_valid_shuffle_proof_batch(lane, crs, hi - lo, pre_trackers + lo * tb, post_trackers + lo * tb,
                                                     proofs + lo * proof_len, proof_len, rands_in + lo, ok + lo,
                                                     status_out + lo);
@@ -827,6 +891,11 @@ cdlh::Fr tracker_challenge(const uint8_t* kG, const uint8_t* krG, const uint8_t*
 int32_t cdl_whisk_generate_tracker_proof_batch(cdl_ctx* c, size_t B, const uint8_t* trackers, const cdl_fr* ks,
                                                cdl_rand* const* rands, uint8_t* proofs, int32_t* status_out) {
   if (!c || !trackers || !ks || !rands || !proofs || !status_out || B == 0 || B > (1u << 24)) return CDL_ERR_INVALID_ARG;
+  if (slots_for(c, B) > 1)
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_whisk_generate_tracker_proof_batch(lane, hi - lo, trackers + 96 * lo, ks + lo, rands + lo,
+                                                    proofs + 128 * lo, status_out + lo);
+    }, false);
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   Engine* E = engine_of(c);
@@ -874,6 +943,11 @@ int32_t cdl_whisk_generate_tracker_proof_batch(cdl_ctx* c, size_t B, const uint8
 int32_t cdl_whisk_is_valid_tracker_proof_batch(cdl_ctx* c, size_t B, const uint8_t* trackers, const uint8_t* k_comms,
                                                const uint8_t* proofs, int32_t* ok, int32_t* status_out) {
   if (!c || !trackers || !k_comms || !proofs || !ok || !status_out || B == 0 || B > (1u << 24)) return CDL_ERR_INVALID_ARG;
+  if (slots_for(c, B) > 1)
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_whisk_is_valid_tracker_proof_batch(lane, hi - lo, trackers + 96 * lo, k_comms + 48 * lo,
+                                                    proofs + 128 * lo, ok + lo, status_out + lo);
+    }, false);
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   Engine* E = engine_of(c);

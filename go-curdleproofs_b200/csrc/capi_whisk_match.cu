@@ -91,9 +91,16 @@ extern "C" {
 int32_t cdl_whisk_match_trackers(cdl_ctx* c, size_t T, const uint8_t* trackers, size_t V, const cdl_fr* ks,
                                  int32_t* owner, int32_t* status) {
   if (!c || !trackers || !ks || !owner || !status || T == 0 || V == 0) return CDL_ERR_INVALID_ARG;
-  std::lock_guard<std::mutex> lk(c->mu);
-  if (T > CDL_WHISK_MATCH_MAX || V > CDL_WHISK_MATCH_MAX)
+  if (T > CDL_WHISK_MATCH_MAX || V > CDL_WHISK_MATCH_MAX) {
+    std::lock_guard<std::mutex> lk(c->mu);
     return c->fail(CDL_ERR_TOO_LARGE, "whisk_match_trackers: %zu trackers x %zu keys exceed 2^24", T, V);
+  }
+  // every slot matches its own block of trackers against all keys; blocks start on table tiles
+  if (cdlh::slots_for(c, T) > 1)
+    return cdlh::run_split(c, T, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_whisk_match_trackers(lane, hi - lo, trackers + 96 * lo, V, ks, owner + lo, status + lo);
+    }, false, cdl::kMatchTile);
+  std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   Engine* E = engine_of(c);
   int32_t rc;

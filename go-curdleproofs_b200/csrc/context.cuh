@@ -1,4 +1,4 @@
-// Library context: one CUDA device, one stream, grow-only device scratch buffers.
+// Library context: a CUDA device, one stream, grow-only device scratch buffers.
 #pragma once
 #include <cuda_runtime.h>
 #include <cstdarg>
@@ -41,13 +41,20 @@ struct cdl_ctx {
   int batch_verify_min = -1;  // cdl_set_batch_verify_min: proofs per (lane) verification from which one combined MSM checks the batch first; -1 = default, 0 = never
   int msm_ba_override = -1;  // cdl_set_msm_batch_affine: batch-affine rounds of the large MSM, -1 = pick by bucket load
   // Batched protocol calls are cut into up to n_lanes sub-batches that advance
-  // concurrently, each on its own lane context (same device, own stream, engine,
-  // staging): one lane's host-side Fiat-Shamir work overlaps the other lanes'
-  // kernels, and their latency-bound kernels overlap each other.
+  // concurrently, each on its own lane context (own stream, engine, staging): one
+  // lane's host-side Fiat-Shamir work overlaps the other lanes' kernels, and their
+  // latency-bound kernels overlap each other.  A root context has one device slot per
+  // entry of its device list (cdl_create_devices); every slot has its own lanes on its
+  // device, and slot 0 is the root context's own device.
+  struct Slot {
+    int device = 0;
+    cudaEvent_t base_ev = nullptr;  // origin of the slot's kernel-interval timeline (busy-time accounting)
+    std::vector<cdl_ctx*> lanes;
+  };
   cdl_ctx* parent = nullptr;
-  std::vector<cdl_ctx*> lanes;
-  int n_lanes = 4;               // CDL_LANES / cdl_set_lanes
-  cudaEvent_t base_ev = nullptr; // origin of the kernel-interval timeline (busy-time accounting)
+  std::vector<Slot> slots;       // root only
+  size_t dev_slot = 0;           // lanes: the slot of root()->slots they belong to
+  int n_lanes = 4;               // CDL_LANES / cdl_set_lanes: lanes per slot
   cdl_ctx* root() { return parent ? parent : this; }
   static constexpr int kSlots = 8;
   void* slot[kSlots] = {};

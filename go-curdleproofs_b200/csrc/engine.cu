@@ -40,18 +40,20 @@ Layout::Layout(uint32_t ell_) {
 }
 
 // ------------------------------------------------------------------ plumbing
-// a lane engine shares the host cores with its sibling lanes
+// a lane engine shares the host cores with its sibling lanes, and the device slots of a context share them
 Engine::Engine(cdl_ctx* ctx)
     : ctx_(ctx),
-      pool_(host_threads(ctx->parent != nullptr)) {}
+      pool_(host_threads(ctx->parent != nullptr, ctx->root()->slots.size())) {}
 
-// CDL_HOST_THREADS caps the host cores one context may use (several ranks on one box share them)
-unsigned Engine::host_threads(bool lane) {
+// CDL_HOST_THREADS caps the host cores one context may use (several ranks on one box share them); each of
+// the context's device slots gets an equal share
+unsigned Engine::host_threads(bool lane, size_t slots) {
   unsigned hw = std::max(1u, std::thread::hardware_concurrency());
   if (const char* e = getenv("CDL_HOST_THREADS")) {
     int v = atoi(e);
     if (v >= 1) hw = std::min(hw, (unsigned)v);
   }
+  hw = std::max(1u, hw / (unsigned)std::max<size_t>(1, slots));
   return lane ? std::max(2u, std::min(32u, hw / 2)) : std::max(1u, std::min(64u, hw));
 }
 
@@ -102,7 +104,7 @@ void Engine::finish_timing() {
   float ms = 0;
   if (cudaEventElapsedTime(&ms, ctx_->ev0, ctx_->ev1) == cudaSuccess) stats.ms[pending_cls_] += ms;
   float t0 = 0;
-  if (cudaEventElapsedTime(&t0, ctx_->root()->base_ev, ctx_->ev0) == cudaSuccess && intervals.size() < (1u << 22))
+  if (cudaEventElapsedTime(&t0, ctx_->root()->slots[ctx_->dev_slot].base_ev, ctx_->ev0) == cudaSuccess && intervals.size() < (1u << 22))
     intervals.emplace_back(t0, t0 + ms);
   pending_cls_ = -1;
 }
@@ -135,14 +137,21 @@ int32_t Engine::ensure_pool(size_t npoints) {
 }
 
 int32_t Engine::load_crs(const Layout& L, const cdl_crs* crs) {
-  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_, crs->d_points, (size_t)L.crs_size * sizeof(G1Affine),
-                                 cudaMemcpyDeviceToDevice, ctx_->stream));
+  const G1Affine* pts;
+  {
+    std::lock_guard<std::mutex> lk(crs->fixed_mu);
+    pts = crs->points_on(ctx_->dev_slot);
+  }
+  if (!pts) return ctx_->fail(CDL_ERR_CUDA, "crs replica for device slot %zu could not be made", ctx_->dev_slot);
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_, pts, (size_t)L.crs_size * sizeof(G1Affine), cudaMemcpyDeviceToDevice,
+                                 ctx_->stream));
   return CDL_OK;
 }
 
 // Batches of at least CDL_FIXED_BASE_MINB instances (default 64 per lane; 0 = never) use fixed-base tables
-// for the CRS points.  The tables belong to the CRS object and are built on first use (~ 10 ms and
-// 4.3 MB per point); a failed allocation simply leaves the generic kernels in charge.
+// for the CRS points.  The tables belong to the CRS object, one copy per device slot, and are built on
+// that slot's first use (~ 10 ms and 4.3 MB per point); a failed allocation simply leaves the generic
+// kernels in charge.
 void Engine::select_fixed(const Layout& L, const cdl_crs* crs, size_t B) {
   fixed_ = cdl::FixedTable();
   static const long min_b = [] {
@@ -153,23 +162,25 @@ void Engine::select_fixed(const Layout& L, const cdl_crs* crs, size_t B) {
   const long lim = over >= 0 ? over : min_b;
   if (lim <= 0 || (long)B < lim) return;
   std::lock_guard<std::mutex> lk(crs->fixed_mu);
-  if (!crs->d_fixed && !crs->fixed_failed) {
+  cdl_crs::Replica& r = crs->rep[ctx_->dev_slot];
+  if (!r.d_fixed && !r.fixed_failed) {
+    const G1Affine* pts = crs->points_on(ctx_->dev_slot);
     cdl::G1Affine* tab = nullptr;
-    if (cudaMalloc(&tab, cdl::fixed_table_bytes(L.crs_size)) != cudaSuccess) {
+    if (!pts || cudaMalloc(&tab, cdl::fixed_table_bytes(L.crs_size)) != cudaSuccess) {
       cudaGetLastError();
-      crs->fixed_failed = true;
+      r.fixed_failed = true;
       return;
     }
-    cdl::launch_fixed_build(crs->d_points, L.crs_size, tab, ctx_->stream);
+    cdl::launch_fixed_build(pts, L.crs_size, tab, ctx_->stream);
     if (cudaStreamSynchronize(ctx_->stream) != cudaSuccess) {
       cudaFree(tab);
-      crs->fixed_failed = true;
+      r.fixed_failed = true;
       return;
     }
-    crs->d_fixed = tab;
+    r.d_fixed = tab;
   }
-  if (crs->d_fixed) {
-    fixed_.tab = crs->d_fixed;
+  if (r.d_fixed) {
+    fixed_.tab = r.d_fixed;
     fixed_.nbase = L.crs_size;
   }
 }

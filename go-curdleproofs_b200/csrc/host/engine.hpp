@@ -27,17 +27,25 @@ struct cdl_rand {
   explicit cdl_rand(uint64_t seed) : r(seed) {}
 };
 
-// crs.go:10-18.  Points are kept on the device (pool image) and as compressed
-// encodings on the host (for transcript appends of H).
+// crs.go:10-18.  Points are kept on the host (image), on the device of every slot of the owning context
+// (pool image) and as compressed encodings on the host (for transcript appends of H).
 struct cdl_crs {
   cdl_ctx* ctx = nullptr;
   uint32_t ell = 0;
-  cdl::G1Affine* d_points = nullptr;  // Gs[ell] Hs[4] H Gt Gu Gsum Hsum INF  (ell + 10 points)
+  std::vector<cdl_g1_affine> host;    // Gs[ell] Hs[4] H Gt Gu Gsum Hsum INF  (ell + 10 points)
   std::vector<uint8_t> enc;           // same order, 48 B each
-  // fixed-base tables of those points (csrc/fixed_base.cuh), built by the first large batch that uses this CRS
+  // One replica per device slot of ctx: the image (slot 0's made with the CRS, the others uploaded from `host`
+  // by their first call) and its fixed-base tables (csrc/fixed_base.cuh), built by the first large batch of
+  // that slot that uses this CRS.  Guarded by fixed_mu.
+  struct Replica {
+    cdl::G1Affine* d_points = nullptr;
+    cdl::G1Affine* d_fixed = nullptr;
+    bool fixed_failed = false;
+  };
   mutable std::mutex fixed_mu;
-  mutable cdl::G1Affine* d_fixed = nullptr;
-  mutable bool fixed_failed = false;
+  mutable std::vector<Replica> rep;
+  // slot `s`'s image, uploaded on first use (fixed_mu held, the slot's device current); null if that fails
+  const cdl::G1Affine* points_on(size_t s) const;
 };
 
 namespace cdlh {
@@ -171,8 +179,8 @@ class Engine {
   // 3 compress / normalise): launches, CUDA-event time on the launching stream,
   // algorithmic modmul (SURVEY.md §8d conventions) and algorithmic bytes
   uint64_t launches = 0;
-  // [start, end) of every timed kernel chain on the root context's timeline (ms since base_ev);
-  // the union over all lanes is the device busy time
+  // [start, end) of every timed kernel chain on its slot's timeline (ms since the slot's base_ev);
+  // the union over the slot's engines is that device slot's busy time
   std::vector<std::pair<float, float>> intervals;
   struct Stats {
     uint64_t n[4] = {};
@@ -205,7 +213,7 @@ class Engine {
     prof.par += now() - t0;
   }
   static double now();
-  static unsigned host_threads(bool lane);
+  static unsigned host_threads(bool lane, size_t slots);
 
  private:
   cdl_ctx* ctx_;
@@ -255,5 +263,14 @@ std::string parse_wire_proof(const uint8_t* buf, size_t len, bool with_m, WirePr
 Engine* engine_of(cdl_ctx* c);
 // gnark's G1Jac of an affine point: (x, y, 1), or (1, 1, 0) for infinity
 void affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a);
+// Device slots a batched call of B units on c uses: max(1, min(slots, B / 32)); 1 on a lane context.
+size_t slots_for(cdl_ctx* c, size_t B);
+// Runs fn(lane ctx, lo, hi) for contiguous pieces [lo, hi) of a call of B units on a root context concurrently,
+// one host thread per piece (DESIGN §4): slot s of the D = slots_for(c, B) slots in use takes the block that
+// sharding.shard_bounds(B, D, s) gives, its bounds rounded to multiples of `align` (empty blocks are skipped);
+// with `lanes` it cuts its block into up to n_lanes lanes of at least 32 units, else the block is one piece
+// on the slot's lane 0.
+int32_t run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes = true,
+                  size_t align = 1);
 
 }  // namespace cdlh

@@ -18,9 +18,10 @@
  *    cdl_last_error(ctx) gives a human-readable message for the calling thread's
  *    last failure on that context.
  *  - host-pointer entry points copy in/out and retain nothing after return (cgo
- *    pointer rule).  A context is bound to one CUDA device and is safe to call
- *    from many OS threads (calls serialise on an internal mutex; use one context
- *    per thread or the *_batch entry points for concurrency).
+ *    pointer rule).  A context is bound to one CUDA device, or to a list of them
+ *    (cdl_create_devices), and is safe to call from many OS threads (calls
+ *    serialise on an internal mutex; use one context per thread or the *_batch
+ *    entry points for concurrency).
  *  - there is NO CPU fallback: without a CUDA device cdl_create fails with
  *    CDL_ERR_NO_DEVICE.
  */
@@ -54,6 +55,27 @@ typedef struct cdl_g1_jac { cdl_fp x, y, z; } cdl_g1_jac;       /* gnark bls1238
 
 /* ---- context ---------------------------------------------------------- */
 int32_t cdl_create(int device, cdl_ctx** out);
+/* A context whose batched calls use the GPUs devices[0 .. n).  cdl_create(d) is cdl_create_devices(&d, 1).
+ * Each entry is a device slot with its own lanes (cdl_set_lanes = lanes per slot), pools and CRS replicas;
+ * a device may be listed more than once.  Results never depend on the device list.
+ *
+ * Split over the slots: the batched Whisk shuffle-proof calls, cdl_shuffle_permute_commit_batch,
+ * cdl_prove_batch, cdl_verify_batch, the batched tracker-proof calls and cdl_whisk_match_trackers.  Slot s
+ * of the D' = max(1, min(n, B / 32)) slots in use takes the contiguous block s of B instances (block sizes
+ * differ by at most one, as sharding.shard_bounds deals them; for matching the block bounds are rounded to
+ * multiples of 256 trackers and every slot matches its block against all keys), and cuts it into lanes
+ * as a one-device context cuts a batch.  A call of fewer than 64 instances, and every single
+ * (non-batched) protocol call, runs on slot 0.
+ *
+ * Everything else runs on slot 0's device (devices[0]): the cdl_g1_* primitives, the large and device
+ * MSMs, cdl_dev_* buffers (device memory of devices[0]), cdl_rand_get_g1_affines and CRS generation.
+ * cdl_comm_init refuses a context of more than one slot: the NCCL-sharded MSM runs one process (and
+ * one single-device context) per GPU.
+ * CDL_ERR_INVALID_ARG for n == 0, n > 16 or a device id out of range; CDL_ERR_NO_DEVICE without a
+ * CUDA device. */
+int32_t cdl_create_devices(const int32_t* devices, size_t n, cdl_ctx** out);
+/* The device list of the context: *n receives its length, devices[0 .. min(cap, *n)) its entries. */
+int32_t cdl_context_devices(cdl_ctx* ctx, int32_t* devices, size_t cap, size_t* n);
 void cdl_destroy(cdl_ctx* ctx);
 const char* cdl_last_error(cdl_ctx* ctx);
 /* ABI version of this build (major << 16 | minor). */
@@ -264,15 +286,20 @@ int32_t cdl_host_selftest_fibers(uint32_t n, uint32_t rounds, uint8_t* digest32,
 int32_t cdl_engine_stats(cdl_ctx* ctx, uint64_t* launches, double* ms, double* modmul, double* bytes, int reset);
 /* Device busy time since the last cdl_engine_stats(.., reset = 1): the length of
  * the union of all timed kernel intervals over every lane's stream (lanes overlap,
- * so the per-class sums above can exceed it). */
+ * so the per-class sums above can exceed it).  With several device slots, the
+ * largest busy time of one slot. */
 int32_t cdl_engine_busy_ms(cdl_ctx* ctx, double* busy_ms);
+/* Device busy time of slot `slot` since the last stats reset (union of that slot's lanes' kernel intervals).
+ * CDL_ERR_INVALID_ARG for a slot beyond the device list. */
+int32_t cdl_engine_busy_ms_device(cdl_ctx* ctx, size_t slot, double* busy_ms);
 /* A batched protocol call is cut into up to `lanes` sub-batches (default 4, at
  * least 32 instances each) that advance concurrently on their own CUDA streams
  * and host threads: one lane's host-side transcript work overlaps the other
- * lanes' kernels.  Results do not depend on it.  Also environment CDL_LANES. */
+ * lanes' kernels.  Results do not depend on it.  Also environment CDL_LANES.
+ * With several device slots this is the number of lanes per slot. */
 int32_t cdl_set_lanes(cdl_ctx* ctx, int32_t lanes);
 /* Number of GPU kernels launched by protocol-level calls, batched MSMs and tracker matching on this
- * context so far. */
+ * context so far, summed over its device slots. */
 uint64_t cdl_launch_count(cdl_ctx* ctx);
 
 /* ---- large MSM, device-resident vectors, multi-GPU ----------------------
@@ -333,7 +360,8 @@ int32_t cdl_set_msm_batch_affine(cdl_ctx* ctx, int32_t rounds);
 
 /* One process per GPU: rank 0 calls cdl_comm_unique_id, the host application
  * ships the 128 bytes to every rank (any transport), every rank calls
- * cdl_comm_init (collective; NCCL over NVLink / NVSwitch, bound with dlopen). */
+ * cdl_comm_init (collective; NCCL over NVLink / NVSwitch, bound with dlopen)
+ * on a single-device context (CDL_ERR_INVALID_ARG with more than one slot). */
 int32_t cdl_comm_unique_id(uint8_t* id128);
 int32_t cdl_comm_init(cdl_ctx* ctx, const uint8_t* id128, int32_t rank, int32_t world);
 int32_t cdl_comm_destroy(cdl_ctx* ctx);

@@ -32,7 +32,8 @@ import (
 	"github.com/consensys/gnark-crypto/ecc/bls12-381/fr"
 )
 
-// Context is one device + stream; safe for concurrent use (calls serialise on the context).
+// Context is one device + stream (or a list of devices, NewDevices); safe for concurrent use (calls
+// serialise on the context).
 type Context struct{ h *C.cdl_ctx }
 
 // New opens CUDA device `device`.
@@ -42,6 +43,45 @@ func New(device int) (*Context, error) {
 		return nil, fmt.Errorf("cdl_create: status %d (no CPU fallback)", int(rc))
 	}
 	return &Context{h}, nil
+}
+
+// NewDevices opens one context over the CUDA devices listed (at most 16; a device may appear more
+// than once).  Its batched calls (Whisk shuffle and tracker proofs, the curdleproof batches, tracker
+// matching) are dealt to the devices in contiguous blocks; everything else runs on devices[0].
+// Results do not depend on the list.  A multi-GPU node uses one such context instead of a process
+// per GPU.
+func NewDevices(devices []int) (*Context, error) {
+	if len(devices) == 0 {
+		return nil, errors.New("NewDevices: empty device list")
+	}
+	ids := make([]C.int32_t, len(devices))
+	for i, d := range devices {
+		ids[i] = C.int32_t(d)
+	}
+	var h *C.cdl_ctx
+	if rc := C.cdl_create_devices(&ids[0], C.size_t(len(ids)), &h); rc != 0 {
+		return nil, fmt.Errorf("cdl_create_devices: status %d (no CPU fallback)", int(rc))
+	}
+	return &Context{h}, nil
+}
+
+// Devices returns the context's device list (one entry per device slot).
+func (c *Context) Devices() ([]int, error) {
+	var n C.size_t
+	if rc := C.cdl_context_devices(c.h, nil, 0, &n); rc != 0 {
+		return nil, c.err(rc)
+	}
+	ids := make([]C.int32_t, n)
+	if n > 0 {
+		if rc := C.cdl_context_devices(c.h, &ids[0], n, &n); rc != 0 {
+			return nil, c.err(rc)
+		}
+	}
+	out := make([]int, len(ids))
+	for i, d := range ids {
+		out[i] = int(d)
+	}
+	return out, nil
 }
 
 // Close releases the device resources of the context.
