@@ -63,6 +63,7 @@ def load_library():
     lib.cdl_g1_msm_batch_device.argtypes = [vp, vp, vp, vp, vp, sz, vp, vp, vp]
     lib.cdl_g1_scalar_mul_affine.argtypes = [vp, vp, vp, sz, sz, vp]
     lib.cdl_g1_fold.argtypes = [vp, vp, vp, vp, sz]
+    lib.cdl_g1_batch_scalar_mul_base.argtypes = [vp, vp, vp, sz, vp, vp]
     lib.cdl_g1_batch_to_affine.argtypes = [vp, vp, sz, vp]
     lib.cdl_g1_sum_affine.argtypes = [vp, vp, sz, vp]
     lib.cdl_g1_compress.argtypes = [vp, vp, sz, vp]
@@ -195,6 +196,22 @@ class Context:
         buf = C.create_string_buffer(L, max(1, len(L)))
         self._chk(self.lib.cdl_g1_fold(self.h, buf, R, x, n))
         return buf.raw[: len(L)]
+
+    def g1_batch_scalar_mul_base(self, base: bytes, scalars: bytes, affine: bool = True, compressed: bool = False):
+        """bls12381.BatchScalarMultiplicationG1: scalars[i] * base for n scalars (n x 32 bytes, gnark fr.Element)
+        and one affine base (96 bytes, in G1) -> n x 96 affine bytes if `affine`, n x 48 compressed bytes if
+        `compressed`, or the pair (affine, compressed) when both are asked for."""
+        if not (affine or compressed):
+            raise CdlError(-3, "ask for affine or compressed results")
+        n = len(scalars) // FR_BYTES
+        out = C.create_string_buffer(max(1, n) * G1_AFFINE_BYTES) if affine else None
+        out48 = C.create_string_buffer(max(1, n) * 48) if compressed else None
+        self._chk(self.lib.cdl_g1_batch_scalar_mul_base(self.h, base, scalars, n, out, out48))
+        a = out.raw[: n * G1_AFFINE_BYTES] if affine else None
+        z = out48.raw[: n * 48] if compressed else None
+        if affine and compressed:
+            return a, z
+        return a if affine else z
 
     def g1_batch_to_affine(self, jac: bytes) -> bytes:
         n = len(jac) // G1_JAC_BYTES

@@ -71,8 +71,9 @@ Engine::~Engine() {
   if (d_win_) cudaFree(d_win_);
   if (d_match_) cudaFree(d_match_);
   if (d_bv_) cudaFree(d_bv_);
+  for (BaseTable& b : base_tabs_) cudaFree(b.tab);
   for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_, &s_bv_,
-                     &s_in_}) {
+                     &s_in_, &s_base_}) {
     if (s->h) cudaFreeHost(s->h);
     if (s->d) cudaFree(s->d);
   }

@@ -171,6 +171,10 @@ class Engine {
   // Whisk tracker matching (capi_whisk_match.cu) on decoded trackers pool[t] = rG_t, pool[T + t] = krG_t:
   // owner[t] = the smallest v with ks[v] * rG_t == krG_t, else INT32_MAX.  ks: V gnark fr.Element (Montgomery)
   int32_t match_trackers(uint32_t T, const Fr* ks, uint32_t V, int32_t* owner);
+  // Batched fixed-base scalar multiplication (capi_base_mul.cu): out[i] = sc[i] * base, i < n (sc: gnark
+  // fr.Element, Montgomery), affine to out and / or compressed to out48 (either may be null).  CDL_ERR_INVALID_ARG
+  // for a base outside G1.  The base is not the point at infinity.
+  int32_t base_mul(const cdl_g1_affine& base, const Fr* sc, size_t n, cdl_g1_affine* out, uint8_t* out48);
 
   cdl_ctx* ctx() { return ctx_; }
   cdl::G1Affine* d_pool() { return d_pool_; }
@@ -226,6 +230,16 @@ class Engine {
   void* d_match_ = nullptr;  // tables and window bases of one tile of trackers (match_scratch)
   size_t match_cap_ = 0;
   bool match_scratch(uint32_t tile);
+  // Width-12 fixed-base tables of callers' bases (base_mul), keyed by the 96 base bytes: at most kBaseTables,
+  // the least recently used replaced.  Separate allocations, so the pool and the match scratch stay as they are.
+  struct BaseTable {
+    cdl_g1_affine base;
+    cdl::G1Affine* tab = nullptr;
+    uint64_t used = 0;  // base_clock_ at the last call that used it
+  };
+  static constexpr size_t kBaseTables = 4;
+  std::vector<BaseTable> base_tabs_;
+  uint64_t base_clock_ = 0;
   void* d_bv_ = nullptr;  // combined verifier check: term list, large-MSM scratch, result (batch_check)
   size_t bv_cap_ = 0;
   // The verifier's second MSM stage `st`, uploaded (d_idx, d_sc, d_tasks), as one large MSM with the weight
@@ -240,7 +254,7 @@ class Engine {
     size_t cap = 0;
   };
   Staging s_idx_, s_sc_, s_task_, s_out_, s_ops_, s_enc_, s_st_, s_jac_, s_sub_, s_t2_, s_cr_, s_fsub_, s_vs_, s_as_, s_bv_,
-      s_in_;
+      s_in_, s_base_;
   int32_t reserve(Staging& s, size_t bytes);
   void tick();                                   // event before a kernel
   void tock(int cls, double modmul, double bytes);  // event after; call finish_timing() after the sync

@@ -54,12 +54,24 @@ void launch_match_windows(const G1Affine* rg, uint32_t nt, G1Jac* out, cudaStrea
 // trackers t0 .. t0 + nt - 1 against every key; tab = launch_fixed_build<kMatchC>(window bases of rg + t0, nt, ..)
 void launch_match_table(const G1Affine* tab, const G1Affine* krg, uint32_t t0, uint32_t nt, const Fr* ks,
                         uint32_t V, int32_t* owner, cudaStream_t st);
-// fixed-base tables of window width C for nbase points: C = 12 the CRS tables, bases = the points; C = kMatchC
-// the tracker tables, bases = their fb_windows(C) window bases each (launch_match_windows)
+// fixed-base tables of window width C for nbase points, every (point, window) row built by Seg threads.
+// Point bases (C = 12 the CRS tables): bases = the points.  Row bases (C = kMatchC the tracker tables, C = 12
+// with kBaseSeg the table of a caller's base): bases = their fb_windows(C) window bases each
+// (launch_match_windows, launch_base_windows)
+constexpr int kFbSeg = 8;      // threads per row of the CRS and tracker tables
+constexpr int kBaseSeg = 128;  // threads per row of a caller's base table: 22 x 128 threads, 16 entries each
 template <int C = kFbC>
 size_t fixed_table_bytes(uint32_t nbase);
-template <int C = kFbC>
+template <int C = kFbC, bool RowBases = (C != kFbC), int Seg = kFbSeg>
 void launch_fixed_build(const G1Affine* bases, uint32_t nbase, G1Affine* tab, cudaStream_t st);
+// --- batched fixed-base scalar multiplication (k_base_mul.cu): out[i] = sc[i] * P for one base P.
+// *status = 0 when *base is in G1 (1 non-canonical coordinate, 2 off the curve, 3 outside G1); with wjac, also
+// wjac[w] = 2^(12 w) P for w < kFbW (Jacobian: normalise with launch_jac_to_affine, then
+// launch_fixed_build<kFbC, true, kBaseSeg>(affine window bases, 1, tab, ..))
+void launch_base_prep(const G1Affine* base, uint32_t* status, G1Jac* wjac, cudaStream_t st);
+void launch_base_fill(const G1Affine* base, G1Affine* out, uint32_t n, cudaStream_t st);  // out[0 .. n) = *base
+// from P's table (fixed_table_bytes(1) bytes); sc Montgomery; out (affine) and / or out48 (compressed), either null
+void launch_base_mul(const G1Affine* tab, const Fr* sc, uint32_t n, G1Affine* out, uint8_t* out48, cudaStream_t st);
 void launch_copy_ranges(G1Affine* pool, const CopyRange* ranges, int n, cudaStream_t st);
 // verifier scalar pipeline on the device (k_verify_scalars.cu): per-proof inputs, all Montgomery fr.Element
 constexpr int kVsMaxM = 16;  // rounds (n <= 2^16)

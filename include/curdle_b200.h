@@ -116,6 +116,26 @@ int32_t cdl_g1_scalar_mul_affine(cdl_ctx* ctx, const cdl_g1_affine* in, const cd
  * gamma for G and gamma^-1 for G') and samemultiscalarargument.go:129-135. */
 int32_t cdl_g1_fold(cdl_ctx* ctx, cdl_g1_affine* L, const cdl_g1_affine* R, const cdl_fr* x, size_t n);
 
+/* bls12381.BatchScalarMultiplicationG1: out[i] = scalars[i] * base, i < n, for one base and many scalars: the
+ * k-commitments kG and initial trackers (G, kG) of many validators, or the blinder products r * G of tracker
+ * proofs.  Scalars are gnark fr.Elements (Montgomery), read as cdl_g1_scalar_mul_affine reads them (limbs
+ * >= r included).  out receives affine points in gnark's layout (infinity = (0, 0)) and out48 the 48-byte
+ * compressed encodings cdl_g1_compress gives; either may be NULL, not both.  For every input the output
+ * bytes equal those of cdl_g1_scalar_mul_affine on n copies of base with scalar_stride = 1.
+ * base must be on the curve and in G1 (checked on the device with decompression's subgroup test), else
+ * CDL_ERR_INVALID_ARG with a message; the point at infinity gives infinity for every scalar.
+ * Two device paths, chosen by n and the context's table cache, with the same results: from
+ * the base's width-12 fixed-base table (22 x 2 048 points, 4.3 MB; 22 mixed additions per scalar), used
+ * when that table is cached or n is large enough that building it pays off (the table is then built and
+ * cached); otherwise GLV scalar multiplication of every scalar, which builds no table.  The context keeps
+ * the tables of its 4 most recently used bases (about 17 MB of device memory, freed by cdl_destroy); a base
+ * whose table is cached is not checked again.  Scalars travel in chunks of 2^20.
+ * n == 0 does nothing; CDL_ERR_INVALID_ARG for a null ctx, base or scalars or when both outputs are NULL;
+ * CDL_ERR_TOO_LARGE when n exceeds CDL_BASE_MUL_MAX, before any input is read. */
+#define CDL_BASE_MUL_MAX (1u << 24)
+int32_t cdl_g1_batch_scalar_mul_base(cdl_ctx* ctx, const cdl_g1_affine* base, const cdl_fr* scalars, size_t n,
+                                     cdl_g1_affine* out, uint8_t* out48);
+
 /* bls12381.BatchJacobianToAffineG1 (transcript/transcript.go:26 and every Serialize). */
 int32_t cdl_g1_batch_to_affine(cdl_ctx* ctx, const cdl_g1_jac* in, size_t n, cdl_g1_affine* out);
 
@@ -277,12 +297,13 @@ int32_t cdl_host_selftest(uint8_t* out32, const cdl_fr* a, const cdl_fr* b, cdl_
  * eight-way path was available on this host (0: both runs were scalar). */
 int32_t cdl_host_selftest_fibers(uint32_t n, uint32_t rounds, uint8_t* digest32, int32_t* used_x8);
 /* Per kernel class statistics of the protocol-level calls, of the batched MSMs
- * (cdl_g1_msm_batch, cdl_g1_msm_batch_device, cdl_g1_msm up to 1 024 terms) and of
- * cdl_whisk_match_trackers since the last reset (class 0 small-MSM, 1 elementwise
- * scalar-mul/fold and tracker matching, 2 decompress, 3 compress / normalise): launches,
- * CUDA-event milliseconds on the launching stream, algorithmic modmul (SURVEY.md §8d
- * conventions; 3 193 per matched (key, tracker) pair) and algorithmic bytes.
- * Each output array has 4 entries. */
+ * (cdl_g1_msm_batch, cdl_g1_msm_batch_device, cdl_g1_msm up to 1 024 terms), of
+ * cdl_whisk_match_trackers and of cdl_g1_batch_scalar_mul_base since the last reset (class 0
+ * small-MSM, 1 elementwise scalar-mul/fold, tracker matching and fixed-base scalar
+ * multiplication, 2 decompress, 3 compress / normalise): launches, CUDA-event milliseconds on the
+ * launching stream, algorithmic modmul (SURVEY.md §8d conventions; 3 193 per matched (key, tracker)
+ * pair and per scalar of cdl_g1_batch_scalar_mul_base, which counts one class-1 launch per chunk of
+ * up to 2^20 scalars) and algorithmic bytes.  Each output array has 4 entries. */
 int32_t cdl_engine_stats(cdl_ctx* ctx, uint64_t* launches, double* ms, double* modmul, double* bytes, int reset);
 /* Device busy time since the last cdl_engine_stats(.., reset = 1): the length of
  * the union of all timed kernel intervals over every lane's stream (lanes overlap,
@@ -298,8 +319,8 @@ int32_t cdl_engine_busy_ms_device(cdl_ctx* ctx, size_t slot, double* busy_ms);
  * lanes' kernels.  Results do not depend on it.  Also environment CDL_LANES.
  * With several device slots this is the number of lanes per slot. */
 int32_t cdl_set_lanes(cdl_ctx* ctx, int32_t lanes);
-/* Number of GPU kernels launched by protocol-level calls, batched MSMs and tracker matching on this
- * context so far, summed over its device slots. */
+/* Number of GPU kernels launched by protocol-level calls, batched MSMs, tracker matching and
+ * cdl_g1_batch_scalar_mul_base on this context so far, summed over its device slots. */
 uint64_t cdl_launch_count(cdl_ctx* ctx);
 
 /* ---- large MSM, device-resident vectors, multi-GPU ----------------------

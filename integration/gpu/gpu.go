@@ -163,6 +163,36 @@ func (c *Context) ScalarMulBatch(in []bls12381.G1Affine, s []fr.Element) ([]bls1
 	return out, nil
 }
 
+// BatchScalarMultiplicationG1 replaces bls12381.BatchScalarMultiplicationG1: scalars[i] * base for one base
+// in G1 and many scalars (k-commitments kG, initial trackers (G, kG), blinder products r*G).  A base outside
+// G1 is an error.  The context caches the fixed-base tables of its four most recently used bases.
+func (c *Context) BatchScalarMultiplicationG1(base *bls12381.G1Affine, scalars []fr.Element) ([]bls12381.G1Affine, error) {
+	out := make([]bls12381.G1Affine, len(scalars))
+	if len(scalars) == 0 {
+		return out, nil
+	}
+	if rc := C.cdl_g1_batch_scalar_mul_base(c.h, (*C.cdl_g1_affine)(unsafe.Pointer(base)), frPtr(scalars),
+		C.size_t(len(scalars)), affPtr(out), nil); rc != 0 {
+		return nil, c.err(rc)
+	}
+	return out, nil
+}
+
+// BatchScalarMultiplicationG1Compressed is BatchScalarMultiplicationG1 returning the 48-byte compressed
+// encodings (G1Affine.Bytes()) of the products, len(scalars) * 48 bytes: the k-commitments kG of many
+// validators, or the krG halves of their trackers.
+func (c *Context) BatchScalarMultiplicationG1Compressed(base *bls12381.G1Affine, scalars []fr.Element) ([]byte, error) {
+	out := make([]byte, 48*len(scalars))
+	if len(scalars) == 0 {
+		return out, nil
+	}
+	if rc := C.cdl_g1_batch_scalar_mul_base(c.h, (*C.cdl_g1_affine)(unsafe.Pointer(base)), frPtr(scalars),
+		C.size_t(len(scalars)), nil, (*C.uint8_t)(unsafe.Pointer(&out[0]))); rc != 0 {
+		return nil, c.err(rc)
+	}
+	return out, nil
+}
+
 // BatchJacobianToAffine replaces bls12381.BatchJacobianToAffineG1 (transcript/transcript.go:26).
 func (c *Context) BatchJacobianToAffine(in []bls12381.G1Jac) ([]bls12381.G1Affine, error) {
 	out := make([]bls12381.G1Affine, len(in))
