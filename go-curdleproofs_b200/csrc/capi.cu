@@ -140,7 +140,6 @@ void cdl_destroy(cdl_ctx* c) {
   }
   cudaSetDevice(c->device);
   if (c->engine) cdl_engine_free_(c->engine);
-  c->free_all();
   cudaEventDestroy(c->ev0);
   cudaEventDestroy(c->ev1);
   if (c->ev_sync) cudaEventDestroy(c->ev_sync);
@@ -261,11 +260,13 @@ static int32_t scalar_mul_impl(cdl_ctx* c, const cdl_g1_affine* in, const cdl_fr
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   size_t ns = stride ? n : 1;
-  G1Affine* d_in = (G1Affine*)c->buf(0, n * sizeof(G1Affine));
-  Fr* d_s = (Fr*)c->buf(1, ns * sizeof(Fr));
-  G1Affine* d_add = addend ? (G1Affine*)c->buf(2, n * sizeof(G1Affine)) : nullptr;
-  G1Affine* d_out = (G1Affine*)c->buf(4, n * sizeof(G1Affine));
-  if (!d_in || !d_s || !d_out || (addend && !d_add)) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->in.grow(n * sizeof(G1Affine), c->stream) || !c->in2.grow(ns * sizeof(Fr), c->stream) ||
+      (addend && !c->addend.grow(n * sizeof(G1Affine), c->stream)) || !c->out.grow(n * sizeof(G1Affine), c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  G1Affine* d_in = (G1Affine*)c->in.d();
+  Fr* d_s = (Fr*)c->in2.d();
+  G1Affine* d_add = addend ? (G1Affine*)c->addend.d() : nullptr;
+  G1Affine* d_out = (G1Affine*)c->out.d();
   CDL_CUDA(c, cudaMemcpyAsync(d_in, in, n * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
   CDL_CUDA(c, cudaMemcpyAsync(d_s, s, ns * sizeof(Fr), cudaMemcpyHostToDevice, c->stream));
   if (addend) CDL_CUDA(c, cudaMemcpyAsync(d_add, addend, n * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
@@ -292,9 +293,10 @@ int32_t cdl_g1_batch_to_affine(cdl_ctx* c, const cdl_g1_jac* in, size_t n, cdl_g
   if (n == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  G1Jac* d_in = (G1Jac*)c->buf(0, n * sizeof(G1Jac));
-  G1Affine* d_out = (G1Affine*)c->buf(4, n * sizeof(G1Affine));
-  if (!d_in || !d_out) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->in.grow(n * sizeof(G1Jac), c->stream) || !c->out.grow(n * sizeof(G1Affine), c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  G1Jac* d_in = (G1Jac*)c->in.d();
+  G1Affine* d_out = (G1Affine*)c->out.d();
   CDL_CUDA(c, cudaMemcpyAsync(d_in, in, n * sizeof(G1Jac), cudaMemcpyHostToDevice, c->stream));
   launch_jac_to_affine(d_in, d_out, (int)n, c->stream);
   CDL_CUDA(c, cudaGetLastError());
@@ -309,9 +311,10 @@ int32_t cdl_g1_compress(cdl_ctx* c, const cdl_g1_affine* in, size_t n, uint8_t* 
   if (n == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  G1Affine* d_in = (G1Affine*)c->buf(0, n * sizeof(G1Affine));
-  uint8_t* d_out = (uint8_t*)c->buf(4, n * 48);
-  if (!d_in || !d_out) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->in.grow(n * sizeof(G1Affine), c->stream) || !c->out.grow(n * 48, c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  G1Affine* d_in = (G1Affine*)c->in.d();
+  uint8_t* d_out = (uint8_t*)c->out.d();
   CDL_CUDA(c, cudaMemcpyAsync(d_in, in, n * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
   launch_compress(d_in, d_out, (int)n, c->stream);
   CDL_CUDA(c, cudaGetLastError());
@@ -325,10 +328,11 @@ int32_t cdl_g1_decompress(cdl_ctx* c, const uint8_t* in48, size_t n, cdl_g1_affi
   if (n == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  uint8_t* d_in = (uint8_t*)c->buf(0, n * 48);
-  G1Affine* d_out = (G1Affine*)c->buf(4, n * sizeof(G1Affine));
-  uint8_t* d_st = (uint8_t*)c->buf(3, n);
-  if (!d_in || !d_out || !d_st) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->in.grow(n * 48, c->stream) || !c->out.grow(n * sizeof(G1Affine), c->stream) || !c->status.grow(n, c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  uint8_t* d_in = (uint8_t*)c->in.d();
+  G1Affine* d_out = (G1Affine*)c->out.d();
+  uint8_t* d_st = (uint8_t*)c->status.d();
   CDL_CUDA(c, cudaMemcpyAsync(d_in, in48, n * 48, cudaMemcpyHostToDevice, c->stream));
   launch_decompress(d_in, d_out, d_st, (int)n, c->stream);
   CDL_CUDA(c, cudaGetLastError());
@@ -346,10 +350,11 @@ int32_t cdl_fp_mul(cdl_ctx* c, const cdl_fp* a, const cdl_fp* b, size_t n, cdl_f
   if (n == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  Fp* d_a = (Fp*)c->buf(0, n * sizeof(Fp));
-  Fp* d_b = (Fp*)c->buf(1, n * sizeof(Fp));
-  Fp* d_o = (Fp*)c->buf(4, n * sizeof(Fp));
-  if (!d_a || !d_b || !d_o) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->in.grow(n * sizeof(Fp), c->stream) || !c->in2.grow(n * sizeof(Fp), c->stream) || !c->out.grow(n * sizeof(Fp), c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  Fp* d_a = (Fp*)c->in.d();
+  Fp* d_b = (Fp*)c->in2.d();
+  Fp* d_o = (Fp*)c->out.d();
   CDL_CUDA(c, cudaMemcpyAsync(d_a, a, n * sizeof(Fp), cudaMemcpyHostToDevice, c->stream));
   CDL_CUDA(c, cudaMemcpyAsync(d_b, b, n * sizeof(Fp), cudaMemcpyHostToDevice, c->stream));
   launch_fp_mul(d_a, d_b, d_o, (int)n, c->stream);
@@ -370,8 +375,8 @@ int32_t cdl_int_peak_cfg(cdl_ctx* c, int kind, int iters, int blocks_per_sm, int
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   const int blocks = c->sm_count * blocks_per_sm;
-  void* d = c->buf(4, (size_t)blocks * tpb * sizeof(Fp));
-  if (!d) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->out.grow((size_t)blocks * tpb * sizeof(Fp), c->stream)) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  void* d = c->out.d();
   float best = 1e30f;
   for (int rep = 0; rep < 4; rep++) {  // rep 0 is the warm-up
     CDL_CUDA(c, cudaEventRecord(c->ev0, c->stream));

@@ -60,24 +60,24 @@ int32_t Engine::base_mul(const cdl_g1_affine& base, const Fr* sc, size_t n, cdl_
                         cdl::fixed_table_bytes(1));
     }
   }
-  char* d_scr = (char*)s_base_.d;
+  char* d_scr = (char*)s_base_.d();
   const cdl::G1Affine* d_base = (const cdl::G1Affine*)d_scr;
   uint32_t* d_status = (uint32_t*)(d_scr + kOffStatus);
   cdl::G1Jac* wjac = (cdl::G1Jac*)(d_scr + kOffWjac);
   cdl::G1Affine* waff = (cdl::G1Affine*)(d_scr + kOffWaff);
   cdl::G1Affine* copies = (cdl::G1Affine*)(d_scr + kOffCopies);
-  cdl::Fr* d_sc = (cdl::Fr*)s_sc_.d;
-  cdl::G1Affine* d_out = (cdl::G1Affine*)s_out_.d;
-  uint8_t* d_enc = (uint8_t*)s_enc_.d;
+  cdl::Fr* d_sc = (cdl::Fr*)s_sc_.d();
+  cdl::G1Affine* d_out = (cdl::G1Affine*)s_out_.d();
+  uint8_t* d_enc = (uint8_t*)s_enc_.d();
   const bool check = !hit;  // a cached table's base passed the check when its table was built
-  memcpy(s_base_.h, &base, sizeof base);
+  memcpy(s_base_.h(), &base, sizeof base);
   uint32_t status = 0;
   for (size_t c0 = 0; c0 < n; c0 += kBaseMulChunk) {
     const size_t m = std::min(n - c0, kBaseMulChunk);
     const bool first = c0 == 0;
-    memcpy(s_sc_.h, sc + c0, m * sizeof(Fr));
-    if (first) CDL_CUDA(ctx_, cudaMemcpyAsync(s_base_.d, s_base_.h, sizeof base, cudaMemcpyHostToDevice, ctx_->stream));
-    CDL_CUDA(ctx_, cudaMemcpyAsync(d_sc, s_sc_.h, m * sizeof(Fr), cudaMemcpyHostToDevice, ctx_->stream));
+    memcpy(s_sc_.h(), sc + c0, m * sizeof(Fr));
+    if (first) CDL_CUDA(ctx_, cudaMemcpyAsync(s_base_.d(), s_base_.h(), sizeof base, cudaMemcpyHostToDevice, ctx_->stream));
+    CDL_CUDA(ctx_, cudaMemcpyAsync(d_sc, s_sc_.h(), m * sizeof(Fr), cudaMemcpyHostToDevice, ctx_->stream));
     tick();
     uint64_t kernels = 0;
     double bytes = 32.0 * m + (out ? 96.0 * m : 0.0) + (out48 ? 48.0 * m : 0.0);
@@ -108,12 +108,12 @@ int32_t Engine::base_mul(const cdl_g1_affine& base, const Fr* sc, size_t n, cdl_
     launches += kernels - 1;  // tock counted one
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess && first && check)
-      e = cudaMemcpyAsync((char*)s_base_.h + kOffStatus, d_status, 4, cudaMemcpyDeviceToHost, ctx_->stream);
-    if (e == cudaSuccess && out) e = cudaMemcpyAsync(s_out_.h, d_out, m * sizeof(cdl::G1Affine), cudaMemcpyDeviceToHost, ctx_->stream);
-    if (e == cudaSuccess && out48) e = cudaMemcpyAsync(s_enc_.h, d_enc, m * 48, cudaMemcpyDeviceToHost, ctx_->stream);
+      e = cudaMemcpyAsync((char*)s_base_.h() + kOffStatus, d_status, 4, cudaMemcpyDeviceToHost, ctx_->stream);
+    if (e == cudaSuccess && out) e = cudaMemcpyAsync(s_out_.h(), d_out, m * sizeof(cdl::G1Affine), cudaMemcpyDeviceToHost, ctx_->stream);
+    if (e == cudaSuccess && out48) e = cudaMemcpyAsync(s_enc_.h(), d_enc, m * 48, cudaMemcpyDeviceToHost, ctx_->stream);
     if (e == cudaSuccess) e = ctx_->sync_stream();
     finish_timing();
-    if (e == cudaSuccess && first && check) memcpy(&status, (char*)s_base_.h + kOffStatus, 4);
+    if (e == cudaSuccess && first && check) memcpy(&status, (char*)s_base_.h() + kOffStatus, 4);
     if (e != cudaSuccess || status) {
       if (build) cudaFree(tab);
       if (e != cudaSuccess)
@@ -126,8 +126,8 @@ int32_t Engine::base_mul(const cdl_g1_affine& base, const Fr* sc, size_t n, cdl_
       base_tabs_.push_back(BaseTable{base, tab, 0});
       hit = &base_tabs_.back();
     }
-    if (out) memcpy(out + c0, s_out_.h, m * sizeof(cdl::G1Affine));
-    if (out48) memcpy(out48 + 48 * c0, s_enc_.h, m * 48);
+    if (out) memcpy(out + c0, s_out_.h(), m * sizeof(cdl::G1Affine));
+    if (out48) memcpy(out48 + 48 * c0, s_enc_.h(), m * 48);
   }
   if (hit) hit->used = ++base_clock_;
   return CDL_OK;

@@ -90,10 +90,27 @@ int32_t big_msm_on_device(cdl_ctx* c, const G1Affine* d_pts, const Fr* d_sc, siz
   if (big_msm_entries(d) >= ((uint64_t)1 << 32))
     return c->fail(CDL_ERR_TOO_LARGE, "msm: %zu terms x %d windows exceed 2^32 - 1 sorted entries; use more ranks or a wider window",
                    n, d.nlocal);
-  void* scr = c->buf(7, big_msm_scratch_bytes(d));
-  if (!scr) return c->fail(CDL_ERR_CUDA, "msm scratch allocation of %zu bytes failed", big_msm_scratch_bytes(d));
-  cudaError_t e = launch_big_msm(d_pts, d_sc, d, normalize, scr, c->sm_count, d_out, c->stream);
+  if (!c->msm_scratch.grow(big_msm_scratch_bytes(d), c->stream))
+    return c->fail(CDL_ERR_CUDA, "msm scratch allocation of %zu bytes failed", big_msm_scratch_bytes(d));
+  cudaError_t e = launch_big_msm(d_pts, d_sc, d, normalize, c->msm_scratch.d(), c->sm_count, d_out, c->stream);
   if (e != cudaSuccess) return c->fail(CDL_ERR_CUDA, "large-MSM launch failed: %s", cudaGetErrorString(e));
+  return CDL_OK;
+}
+
+// An MSM of host vectors: the points and scalars go to the context's input buffers, `msm(d_pts, d_sc, d_out)`
+// leaves the result in its output buffer, and that G1Jac is downloaded to `out`.  Caller holds the context mutex.
+template <class Msm>
+int32_t msm_of_host_vectors(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out,
+                            Msm&& msm) {
+  if (!c->in.grow(n * sizeof(G1Affine), c->stream) || !c->in2.grow(n * sizeof(Fr), c->stream) ||
+      !c->out.grow(sizeof(G1Jac), c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  CDL_CUDA(c, cudaMemcpyAsync(c->in.d(), points, n * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
+  CDL_CUDA(c, cudaMemcpyAsync(c->in2.d(), scalars, n * sizeof(Fr), cudaMemcpyHostToDevice, c->stream));
+  int32_t rc = msm((const G1Affine*)c->in.d(), (const Fr*)c->in2.d(), (G1Jac*)c->out.d());
+  if (rc) return rc;
+  CDL_CUDA(c, cudaMemcpyAsync(out, c->out.d(), sizeof(G1Jac), cudaMemcpyDeviceToHost, c->stream));
+  CDL_CUDA(c, cudaStreamSynchronize(c->stream));
   return CDL_OK;
 }
 
@@ -101,17 +118,9 @@ int32_t big_msm_on_device(cdl_ctx* c, const G1Affine* d_pts, const Fr* d_sc, siz
 
 // used by cdl_g1_msm (capi.cu) above kBigMsmThreshold terms; caller holds the context mutex
 extern "C" int32_t cdl_big_msm_host_(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out) {
-  G1Affine* d_pts = (G1Affine*)c->buf(0, n * sizeof(G1Affine));
-  Fr* d_sc = (Fr*)c->buf(1, n * sizeof(Fr));
-  G1Jac* d_out = (G1Jac*)c->buf(4, sizeof(G1Jac));
-  if (!d_pts || !d_sc || !d_out) return c->fail(CDL_ERR_CUDA, "device allocation failed");
-  CDL_CUDA(c, cudaMemcpyAsync(d_pts, points, n * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
-  CDL_CUDA(c, cudaMemcpyAsync(d_sc, scalars, n * sizeof(Fr), cudaMemcpyHostToDevice, c->stream));
-  int32_t rc = big_msm_on_device(c, d_pts, d_sc, n, 0, 1, 1, d_out);
-  if (rc) return rc;
-  CDL_CUDA(c, cudaMemcpyAsync(out, d_out, sizeof(G1Jac), cudaMemcpyDeviceToHost, c->stream));
-  CDL_CUDA(c, cudaStreamSynchronize(c->stream));
-  return CDL_OK;
+  return msm_of_host_vectors(c, points, scalars, n, out, [&](const G1Affine* d_pts, const Fr* d_sc, G1Jac* d_out) {
+    return big_msm_on_device(c, d_pts, d_sc, n, 0, 1, 1, d_out);
+  });
 }
 
 extern "C" {
@@ -279,8 +288,8 @@ static int32_t msm_sharded_device_locked(cdl_ctx* c, const cdl_g1_affine* d_poin
   CDL_CUDA(c, cudaSetDevice(c->device));
   const int world = c->comm_world, rank = c->comm_rank;
   if (world > 1 && !c->nccl_comm) return c->fail(CDL_ERR_INVALID_ARG, "cdl_comm_init has not been called");
-  G1Jac* d_part = (G1Jac*)c->buf(6, (size_t)(world + 1) * sizeof(G1Jac));
-  if (!d_part) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  if (!c->partials.grow((size_t)(world + 1) * sizeof(G1Jac), c->stream)) return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  G1Jac* d_part = (G1Jac*)c->partials.d();
   CDL_CUDA(c, cudaEventRecord(c->ev0, c->stream));
   if (world == 1) {
     int32_t rc = big_msm_on_device(c, (const G1Affine*)d_points, (const Fr*)d_scalars, n, 0, 1, 1, (G1Jac*)d_out);
@@ -339,17 +348,9 @@ int32_t cdl_g1_msm_sharded(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr
   // one lock across staging, MSM and download: the staging slots belong to the context
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
-  G1Affine* d_pts = (G1Affine*)c->buf(0, n * sizeof(G1Affine));
-  Fr* d_sc = (Fr*)c->buf(1, n * sizeof(Fr));
-  G1Jac* d_out = (G1Jac*)c->buf(4, sizeof(G1Jac));
-  if (!d_pts || !d_sc || !d_out) return c->fail(CDL_ERR_CUDA, "device allocation failed");
-  CDL_CUDA(c, cudaMemcpyAsync(d_pts, points, n * sizeof(G1Affine), cudaMemcpyHostToDevice, c->stream));
-  CDL_CUDA(c, cudaMemcpyAsync(d_sc, scalars, n * sizeof(Fr), cudaMemcpyHostToDevice, c->stream));
-  int32_t rc = msm_sharded_device_locked(c, (const cdl_g1_affine*)d_pts, (const cdl_fr*)d_sc, n, (cdl_g1_jac*)d_out, nullptr);
-  if (rc) return rc;
-  CDL_CUDA(c, cudaMemcpyAsync(out, d_out, sizeof(G1Jac), cudaMemcpyDeviceToHost, c->stream));
-  CDL_CUDA(c, cudaStreamSynchronize(c->stream));
-  return CDL_OK;
+  return msm_of_host_vectors(c, points, scalars, n, out, [&](const G1Affine* d_pts, const Fr* d_sc, G1Jac* d_out) {
+    return msm_sharded_device_locked(c, (const cdl_g1_affine*)d_pts, (const cdl_fr*)d_sc, n, (cdl_g1_jac*)d_out, nullptr);
+  });
 }
 
 }  // extern "C"

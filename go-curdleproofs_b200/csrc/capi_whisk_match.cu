@@ -25,21 +25,8 @@ const uint8_t kInfEnc[48] = {0xc0};  // compressed point at infinity
 // affine).  Grow-only and kept by the engine, like the pool; false if it cannot be had.
 bool Engine::match_scratch(uint32_t tile) {
   constexpr size_t W = cdl::fb_windows(cdl::kMatchC);
-  const size_t bytes = cdl::fixed_table_bytes<cdl::kMatchC>(tile) + tile * W * (sizeof(cdl::G1Jac) + sizeof(cdl::G1Affine));
-  if (bytes <= match_cap_) return true;
-  if (d_match_) {
-    cudaStreamSynchronize(ctx_->stream);
-    cudaFree(d_match_);
-  }
-  d_match_ = nullptr;
-  match_cap_ = 0;
-  if (cudaMalloc(&d_match_, bytes) != cudaSuccess) {
-    cudaGetLastError();
-    d_match_ = nullptr;
-    return false;
-  }
-  match_cap_ = bytes;
-  return true;
+  return d_match_.grow(cdl::fixed_table_bytes<cdl::kMatchC>(tile) + tile * W * (sizeof(cdl::G1Jac) + sizeof(cdl::G1Affine)),
+                       ctx_->stream);
 }
 
 int32_t Engine::match_trackers(uint32_t T, const Fr* ks, uint32_t V, int32_t* owner) {
@@ -49,15 +36,15 @@ int32_t Engine::match_trackers(uint32_t T, const Fr* ks, uint32_t V, int32_t* ow
   // without room for the tables the shared-scalar path gives the same owners
   const bool tables = V >= kMatchTableMinKeys && match_scratch(tile);
   constexpr uint32_t W = cdl::fb_windows(cdl::kMatchC);
-  cdl::G1Affine* tab = (cdl::G1Affine*)d_match_;
-  cdl::G1Jac* wjac = (cdl::G1Jac*)((char*)d_match_ + cdl::fixed_table_bytes<cdl::kMatchC>(tile));
+  cdl::G1Affine* tab = (cdl::G1Affine*)d_match_.d();
+  cdl::G1Jac* wjac = (cdl::G1Jac*)((char*)d_match_.d() + cdl::fixed_table_bytes<cdl::kMatchC>(tile));
   cdl::G1Affine* wbase = (cdl::G1Affine*)(wjac + (size_t)tile * W);
-  memcpy(s_sc_.h, ks, (size_t)V * sizeof(Fr));
-  cdl::Fr* d_ks = (cdl::Fr*)s_sc_.d;
-  int32_t* d_owner = (int32_t*)s_out_.d;
-  const cdl::G1Affine* rg = d_pool_;
-  const cdl::G1Affine* krg = d_pool_ + T;
-  CDL_CUDA(ctx_, cudaMemcpyAsync(d_ks, s_sc_.h, (size_t)V * sizeof(Fr), cudaMemcpyHostToDevice, ctx_->stream));
+  memcpy(s_sc_.h(), ks, (size_t)V * sizeof(Fr));
+  cdl::Fr* d_ks = (cdl::Fr*)s_sc_.d();
+  int32_t* d_owner = (int32_t*)s_out_.d();
+  const cdl::G1Affine* rg = d_pool();
+  const cdl::G1Affine* krg = d_pool() + T;
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_ks, s_sc_.h(), (size_t)V * sizeof(Fr), cudaMemcpyHostToDevice, ctx_->stream));
   tick();
   cdl::launch_match_prep(d_ks, V, d_owner, T, ctx_->stream);
   uint64_t kernels = 1;
@@ -79,10 +66,10 @@ int32_t Engine::match_trackers(uint32_t T, const Fr* ks, uint32_t V, int32_t* ow
   tock(1, 3193.0 * T * (double)V, 196.0 * T + 32.0 * V);
   launches += kernels - 1;  // tock counted one
   CDL_CUDA(ctx_, cudaGetLastError());
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_out_.h, d_owner, (size_t)T * 4, cudaMemcpyDeviceToHost, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_out_.h(), d_owner, (size_t)T * 4, cudaMemcpyDeviceToHost, ctx_->stream));
   CDL_CUDA(ctx_, ctx_->sync_stream());
   finish_timing();
-  memcpy(owner, s_out_.h, (size_t)T * 4);
+  memcpy(owner, s_out_.h(), (size_t)T * 4);
   return CDL_OK;
 }
 

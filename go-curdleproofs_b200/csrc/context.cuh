@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "../../include/curdle_b200.h"
+#include "scratch.cuh"
 
 struct cdl_ctx {
   int device = 0;
@@ -56,23 +57,14 @@ struct cdl_ctx {
   size_t dev_slot = 0;           // lanes: the slot of root()->slots they belong to
   int n_lanes = 4;               // CDL_LANES / cdl_set_lanes: lanes per slot
   cdl_ctx* root() { return parent ? parent : this; }
-  static constexpr int kSlots = 8;
-  void* slot[kSlots] = {};
-  size_t cap[kSlots] = {};
-
-  // grow-only scratch buffer `i` of at least `bytes`
-  void* buf(int i, size_t bytes) {
-    if (bytes == 0) bytes = 16;
-    if (cap[i] >= bytes) return slot[i];
-    if (slot[i]) { cudaStreamSynchronize(stream); cudaFree(slot[i]); slot[i] = nullptr; cap[i] = 0; }
-    size_t want = bytes + bytes / 2;
-    if (cudaMalloc(&slot[i], want) != cudaSuccess) { slot[i] = nullptr; return nullptr; }
-    cap[i] = want;
-    return slot[i];
-  }
-  void free_all() {
-    for (int i = 0; i < kSlots; i++) if (slot[i]) { cudaFree(slot[i]); slot[i] = nullptr; cap[i] = 0; }
-  }
+  // device scratch of the host-pointer calls (capi.cu, capi_msm.cu), freed with the context
+  DeviceScratch in;           // first input
+  DeviceScratch in2;          // second input, or the scalars
+  DeviceScratch addend;
+  DeviceScratch status;       // per-point decode status
+  DeviceScratch out;
+  DeviceScratch partials;     // the sharded MSM's per-rank partial sums
+  DeviceScratch msm_scratch;  // the large MSM's working memory
   int32_t fail(int32_t code, const char* fmt, ...) {
     char tmp[512];
     va_list ap;
@@ -84,10 +76,14 @@ struct cdl_ctx {
   }
 };
 
-#define CDL_CUDA(ctx, call)                                                                   \
-  do {                                                                                        \
-    cudaError_t e__ = (call);                                                                 \
-    if (e__ != cudaSuccess)                                                                   \
+// On failure the error is also taken off the thread's last-error slot: a call made after this one checks
+// cudaGetLastError() after its launches and must not report this call's error (a sticky error still fails it).
+#define CDL_CUDA(ctx, call)                                                                     \
+  do {                                                                                          \
+    cudaError_t e__ = (call);                                                                   \
+    if (e__ != cudaSuccess) {                                                                   \
+      cudaGetLastError();                                                                       \
       return (ctx)->fail(CDL_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), \
-                         __FILE__, __LINE__);                                                 \
+                         __FILE__, __LINE__);                                                   \
+    }                                                                                           \
   } while (0)

@@ -66,17 +66,8 @@ Engine::~Engine() {
     fprintf(stderr, "[cdl profile] engine %p (lane %d): total %.1f ms = parallel host %.1f + gpu stages %.1f (staging copies %.1f) + serial host %.1f\n",
             (void*)this, ctx_->parent ? 1 : 0, prof.total * 1e3, prof.par * 1e3, prof.gpu * 1e3, prof.copy * 1e3,
             (prof.total - prof.par - prof.gpu) * 1e3);
-  cudaSetDevice(ctx_->device);
-  if (d_pool_) cudaFree(d_pool_);
-  if (d_win_) cudaFree(d_win_);
-  if (d_match_) cudaFree(d_match_);
-  if (d_bv_) cudaFree(d_bv_);
+  cudaSetDevice(ctx_->device);  // before the members free their memory
   for (BaseTable& b : base_tabs_) cudaFree(b.tab);
-  for (Staging* s : {&s_idx_, &s_sc_, &s_task_, &s_out_, &s_ops_, &s_enc_, &s_st_, &s_jac_, &s_sub_, &s_t2_, &s_cr_, &s_vs_, &s_as_, &s_fsub_, &s_bv_,
-                     &s_in_, &s_base_}) {
-    if (s->h) cudaFreeHost(s->h);
-    if (s->d) cudaFree(s->d);
-  }
 }
 
 // SURVEY.md §8d: modmul(N) = min_c [6 N W + 28 2^(c-1) W + 9 c (W-1) + 14 W], W = ceil(256/c)
@@ -111,30 +102,13 @@ void Engine::finish_timing() {
 }
 
 int32_t Engine::reserve(Staging& s, size_t bytes) {
-  if (bytes <= s.cap) return CDL_OK;
-  cudaStreamSynchronize(ctx_->stream);
-  if (s.h) cudaFreeHost(s.h);
-  if (s.d) cudaFree(s.d);
-  s.h = s.d = nullptr;
-  s.cap = 0;
-  size_t want = bytes + bytes / 2 + 256;
-  if (cudaMallocHost(&s.h, want) != cudaSuccess || cudaMalloc(&s.d, want) != cudaSuccess)
-    return ctx_->fail(CDL_ERR_CUDA, "engine staging allocation of %zu bytes failed", want);
-  s.cap = want;
-  return CDL_OK;
+  if (s.grow(bytes, ctx_->stream)) return CDL_OK;
+  return ctx_->fail(CDL_ERR_CUDA, "engine staging allocation of %zu bytes failed", bytes);
 }
 
 int32_t Engine::ensure_pool(size_t npoints) {
-  if (npoints <= pool_cap_) return CDL_OK;
-  cudaStreamSynchronize(ctx_->stream);
-  if (d_pool_) cudaFree(d_pool_);
-  d_pool_ = nullptr;
-  pool_cap_ = 0;
-  size_t want = npoints + npoints / 4;
-  if (cudaMalloc(&d_pool_, want * sizeof(G1Affine)) != cudaSuccess)
-    return ctx_->fail(CDL_ERR_CUDA, "point pool allocation of %zu points failed", want);
-  pool_cap_ = want;
-  return CDL_OK;
+  if (pool_mem_.grow(npoints * sizeof(G1Affine), ctx_->stream)) return CDL_OK;
+  return ctx_->fail(CDL_ERR_CUDA, "point pool allocation of %zu points failed", npoints);
 }
 
 int32_t Engine::load_crs(const Layout& L, const cdl_crs* crs) {
@@ -144,7 +118,7 @@ int32_t Engine::load_crs(const Layout& L, const cdl_crs* crs) {
     pts = crs->points_on(ctx_->dev_slot);
   }
   if (!pts) return ctx_->fail(CDL_ERR_CUDA, "crs replica for device slot %zu could not be made", ctx_->dev_slot);
-  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_, pts, (size_t)L.crs_size * sizeof(G1Affine), cudaMemcpyDeviceToDevice,
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool(), pts, (size_t)L.crs_size * sizeof(G1Affine), cudaMemcpyDeviceToDevice,
                                  ctx_->stream));
   return CDL_OK;
 }
@@ -188,27 +162,27 @@ void Engine::select_fixed(const Layout& L, const cdl_crs* crs, size_t B) {
 
 int32_t Engine::upload_points(uint32_t dst, const void* host_affine, size_t count) {
   if (!count) return CDL_OK;
-  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_ + dst, host_affine, count * sizeof(G1Affine), cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool() + dst, host_affine, count * sizeof(G1Affine), cudaMemcpyHostToDevice, ctx_->stream));
   CDL_CUDA(ctx_, ctx_->sync_stream());  // caller memory is pageable and may go away
   return CDL_OK;
 }
 
 int32_t Engine::download_points(uint32_t src, void* host_affine, size_t count) {
   if (!count) return CDL_OK;
-  CDL_CUDA(ctx_, cudaMemcpyAsync(host_affine, d_pool_ + src, count * sizeof(G1Affine), cudaMemcpyDeviceToHost, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(host_affine, d_pool() + src, count * sizeof(G1Affine), cudaMemcpyDeviceToHost, ctx_->stream));
   CDL_CUDA(ctx_, ctx_->sync_stream());
   return CDL_OK;
 }
 
 int32_t Engine::copy_points(uint32_t dst, uint32_t src, size_t count) {
   if (!count) return CDL_OK;
-  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_ + dst, d_pool_ + src, count * sizeof(G1Affine), cudaMemcpyDeviceToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool() + dst, d_pool() + src, count * sizeof(G1Affine), cudaMemcpyDeviceToDevice, ctx_->stream));
   return CDL_OK;
 }
 
 int32_t Engine::set_infinity(uint32_t dst, size_t count) {
   if (!count) return CDL_OK;
-  CDL_CUDA(ctx_, cudaMemsetAsync(d_pool_ + dst, 0, count * sizeof(G1Affine), ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemsetAsync(d_pool() + dst, 0, count * sizeof(G1Affine), ctx_->stream));
   return CDL_OK;
 }
 
@@ -220,9 +194,9 @@ int32_t Engine::copy_ranges(const std::vector<cdl::CopyRange>& ranges) {
   CDL_CUDA(ctx_, ctx_->sync_stream());  // a previous copy_ranges may still be reading s_cr_
   int32_t rc = reserve(s_cr_, n * sizeof(cdl::CopyRange));
   if (rc) return rc;
-  memcpy(s_cr_.h, ranges.data(), n * sizeof(cdl::CopyRange));
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_cr_.d, s_cr_.h, n * sizeof(cdl::CopyRange), cudaMemcpyHostToDevice, ctx_->stream));
-  cdl::launch_copy_ranges(d_pool_, (const cdl::CopyRange*)s_cr_.d, (int)n, ctx_->stream);
+  memcpy(s_cr_.h(), ranges.data(), n * sizeof(cdl::CopyRange));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_cr_.d(), s_cr_.h(), n * sizeof(cdl::CopyRange), cudaMemcpyHostToDevice, ctx_->stream));
+  cdl::launch_copy_ranges(d_pool(), (const cdl::CopyRange*)s_cr_.d(), (int)n, ctx_->stream);
   CDL_CUDA(ctx_, cudaGetLastError());
   launches++;
   return CDL_OK;
@@ -248,19 +222,19 @@ int32_t Engine::load_instances(const Layout& L, const std::vector<uint32_t>& sel
     return rc;
   {
     ProfScope pc(prof.copy);
-    G1Affine* h = (G1Affine*)s_in_.h;
+    G1Affine* h = (G1Affine*)s_in_.h();
     pool_.parallel_for(B, std::function<void(size_t)>([&](size_t j) {
       for (uint32_t a = 0; a < npts; a++)
         memcpy(h + j * per + (size_t)a * L.ell, pts[a] + (size_t)sel[j] * L.ell, (size_t)L.ell * sizeof(G1Affine));
     }));
     if (M)
-      for (size_t j = 0; j < B; j++) memcpy((cdl::G1Jac*)s_jac_.h + j, M + sel[j], sizeof(cdl::G1Jac));
+      for (size_t j = 0; j < B; j++) memcpy((cdl::G1Jac*)s_jac_.h() + j, M + sel[j], sizeof(cdl::G1Jac));
   }
-  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool_ + tail, s_in_.h, B * per * sizeof(G1Affine), cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(d_pool() + tail, s_in_.h(), B * per * sizeof(G1Affine), cudaMemcpyHostToDevice, ctx_->stream));
   if (M) {
-    CDL_CUDA(ctx_, cudaMemcpyAsync(s_jac_.d, s_jac_.h, B * sizeof(cdl::G1Jac), cudaMemcpyHostToDevice, ctx_->stream));
+    CDL_CUDA(ctx_, cudaMemcpyAsync(s_jac_.d(), s_jac_.h(), B * sizeof(cdl::G1Jac), cudaMemcpyHostToDevice, ctx_->stream));
     tick();
-    cdl::launch_jac_to_affine((const cdl::G1Jac*)s_jac_.d, d_pool_ + tail_m, (int)B, ctx_->stream);
+    cdl::launch_jac_to_affine((const cdl::G1Jac*)s_jac_.d(), d_pool() + tail_m, (int)B, ctx_->stream);
     tock(3, 0, 240.0 * B);
     CDL_CUDA(ctx_, cudaGetLastError());
   }
@@ -285,16 +259,16 @@ int32_t Engine::compress(const std::vector<uint32_t>& src, std::vector<uint8_t>&
   if (!n) return CDL_OK;
   int32_t rc;
   if ((rc = reserve(s_idx_, n * 4)) || (rc = reserve(s_out_, n * 48))) return rc;
-  memcpy(s_idx_.h, src.data(), n * 4);
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_idx_.d, s_idx_.h, n * 4, cudaMemcpyHostToDevice, ctx_->stream));
+  memcpy(s_idx_.h(), src.data(), n * 4);
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_idx_.d(), s_idx_.h(), n * 4, cudaMemcpyHostToDevice, ctx_->stream));
   tick();
-  cdl::launch_compress_idx(d_pool_, (const uint32_t*)s_idx_.d, (uint8_t*)s_out_.d, (int)n, ctx_->stream);
+  cdl::launch_compress_idx(d_pool(), (const uint32_t*)s_idx_.d(), (uint8_t*)s_out_.d(), (int)n, ctx_->stream);
   tock(3, 3.0 * n, 148.0 * n);
   CDL_CUDA(ctx_, cudaGetLastError());
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_out_.h, s_out_.d, n * 48, cudaMemcpyDeviceToHost, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_out_.h(), s_out_.d(), n * 48, cudaMemcpyDeviceToHost, ctx_->stream));
   CDL_CUDA(ctx_, ctx_->sync_stream());
   finish_timing();
-  memcpy(out48.data(), s_out_.h, n * 48);
+  memcpy(out48.data(), s_out_.h(), n * 48);
   return CDL_OK;
 }
 
@@ -305,19 +279,19 @@ int32_t Engine::decompress(const uint8_t* enc48, const std::vector<uint32_t>& ds
   if (!n) return CDL_OK;
   int32_t rc;
   if ((rc = reserve(s_idx_, n * 4)) || (rc = reserve(s_enc_, n * 48)) || (rc = reserve(s_st_, n))) return rc;
-  memcpy(s_idx_.h, dst.data(), n * 4);
-  memcpy(s_enc_.h, enc48, n * 48);
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_idx_.d, s_idx_.h, n * 4, cudaMemcpyHostToDevice, ctx_->stream));
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_enc_.d, s_enc_.h, n * 48, cudaMemcpyHostToDevice, ctx_->stream));
+  memcpy(s_idx_.h(), dst.data(), n * 4);
+  memcpy(s_enc_.h(), enc48, n * 48);
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_idx_.d(), s_idx_.h(), n * 4, cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_enc_.d(), s_enc_.h(), n * 48, cudaMemcpyHostToDevice, ctx_->stream));
   tick();
-  cdl::launch_decompress_idx((const uint8_t*)s_enc_.d, d_pool_, (const uint32_t*)s_idx_.d, (uint8_t*)s_st_.d, (int)n, ctx_->stream);
+  cdl::launch_decompress_idx((const uint8_t*)s_enc_.d(), d_pool(), (const uint32_t*)s_idx_.d(), (uint8_t*)s_st_.d(), (int)n, ctx_->stream);
   // sqrt = one fixed 381-bit exponentiation (~480 modmul) + subgroup check [r]P (3193 by the §8d convention)
   tock(2, (480.0 + 3193.0) * n, 148.0 * n);
   CDL_CUDA(ctx_, cudaGetLastError());
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_st_.h, s_st_.d, n, cudaMemcpyDeviceToHost, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_st_.h(), s_st_.d(), n, cudaMemcpyDeviceToHost, ctx_->stream));
   CDL_CUDA(ctx_, ctx_->sync_stream());
   finish_timing();
-  memcpy(status.data(), s_st_.h, n);
+  memcpy(status.data(), s_st_.h(), n);
   return CDL_OK;
 }
 
@@ -328,7 +302,7 @@ int32_t Engine::run_msm(MsmStage& st, const MsmBefore& before, const G1Affine* p
   size_t nt = st.tasks.size(), nterm = st.idx.size();
   st.out48.resize(nt * 48);
   if (!nt) return CDL_OK;
-  if (!points) points = d_pool_;
+  if (!points) points = d_pool();
   size_t max_terms = 0;
   for (auto& t : st.tasks) max_terms = std::max<size_t>(max_terms, t.term_cnt);
   int32_t rc;
@@ -341,13 +315,13 @@ int32_t Engine::run_msm(MsmStage& st, const MsmBefore& before, const G1Affine* p
   std::vector<uint32_t> fixed_tasks;  // tasks whose CRS terms go through the fixed-base tables
   {
     ProfScope pc(prof.copy);
-    memcpy(s_idx_.h, st.idx.data(), nterm * 4);
-    memcpy(s_sc_.h, st.sc.data(), nterm * 32);
-    memcpy(s_task_.h, st.tasks.data(), nt * sizeof(MsmTask));
+    memcpy(s_idx_.h(), st.idx.data(), nterm * 4);
+    memcpy(s_sc_.h(), st.sc.data(), nterm * 32);
+    memcpy(s_task_.h(), st.tasks.data(), nt * sizeof(MsmTask));
     if (throughput && fixed_.tab) {
       // terms on CRS points go through the fixed-base tables when their task holds enough of them to pay
       // for the extra pass (a chunk's lanes share 22 look-ups per 32 such terms; a lone term costs as much)
-      uint32_t* idx = (uint32_t*)s_idx_.h;
+      uint32_t* idx = (uint32_t*)s_idx_.h();
       for (size_t j = 0; j < nt; j++) {
         const MsmTask& t = st.tasks[j];
         uint32_t cnt = 0;
@@ -359,12 +333,12 @@ int32_t Engine::run_msm(MsmStage& st, const MsmBefore& before, const G1Affine* p
       }
     }
   }
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_idx_.d, s_idx_.h, nterm * 4, cudaMemcpyHostToDevice, ctx_->stream));
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_sc_.d, s_sc_.h, nterm * 32, cudaMemcpyHostToDevice, ctx_->stream));
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_task_.d, s_task_.h, nt * sizeof(MsmTask), cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_idx_.d(), s_idx_.h(), nterm * 4, cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_sc_.d(), s_sc_.h(), nterm * 32, cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_task_.d(), s_task_.h(), nt * sizeof(MsmTask), cudaMemcpyHostToDevice, ctx_->stream));
   if (before) {
     bool done = false;
-    int32_t brc = before((const uint32_t*)s_idx_.d, (cdl::Fr*)s_sc_.d, (const MsmTask*)s_task_.d, done);
+    int32_t brc = before((const uint32_t*)s_idx_.d(), (cdl::Fr*)s_sc_.d(), (const MsmTask*)s_task_.d(), done);
     if (brc) return brc;
     if (done) {
       std::fill(st.out48.begin(), st.out48.end(), 0);
@@ -382,44 +356,37 @@ int32_t Engine::run_msm(MsmStage& st, const MsmBefore& before, const G1Affine* p
     cdl::msm_build_subs(st.tasks.data(), nt, cdl::msm_tp_pick_chunk(nterm, ctx_->sm_count), subs, tasks2);
     if ((rc = reserve(s_sub_, subs.size() * sizeof(cdl::MsmSub))) || (rc = reserve(s_t2_, tasks2.size() * sizeof(cdl::MsmTask2))))
       return rc;
-    size_t wb = cdl::msm_tp_scratch_bytes(nterm, subs.size(), nt);
-    if (wb > win_cap_) {
-      cudaStreamSynchronize(ctx_->stream);
-      if (d_win_) cudaFree(d_win_);
-      d_win_ = nullptr;
-      win_cap_ = 0;
-      if (cudaMalloc(&d_win_, wb + wb / 4) != cudaSuccess) return ctx_->fail(CDL_ERR_CUDA, "MSM scratch allocation failed");
-      win_cap_ = wb + wb / 4;
-    }
+    if (!d_win_.grow(cdl::msm_tp_scratch_bytes(nterm, subs.size(), nt), ctx_->stream))
+      return ctx_->fail(CDL_ERR_CUDA, "MSM scratch allocation failed");
     std::vector<uint32_t> fsubs;  // the chunks of those tasks
     for (uint32_t j : fixed_tasks)
       for (uint32_t c = 0; c < tasks2[j].sub_cnt; c++) fsubs.push_back(tasks2[j].sub_off + c);
     if (!fsubs.empty()) {
       if ((rc = reserve(s_fsub_, fsubs.size() * 4))) return rc;
-      memcpy(s_fsub_.h, fsubs.data(), fsubs.size() * 4);
-      CDL_CUDA(ctx_, cudaMemcpyAsync(s_fsub_.d, s_fsub_.h, fsubs.size() * 4, cudaMemcpyHostToDevice, ctx_->stream));
+      memcpy(s_fsub_.h(), fsubs.data(), fsubs.size() * 4);
+      CDL_CUDA(ctx_, cudaMemcpyAsync(s_fsub_.d(), s_fsub_.h(), fsubs.size() * 4, cudaMemcpyHostToDevice, ctx_->stream));
     }
-    memcpy(s_sub_.h, subs.data(), subs.size() * sizeof(cdl::MsmSub));
-    memcpy(s_t2_.h, tasks2.data(), tasks2.size() * sizeof(cdl::MsmTask2));
-    CDL_CUDA(ctx_, cudaMemcpyAsync(s_sub_.d, s_sub_.h, subs.size() * sizeof(cdl::MsmSub), cudaMemcpyHostToDevice, ctx_->stream));
-    CDL_CUDA(ctx_, cudaMemcpyAsync(s_t2_.d, s_t2_.h, tasks2.size() * sizeof(cdl::MsmTask2), cudaMemcpyHostToDevice, ctx_->stream));
+    memcpy(s_sub_.h(), subs.data(), subs.size() * sizeof(cdl::MsmSub));
+    memcpy(s_t2_.h(), tasks2.data(), tasks2.size() * sizeof(cdl::MsmTask2));
+    CDL_CUDA(ctx_, cudaMemcpyAsync(s_sub_.d(), s_sub_.h(), subs.size() * sizeof(cdl::MsmSub), cudaMemcpyHostToDevice, ctx_->stream));
+    CDL_CUDA(ctx_, cudaMemcpyAsync(s_t2_.d(), s_t2_.h(), tasks2.size() * sizeof(cdl::MsmTask2), cudaMemcpyHostToDevice, ctx_->stream));
     tick();
-    cdl::launch_msm_tp(points, (const uint32_t*)s_idx_.d, (const cdl::Fr*)s_sc_.d, (int)nterm, (const cdl::MsmSub*)s_sub_.d,
-                       (int)subs.size(), (const cdl::MsmTask2*)s_t2_.d, (int)nt, d_pool_, (uint8_t*)s_out_.d, d_win_,
-                       ctx_->stream, fixed_, fsubs.empty() ? nullptr : (const uint32_t*)s_fsub_.d, (int)fsubs.size());
+    cdl::launch_msm_tp(points, (const uint32_t*)s_idx_.d(), (const cdl::Fr*)s_sc_.d(), (int)nterm, (const cdl::MsmSub*)s_sub_.d(),
+                       (int)subs.size(), (const cdl::MsmTask2*)s_t2_.d(), (int)nt, d_pool(), (uint8_t*)s_out_.d(), d_win_.d(),
+                       ctx_->stream, fixed_, fsubs.empty() ? nullptr : (const uint32_t*)s_fsub_.d(), (int)fsubs.size());
     tock(0, alg, 128.0 * nterm);
     launches += fsubs.empty() ? 3 : 4;  // recode, bucket warps, chunk sums (+ fixed-base warps); tock counted the combine
   } else {
     tick();
-    cdl::launch_msm_small(points, (const uint32_t*)s_idx_.d, (const cdl::Fr*)s_sc_.d, (const MsmTask*)s_task_.d, (int)nt,
-                          max_terms, d_pool_, (uint8_t*)s_out_.d, ctx_->stream);
+    cdl::launch_msm_small(points, (const uint32_t*)s_idx_.d(), (const cdl::Fr*)s_sc_.d(), (const MsmTask*)s_task_.d(), (int)nt,
+                          max_terms, d_pool(), (uint8_t*)s_out_.d(), ctx_->stream);
     tock(0, alg, 128.0 * nterm);
   }
   CDL_CUDA(ctx_, cudaGetLastError());
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_out_.h, s_out_.d, nt * 48, cudaMemcpyDeviceToHost, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_out_.h(), s_out_.d(), nt * 48, cudaMemcpyDeviceToHost, ctx_->stream));
   CDL_CUDA(ctx_, ctx_->sync_stream());
   finish_timing();
-  memcpy(st.out48.data(), s_out_.h, nt * 48);
+  memcpy(st.out48.data(), s_out_.h(), nt * 48);
   return CDL_OK;
 }
 
@@ -429,12 +396,12 @@ int32_t Engine::run_elem(const std::vector<ElemOp>& ops, const std::vector<Fr>& 
   if (!n) return CDL_OK;
   int32_t rc;
   if ((rc = reserve(s_ops_, n * sizeof(ElemOp))) || (rc = reserve(s_sc_, sc.size() * 32))) return rc;
-  memcpy(s_ops_.h, ops.data(), n * sizeof(ElemOp));
-  memcpy(s_sc_.h, sc.data(), sc.size() * 32);
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_ops_.d, s_ops_.h, n * sizeof(ElemOp), cudaMemcpyHostToDevice, ctx_->stream));
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_sc_.d, s_sc_.h, sc.size() * 32, cudaMemcpyHostToDevice, ctx_->stream));
+  memcpy(s_ops_.h(), ops.data(), n * sizeof(ElemOp));
+  memcpy(s_sc_.h(), sc.data(), sc.size() * 32);
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_ops_.d(), s_ops_.h(), n * sizeof(ElemOp), cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_sc_.d(), s_sc_.h(), sc.size() * 32, cudaMemcpyHostToDevice, ctx_->stream));
   tick();
-  cdl::launch_elem_ops(d_pool_, (const ElemOp*)s_ops_.d, (const cdl::Fr*)s_sc_.d, (int)n, ctx_->stream, fixed_);
+  cdl::launch_elem_ops(d_pool(), (const ElemOp*)s_ops_.d(), (const cdl::Fr*)s_sc_.d(), (int)n, ctx_->stream, fixed_);
   tock(1, 3193.0 * n, 288.0 * n);  // §8d: 3193 modmul per scalar multiplication; src + add + dst points
   CDL_CUDA(ctx_, cudaGetLastError());
   CDL_CUDA(ctx_, ctx_->sync_stream());

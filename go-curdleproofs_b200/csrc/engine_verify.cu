@@ -95,7 +95,7 @@ int32_t Engine::batch_check(const MsmStage& st, const std::vector<Fr>& rho, uint
                h_flag = h_pos + al256((size_t)npos * 4);
   int32_t rc;
   if ((rc = reserve(s_bv_, h_flag + 4))) return rc;
-  uint8_t* hb = (uint8_t*)s_bv_.h;
+  uint8_t* hb = (uint8_t*)s_bv_.h();
   memcpy(hb, rho.data(), (size_t)nt * 32);
   memcpy(hb + h_off, off.data(), off.size() * 4);
   uint32_t* pos = (uint32_t*)(hb + h_pos);
@@ -104,30 +104,20 @@ int32_t Engine::batch_check(const MsmStage& st, const std::vector<Fr>& rho, uint
   // device: combined indices | scalars | result | flag | large-MSM scratch (grow-only)
   const size_t d_csc = al256(nc * 4), d_res = d_csc + al256(nc * 32), d_flag = d_res + al256(sizeof(cdl::G1Jac)),
                d_scr = d_flag + 256, need = d_scr + cdl::big_msm_scratch_bytes(d);
-  if (need > bv_cap_) {
-    cudaStreamSynchronize(ctx_->stream);
-    if (d_bv_) cudaFree(d_bv_);
-    d_bv_ = nullptr;
-    bv_cap_ = 0;
-    if (cudaMalloc(&d_bv_, need + need / 4) != cudaSuccess) {  // the per-proof launch needs no more memory
-      cudaGetLastError();
-      return CDL_OK;
-    }
-    bv_cap_ = need + need / 4;
-  }
-  uint8_t* db = (uint8_t*)d_bv_;
-  const uint8_t* sb = (const uint8_t*)s_bv_.d;
+  if (!d_bv_.grow(need, ctx_->stream)) return CDL_OK;  // the per-proof launch needs no more memory
+  uint8_t* db = (uint8_t*)d_bv_.d();
+  const uint8_t* sb = (const uint8_t*)s_bv_.d();
   uint32_t* cidx = (uint32_t*)db;
   cdl::Fr* csc = (cdl::Fr*)(db + d_csc);
   cdl::G1Jac* res = (cdl::G1Jac*)(db + d_res);
   uint32_t* flag = (uint32_t*)(db + d_flag);
-  CDL_CUDA(ctx_, cudaMemcpyAsync(s_bv_.d, s_bv_.h, h_flag, cudaMemcpyHostToDevice, ctx_->stream));
+  CDL_CUDA(ctx_, cudaMemcpyAsync(s_bv_.d(), s_bv_.h(), h_flag, cudaMemcpyHostToDevice, ctx_->stream));
   tick();
   cdl::launch_bv_assemble(d_idx, d_sc, d_tasks, nt, (const cdl::Fr*)sb, nterm, (const uint32_t*)(sb + h_off),
                           (const uint32_t*)(sb + h_pos), crs_size, cidx, csc, ctx_->stream);
   // the other lanes' bucket warps rely on the persisting-L2 window: leave it in place
   int nk = 0;
-  cudaError_t e = cdl::launch_big_msm(d_pool_, csc, d, 0, db + d_scr, ctx_->sm_count, res, ctx_->stream, cidx,
+  cudaError_t e = cdl::launch_big_msm(d_pool(), csc, d, 0, db + d_scr, ctx_->sm_count, res, ctx_->stream, cidx,
                                       /*release_l2=*/false, &nk);
   cdl::launch_bv_is_inf(res, flag, ctx_->stream);
   tock(0, msm_algorithmic_modmul(nc), 128.0 * nc);
@@ -524,13 +514,13 @@ int32_t Engine::verify(const Layout& L, uint32_t B, const cdl_crs* crs, std::vec
     // per-proof parameter blocks and the vector challenges `as` go up once; the kernel runs on the stream
     // between the stage's uploads and its MSM kernels
     if ((rc = reserve(s_vs_, np * sizeof(cdl::VsParams))) || (rc = reserve(s_as_, (size_t)B * ell * 32))) return rc;
-    memcpy(s_vs_.h, vs_launch.data(), np * sizeof(cdl::VsParams));
-    Fr* as_h = (Fr*)s_as_.h;
+    memcpy(s_vs_.h(), vs_launch.data(), np * sizeof(cdl::VsParams));
+    Fr* as_h = (Fr*)s_as_.h();
     par(B, [&](size_t b) {
       if (have_big[b]) memcpy(as_h + b * ell, S[b]->as.data(), (size_t)ell * 32);
     });
-    CDL_CUDA(ctx_, cudaMemcpyAsync(s_vs_.d, s_vs_.h, np * sizeof(cdl::VsParams), cudaMemcpyHostToDevice, ctx_->stream));
-    CDL_CUDA(ctx_, cudaMemcpyAsync(s_as_.d, s_as_.h, (size_t)B * ell * 32, cudaMemcpyHostToDevice, ctx_->stream));
+    CDL_CUDA(ctx_, cudaMemcpyAsync(s_vs_.d(), s_vs_.h(), np * sizeof(cdl::VsParams), cudaMemcpyHostToDevice, ctx_->stream));
+    CDL_CUDA(ctx_, cudaMemcpyAsync(s_as_.d(), s_as_.h(), (size_t)B * ell * 32, cudaMemcpyHostToDevice, ctx_->stream));
   }
   // Combined check: one weight per task, 128 bits from SHAKE256 over every included proof's digest (never
   // from the caller's Rand, whose position the caller observes); deterministic, so runs are reproducible.
@@ -555,7 +545,7 @@ int32_t Engine::verify(const Layout& L, uint32_t B, const cdl_crs* crs, std::vec
   bool all_pass = false;  // the combined sum is infinity: every task of the stage is
   rc = run_msm(st, [&](const uint32_t* d_idx, cdl::Fr* d_sc, const MsmTask* d_tasks, bool& done) -> int32_t {
     if (np) {
-      cdl::launch_verify_scalars((const cdl::VsParams*)s_vs_.d, (const cdl::Fr*)s_as_.d, d_sc, (uint32_t)np, ell, n, L.m,
+      cdl::launch_verify_scalars((const cdl::VsParams*)s_vs_.d(), (const cdl::Fr*)s_as_.d(), d_sc, (uint32_t)np, ell, n, L.m,
                                  ctx_->stream);
       launches++;
     }

@@ -177,7 +177,7 @@ class Engine {
   int32_t base_mul(const cdl_g1_affine& base, const Fr* sc, size_t n, cdl_g1_affine* out, uint8_t* out48);
 
   cdl_ctx* ctx() { return ctx_; }
-  cdl::G1Affine* d_pool() { return d_pool_; }
+  cdl::G1Affine* d_pool() { return (cdl::G1Affine*)pool_mem_.d(); }
   ThreadPool& threads() { return pool_; }
   // instrumentation for bench.py: per kernel class (0 msm, 1 elementwise, 2 decompress,
   // 3 compress / normalise): launches, CUDA-event time on the launching stream,
@@ -222,13 +222,10 @@ class Engine {
  private:
   cdl_ctx* ctx_;
   ThreadPool pool_;
-  cdl::G1Affine* d_pool_ = nullptr;
+  DeviceScratch pool_mem_;  // the point pool (d_pool())
   cdl::FixedTable fixed_;  // tables of the current call's CRS, or empty
-  size_t pool_cap_ = 0;
-  void* d_win_ = nullptr;  // window sums of the two-kernel MSM path
-  size_t win_cap_ = 0;
-  void* d_match_ = nullptr;  // tables and window bases of one tile of trackers (match_scratch)
-  size_t match_cap_ = 0;
+  DeviceScratch d_win_;  // window sums of the two-kernel MSM path
+  DeviceScratch d_match_;  // tables and window bases of one tile of trackers (match_scratch)
   bool match_scratch(uint32_t tile);
   // Width-12 fixed-base tables of callers' bases (base_mul), keyed by the 96 base bytes: at most kBaseTables,
   // the least recently used replaced.  Separate allocations, so the pool and the match scratch stay as they are.
@@ -240,21 +237,16 @@ class Engine {
   static constexpr size_t kBaseTables = 4;
   std::vector<BaseTable> base_tabs_;
   uint64_t base_clock_ = 0;
-  void* d_bv_ = nullptr;  // combined verifier check: term list, large-MSM scratch, result (batch_check)
-  size_t bv_cap_ = 0;
+  DeviceScratch d_bv_;  // combined verifier check: term list, large-MSM scratch, result (batch_check)
   // The verifier's second MSM stage `st`, uploaded (d_idx, d_sc, d_tasks), as one large MSM with the weight
   // rho[t] (Montgomery) on task t and the CRS bases (pool indices < crs_size) merged: *all_inf = whether it
   // is the point at infinity.
   int32_t batch_check(const MsmStage& st, const std::vector<Fr>& rho, uint32_t crs_size, const uint32_t* d_idx,
                       const cdl::Fr* d_sc, const cdl::MsmTask* d_tasks, bool* all_inf);
-  // pinned host staging + device scratch, grow-only
-  struct Staging {
-    void* h = nullptr;
-    void* d = nullptr;
-    size_t cap = 0;
-  };
+  // pinned host staging + device scratch
   Staging s_idx_, s_sc_, s_task_, s_out_, s_ops_, s_enc_, s_st_, s_jac_, s_sub_, s_t2_, s_cr_, s_fsub_, s_vs_, s_as_, s_bv_,
       s_in_, s_base_;
+  // s.grow on the engine's stream, with the error recorded when it fails
   int32_t reserve(Staging& s, size_t bytes);
   void tick();                                   // event before a kernel
   void tock(int cls, double modmul, double bytes);  // event after; call finish_timing() after the sync
