@@ -32,7 +32,7 @@ static bool msm_tasks(const uint32_t* offsets, size_t k, std::vector<MsmTask>& t
 
 extern "C" {
 
-uint32_t cdl_abi_version(void) { return (1u << 16) | 9u; }
+uint32_t cdl_abi_version(void) { return (1u << 16) | 10u; }
 
 void cdl_destroy(cdl_ctx* c);
 
@@ -104,7 +104,6 @@ cdl_ctx* cdl_lane_(cdl_ctx* root, size_t slot, size_t i) {
     l->name = root->name;
     l->parent = root;
     l->n_lanes = 1;
-    l->msm_c_override = root->msm_c_override;
     cudaDeviceGetAttribute(&l->sm_count, cudaDevAttrMultiProcessorCount, l->device);
     if (cudaSetDevice(l->device) != cudaSuccess ||
         cudaStreamCreateWithFlags(&l->stream, cudaStreamNonBlocking) != cudaSuccess) {
@@ -126,7 +125,7 @@ int32_t cdl_set_lanes(cdl_ctx* c, int32_t lanes) {
 }
 
 void cdl_engine_free_(void* engine);  // capi_protocol.cu
-int32_t cdl_big_msm_host_(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out);  // capi_msm.cu
+int32_t cdl_big_msm_host_(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out);  // capi_msm.cu, takes the mutex
 
 void cdl_destroy(cdl_ctx* c) {
   if (!c) return;
@@ -222,11 +221,9 @@ int32_t cdl_g1_msm_batch_device(cdl_ctx* c, cdl_g1_affine* d_pool, const uint32_
 
 int32_t cdl_g1_msm(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out) {
   if (!c || !out || (n && (!points || !scalars))) return CDL_ERR_INVALID_ARG;
-  if (n > kBigMsmThreshold) {  // Pippenger path (k_msm_big.cu); the small-MSM kernels serve Prove/Verify sizes
-    std::lock_guard<std::mutex> lk(c->mu);
-    CDL_CUDA(c, cudaSetDevice(c->device));
-    return cdl_big_msm_host_(c, points, scalars, n, out);
-  }
+  // Pippenger path (k_msm_big.cu), split over the device slots when large enough; the small-MSM kernels
+  // serve Prove/Verify sizes
+  if (n > kBigMsmThreshold) return cdl_big_msm_host_(c, points, scalars, n, out);
   uint32_t offs[2] = {0, (uint32_t)n};
   cdl_g1_affine a;
   int32_t rc = cdl_g1_msm_batch(c, points, scalars, offs, 1, &a);

@@ -16,11 +16,17 @@ namespace {
 // take less time than building the table and running the table path (cold table path).  The crossover measured
 // on a B200 by tools/base_mul.py (profiles/r8_base_mul.txt).
 constexpr size_t kBaseTableMinScalars = 32768;
+// Scalars per device slot from which a call is split over the slots of a multi-device context:
+// max(1, min(D, n / kBaseSlotScalars)) slots, each running its block on its lane 0's engine.  Equal to
+// kBaseTableMinScalars, so that a fresh base takes the table path on every slot exactly when the one-device
+// call would.  Derived, not tuned: the split's cost and gain have not been measured.
+constexpr size_t kBaseSlotScalars = 32768;
 // Scalars per round trip through the pinned staging: 32 MB of scalars and up to 144 MB of results
 constexpr size_t kBaseMulChunk = (size_t)1 << 20;
 
 static_assert(CDL_BASE_MUL_MAX == (1u << 24), "documented limit of cdl_g1_batch_scalar_mul_base");
 static_assert(kBaseTableMinScalars <= kBaseMulChunk, "the GLV path runs in one chunk");
+static_assert(kBaseSlotScalars >= kBaseTableMinScalars, "a split call's blocks take the table path as the whole call would");
 
 const uint8_t kInfEnc[48] = {0xc0};  // compressed point at infinity
 
@@ -150,6 +156,12 @@ int32_t cdl_g1_batch_scalar_mul_base(cdl_ctx* c, const cdl_g1_affine* base, cons
       for (size_t i = 0; i < n; i++) memcpy(out48 + 48 * i, kInfEnc, 48);
     return CDL_OK;
   }
+  // every slot in use multiplies its own block of scalars with its own engine's tables (disjoint outputs)
+  if (cdlh::slots_for(c, n, kBaseSlotScalars) > 1)
+    return cdlh::run_split(c, n, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_g1_batch_scalar_mul_base(lane, base, scalars + lo, hi - lo, out ? out + lo : nullptr,
+                                          out48 ? out48 + 48 * lo : nullptr);
+    }, false, 1, kBaseSlotScalars);
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   return engine_of(c)->base_mul(*base, reinterpret_cast<const Fr*>(scalars), n, out, out48);

@@ -20,9 +20,11 @@ typedef enum { ncclChar = 0 } ncclDataType_t;
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <vector>
 
 #include "../../include/curdle_b200.h"
 #include "context.cuh"
+#include "host/engine.hpp"
 #include "launch.h"
 
 using namespace cdl;
@@ -72,8 +74,17 @@ NcclApi* nccl_api() {
   return &api;
 }
 
+// Terms per device slot from which cdl_g1_msm of host vectors is split by points over the slots of a
+// multi-device context: max(1, min(D, n / kMsmSlotTerms)) slots.  Derived from the one-GPU sweep
+// (profiles/r3_msm_sweep_1gpu.txt: 1.84 ms at 2^16 terms, 2.24 ms at 2^17), so that each block of a split call
+// is still an MSM the Pippenger path runs near its best per-term rate.  Derived, not tuned: the split's own
+// cost (the partials' round trip and k_big_combine) and its gain have not been measured.
+constexpr size_t kMsmSlotTerms = 65536;
+
+// the window width and batch-affine rounds of the root context (a lane's MSM follows its root's settings)
 int pick_c(cdl_ctx* c, size_t n) {
-  if (c->msm_c_override >= 2 && c->msm_c_override <= 18) return c->msm_c_override;
+  const int o = c->root()->msm_c_override;
+  if (o >= 2 && o <= 18) return o;
   return big_msm_pick_c(n);
 }
 
@@ -81,7 +92,7 @@ int pick_c(cdl_ctx* c, size_t n) {
 int32_t big_msm_on_device(cdl_ctx* c, const G1Affine* d_pts, const Fr* d_sc, size_t n, uint32_t part, uint32_t parts,
                           int normalize, G1Jac* d_out) {
   if (n >= ((size_t)1 << 30)) return c->fail(CDL_ERR_TOO_LARGE, "msm: %zu terms exceed 2^30 - 1", n);
-  BigMsmDims d = big_msm_dims(n, pick_c(c, n), (int)part, (int)parts, c->msm_ba_override);
+  BigMsmDims d = big_msm_dims(n, pick_c(c, n), (int)part, (int)parts, c->root()->msm_ba_override);
   // the batch-affine rounds keep two generations of pair sums and the prefix products (~ 100 B per
   // sorted entry): beyond this budget the XYZZ-only path (36 B per entry less) runs instead
   constexpr size_t kBaScratchBudget = (size_t)48 << 30;
@@ -114,10 +125,47 @@ int32_t msm_of_host_vectors(cdl_ctx* c, const cdl_g1_affine* points, const cdl_f
   return CDL_OK;
 }
 
+// The MSM of host vectors on a root context of several slots, split by points: slot s of the D slots in use
+// sums its block shard_bounds(n, D, s) on lane (s, 0) (own input buffers, scratch and stream, nothing
+// normalised), and the D partial sums (144 bytes each, through the host) are added and normalised by
+// k_big_combine on the root stream.  The root's mutex is held across the pieces and the combine.
+int32_t big_msm_split(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, size_t D,
+                      cdl_g1_jac* out) {
+  std::lock_guard<std::mutex> lk(c->mu);
+  // the whole call's limit, before any input is read (the per-device limits apply to every block)
+  if (n >= ((size_t)1 << 30)) return c->fail(CDL_ERR_TOO_LARGE, "msm: %zu terms exceed 2^30 - 1", n);
+  std::vector<cdl_g1_jac> part(D);
+  int32_t rc = cdlh::run_split_locked(c, n, [&](cdl_ctx* l, size_t lo, size_t hi) -> int32_t {
+    // l's buffers and stream without l's own mutex: every use of a lane happens under its root's mutex, held here
+    CDL_CUDA(l, cudaSetDevice(l->device));
+    return msm_of_host_vectors(l, points + lo, scalars + lo, hi - lo, &part[l->dev_slot],
+                               [&](const G1Affine* d_pts, const Fr* d_sc, G1Jac* d_out) {
+                                 return big_msm_on_device(l, d_pts, d_sc, hi - lo, 0, 1, 0, d_out);
+                               });
+  }, false, 1, kMsmSlotTerms);
+  if (rc) return rc;
+  CDL_CUDA(c, cudaSetDevice(c->device));
+  if (!c->partials.grow(D * sizeof(G1Jac), c->stream) || !c->out.grow(sizeof(G1Jac), c->stream))
+    return c->fail(CDL_ERR_CUDA, "device allocation failed");
+  cdl_g1_jac sum;
+  CDL_CUDA(c, cudaMemcpyAsync(c->partials.d(), part.data(), D * sizeof(G1Jac), cudaMemcpyHostToDevice, c->stream));
+  launch_big_combine((const G1Jac*)c->partials.d(), (int)D, (G1Jac*)c->out.d(), c->stream);
+  CDL_CUDA(c, cudaGetLastError());
+  CDL_CUDA(c, cudaMemcpyAsync(&sum, c->out.d(), sizeof(G1Jac), cudaMemcpyDeviceToHost, c->stream));
+  CDL_CUDA(c, cudaStreamSynchronize(c->stream));
+  *out = sum;
+  return CDL_OK;
+}
+
 }  // namespace
 
-// used by cdl_g1_msm (capi.cu) above kBigMsmThreshold terms; caller holds the context mutex
+// cdl_g1_msm (capi.cu) above kBigMsmThreshold terms: split over the device slots from 2 * kMsmSlotTerms terms,
+// else on the context's own device and buffers
 extern "C" int32_t cdl_big_msm_host_(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out) {
+  const size_t D = cdlh::slots_for(c, n, kMsmSlotTerms);
+  if (D > 1) return big_msm_split(c, points, scalars, n, D, out);
+  std::lock_guard<std::mutex> lk(c->mu);
+  CDL_CUDA(c, cudaSetDevice(c->device));
   return msm_of_host_vectors(c, points, scalars, n, out, [&](const G1Affine* d_pts, const Fr* d_sc, G1Jac* d_out) {
     return big_msm_on_device(c, d_pts, d_sc, n, 0, 1, 1, d_out);
   });

@@ -14,6 +14,7 @@ using cdlh::affine_to_jac;
 using cdlh::Engine;
 using cdlh::engine_of;
 using cdlh::Fr;
+using cdlh::kMinLaneBatch;
 using cdlh::Layout;
 using cdlh::run_split;
 using cdlh::slots_for;
@@ -133,8 +134,6 @@ int32_t begin_call(cdl_ctx* c, const cdl_crs* crs, size_t B, Engine** E, Layout*
   return (*E)->load_crs(*L, crs);
 }
 
-constexpr size_t kMinLaneBatch = 32;  // below this a sub-batch no longer fills its launches
-
 // number of lanes a slot's block of n instances is cut into
 size_t lanes_for(cdl_ctx* c, size_t n) {
   if (c->n_lanes <= 1) return 1;
@@ -143,20 +142,25 @@ size_t lanes_for(cdl_ctx* c, size_t n) {
 
 }  // namespace
 
-size_t cdlh::slots_for(cdl_ctx* c, size_t B) {
+size_t cdlh::slots_for(cdl_ctx* c, size_t B, size_t min_block) {
   if (c->parent) return 1;
-  return std::max<size_t>(1, std::min<size_t>(c->slots.size(), B / kMinLaneBatch));
+  return std::max<size_t>(1, std::min<size_t>(c->slots.size(), B / min_block));
 }
 
 // first unit of block s when B units are dealt to D slots in contiguous blocks (sharding.shard_bounds)
 static size_t shard_lo(size_t B, size_t D, size_t s) { return s * (B / D) + std::min(s, B % D); }
 
 int32_t cdlh::run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes,
-                        size_t align) {
+                        size_t align, size_t min_block) {
   std::lock_guard<std::mutex> lk(c->mu);
+  return run_split_locked(c, B, fn, lanes, align, min_block);
+}
+
+int32_t cdlh::run_split_locked(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn,
+                               bool lanes, size_t align, size_t min_block) {
   struct Piece { cdl_ctx* ctx; size_t lo, hi; };
   std::vector<Piece> pieces;
-  const size_t D = slots_for(c, B);
+  const size_t D = slots_for(c, B, min_block);
   auto bound = [&](size_t s) {
     if (s == D) return B;
     return std::min(B, (shard_lo(B, D, s) + align / 2) / align * align);

@@ -269,14 +269,19 @@ std::string parse_wire_proof(const uint8_t* buf, size_t len, bool with_m, WirePr
 Engine* engine_of(cdl_ctx* c);
 // gnark's G1Jac of an affine point: (x, y, 1), or (1, 1, 0) for infinity
 void affine_to_jac(cdl_g1_jac* out, const cdl_g1_affine& a);
-// Device slots a batched call of B units on c uses: max(1, min(slots, B / 32)); 1 on a lane context.
-size_t slots_for(cdl_ctx* c, size_t B);
+constexpr size_t kMinLaneBatch = 32;  // below this a sub-batch no longer fills its launches
+// Device slots a call of B units on c uses: max(1, min(slots, B / min_block)), with min_block = 32 for the
+// batched protocol calls and matching; 1 on a lane context.
+size_t slots_for(cdl_ctx* c, size_t B, size_t min_block = kMinLaneBatch);
 // Runs fn(lane ctx, lo, hi) for contiguous pieces [lo, hi) of a call of B units on a root context concurrently,
-// one host thread per piece (DESIGN §4): slot s of the D = slots_for(c, B) slots in use takes the block that
-// sharding.shard_bounds(B, D, s) gives, its bounds rounded to multiples of `align` (empty blocks are skipped);
-// with `lanes` it cuts its block into up to n_lanes lanes of at least 32 units, else the block is one piece
-// on the slot's lane 0.
+// one host thread per piece (DESIGN §4): slot s of the D = slots_for(c, B, min_block) slots in use takes the
+// block that sharding.shard_bounds(B, D, s) gives, its bounds rounded to multiples of `align` (empty blocks are
+// skipped); with `lanes` it cuts its block into up to n_lanes lanes of at least 32 units, else the block is one
+// piece on the slot's lane 0.  Holds c's mutex while the pieces run.
 int32_t run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes = true,
-                  size_t align = 1);
+                  size_t align = 1, size_t min_block = kMinLaneBatch);
+// run_split for a caller that already holds c's mutex (and keeps it for work after the pieces)
+int32_t run_split_locked(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn,
+                         bool lanes, size_t align, size_t min_block);
 
 }  // namespace cdlh

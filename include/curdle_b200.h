@@ -67,8 +67,16 @@ int32_t cdl_create(int device, cdl_ctx** out);
  * as a one-device context cuts a batch.  A call of fewer than 64 instances, and every single
  * (non-batched) protocol call, runs on slot 0.
  *
- * Everything else runs on slot 0's device (devices[0]): the cdl_g1_* primitives, the large and device
- * MSMs, cdl_dev_* buffers (device memory of devices[0]), cdl_rand_get_g1_affines and CRS generation.
+ * Two single calls split by size, each slot running its block on its lane 0 (one piece per slot):
+ * cdl_g1_msm of more than 1 024 terms (and cdl_g1_sum_affine through it) over D' = max(1, min(n, terms /
+ * 65 536)) slots, so from 131 072 terms on; slot s sums its contiguous block of the terms and the D' partial
+ * sums are added on devices[0].  cdl_g1_batch_scalar_mul_base over D' = max(1, min(n, scalars / 32 768))
+ * slots, so from 65 536 scalars on; slot s multiplies its contiguous block with its own cached tables.  Below
+ * these sizes both run on slot 0 exactly as on a one-device context.
+ *
+ * Everything else runs on slot 0's device (devices[0]): the other cdl_g1_* primitives, cdl_g1_msm_batch,
+ * the device and sharded MSMs, cdl_dev_* buffers (device memory of devices[0]), cdl_rand_get_g1_affines and
+ * CRS generation.
  * cdl_comm_init refuses a context of more than one slot: the NCCL-sharded MSM runs one process (and
  * one single-device context) per GPU.
  * CDL_ERR_INVALID_ARG for n == 0, n > 16 or a device id out of range; CDL_ERR_NO_DEVICE without a
@@ -91,7 +99,13 @@ int32_t cdl_device_info(cdl_ctx* ctx, int32_t* sm_count, int32_t* clock_khz, cha
  * samemultiscalarargument.go:63-72,93-111; common/util.go:75,82.
  * Infinity bases are skipped; n == 0 gives infinity.  The result is returned
  * normalised (Z = 1, or Z = 0 for infinity) — any representative is valid
- * because only canonical encodings are observable (SURVEY.md §8c). */
+ * because only canonical encodings are observable (SURVEY.md §8c).
+ * CDL_ERR_TOO_LARGE for n >= 2^30 (on a context of several device slots before any input is read).  Above
+ * 1 024 terms the per-device limits - the batch-affine scratch budget (the MSM falls back to extended-Jacobian
+ * buckets beyond it), 2^32 sorted bucket entries (CDL_ERR_TOO_LARGE) and device allocation (CDL_ERR_CUDA) -
+ * apply to the whole MSM on a one-device context and to each slot's block on a split call
+ * (cdl_create_devices), so a split call fails nowhere a one-device call succeeds and may succeed where one
+ * device alone reaches a limit.  The 144 output bytes are the same either way. */
 int32_t cdl_g1_msm(cdl_ctx* ctx, const cdl_g1_affine* points, const cdl_fr* scalars, size_t n, cdl_g1_jac* out);
 
 /* k independent MSMs in one launch; MSM j covers points/scalars
@@ -128,8 +142,13 @@ int32_t cdl_g1_fold(cdl_ctx* ctx, cdl_g1_affine* L, const cdl_g1_affine* R, cons
  * the base's width-12 fixed-base table (22 x 2 048 points, 4.3 MB; 22 mixed additions per scalar), used
  * when that table is cached or n is large enough that building it pays off (the table is then built and
  * cached); otherwise GLV scalar multiplication of every scalar, which builds no table.  The context keeps
- * the tables of its 4 most recently used bases (about 17 MB of device memory, freed by cdl_destroy); a base
- * whose table is cached is not checked again.  Scalars travel in chunks of 2^20.
+ * the tables of its 4 most recently used bases per device slot (about 17 MB of device memory per slot,
+ * freed by cdl_destroy); a base whose table is cached is not checked again.  Scalars travel in chunks of 2^20.
+ * On a context of several slots a call of 65 536 scalars or more is split (cdl_create_devices): every slot
+ * in use runs its block with its own cache, checks the base when its table is not cached and picks its path
+ * by its block size and its cache alone; a smaller call runs on the context's own cache.  Device 0 can
+ * therefore hold both caches (up to 8 tables).  A rejected base fails every block alike, before any output
+ * is written.
  * n == 0 does nothing; CDL_ERR_INVALID_ARG for a null ctx, base or scalars or when both outputs are NULL;
  * CDL_ERR_TOO_LARGE when n exceeds CDL_BASE_MUL_MAX, before any input is read. */
 #define CDL_BASE_MUL_MAX (1u << 24)

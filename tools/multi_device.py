@@ -8,13 +8,20 @@ warm-up call per row:
                     ell = 124 (n = 128), B = 4 096 * D, end to end (host clock around the two calls);
   whisk_validate    the validation call alone;
   prove_batch       cdl_prove_batch at ell = 124, B = 1 024 * D caller-supplied instances;
-  match             cdl_whisk_match_trackers, 8 192 trackers x 16 384 keys.
+  match             cdl_whisk_match_trackers, 8 192 trackers x 16 384 keys;
+and, with --rows bulk (those rows alone) or --rows all (before the others), the two single calls that split by
+size; the base_mul rows at 2^24 hold a 512 MB scalar vector and up to 1.6 GB of results per call:
+  msm               cdl_g1_msm on host vectors at n = 2^16, 2^17, 2^18, 2^20 and 2^22 (a 2^20 set of points
+                    repeated, its scalars rotated per repetition), wall time only (large MSMs are not in the
+                    engine's accounting);
+  base_mul          cdl_g1_batch_scalar_mul_base with a warm table at n = 2^16, 2^20, 2^22 and 2^24, affine and
+                    compressed results.
 Every row gives the median of --reps timed calls and the busy time of every device slot
 (cdl_engine_busy_ms_device, union of that slot's kernel intervals) summed over the timed calls of the row.
-Rows marked [0, 0] run two slots on GPU 0 (the split without a second GPU).  Lanes per slot and host cores
-follow bench.py's per-rank defaults.  Then `bench.py --gpus D` (torchrun for D > 1, headline line only) runs
-in the same process tree as the multi-process comparison, and the card's name and power limit are read in
-the same call."""
+Rows marked [0, 0] run two slots on GPU 0: what the split costs on one GPU (one PCIe link, one device), not a
+speedup.  Lanes per slot and host cores follow bench.py's per-rank defaults.  With the protocol rows,
+`bench.py --gpus D` (torchrun for D > 1, headline line only) then runs in the same process tree as the
+multi-process comparison.  The card's name and power limit are read in the same call."""
 import argparse
 import importlib
 import json
@@ -23,6 +30,8 @@ import statistics
 import subprocess
 import sys
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -135,6 +144,58 @@ def measure(pkg, devices, reps, out):
     return rows
 
 
+MSM_SIZES = [1 << 16, 1 << 17, 1 << 18, 1 << 20, 1 << 22]
+BASE_SIZES = [1 << 16, 1 << 20, 1 << 22, 1 << 24]
+SET = 1 << 20
+
+
+def bulk_inputs(pkg):
+    """a 2^20 set of points a_i * G and canonical scalars, made once on GPU 0; a fixed-base base"""
+    ctx = pkg.Context(0)
+    rng = np.random.default_rng(9)
+    raw = rng.integers(0, 256, size=(SET, 32), dtype=np.uint8)
+    raw[:, 31] &= 0x3F  # below 2^254 < r: canonical Montgomery limbs
+    pts = ctx.g1_scalar_mul_affine(aff_enc(b.G1_GEN) * SET, raw.tobytes(), broadcast=False)
+    raw2 = rng.integers(0, 256, size=(SET, 32), dtype=np.uint8)
+    raw2[:, 31] &= 0x3F
+    base = aff_enc(b.g1_mul(b.G1_GEN, 0x1234567890ABCDEF))
+    ctx.close()
+    return pts, raw2.tobytes(), base
+
+
+def scalars(inputs, n):
+    """n scalars: the 2^20 set repeated, rotated by one term per repetition"""
+    sc = inputs[1]
+    return b"".join(sc[32 * r:] + sc[:32 * r] for r in range(-(-n // SET)))[:32 * n]
+
+
+def points(inputs, n):
+    """n points: the 2^20 set repeated"""
+    return (inputs[0] * -(-n // SET))[:96 * n]
+
+
+def measure_bulk(pkg, devices, reps, inputs, out):
+    D = len(devices)
+    ctx = pkg.Context(devices=devices)
+    ctx.set_lanes(6 if (os.cpu_count() or 1) // len(set(devices)) >= 8 else 8)
+    rows = []
+    for n in MSM_SIZES:
+        P, S = points(inputs, n), scalars(inputs, n)
+        t, _ = timed(ctx, D, reps, lambda i: ctx.g1_msm(P, S))
+        rows.append(f"  {str(devices):14s} msm               n={n:>10d}  {n / t / 1e6:10.2f} M terms/s  median "
+                    f"{t * 1e3:9.2f} ms")
+    base = inputs[2]
+    for n in BASE_SIZES:
+        S = scalars(inputs, n)
+        for kind, kw in (("affine", {}), ("compressed", {"affine": False, "compressed": True})):
+            t, busy = timed(ctx, D, reps, lambda i: ctx.g1_batch_scalar_mul_base(base, S, **kw))
+            rows.append(f"  {str(devices):14s} base_mul {kind:10s} n={n:>10d}  {n / t / 1e6:10.2f} M/s        median "
+                        f"{t * 1e3:9.2f} ms   busy per slot ms: {' / '.join(f'{x:.1f}' for x in busy)}")
+    ctx.close()
+    for line in rows:
+        print(line, file=out, flush=True)
+
+
 def bench(D, steps, warmup):
     args = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", str(D), "--steps", str(steps), "--warmup",
             str(warmup), "--no-cpu-baseline", "--no-msm", "--no-latency", "--no-config4", "--no-n512"]
@@ -154,6 +215,9 @@ def main():
     ap.add_argument("--bench-steps", type=int, default=3)
     ap.add_argument("--bench-warmup", type=int, default=2)
     ap.add_argument("--out", default="", help="also write the report to this file")
+    ap.add_argument("--rows", choices=["protocol", "bulk", "all"], default="protocol",
+                    help="protocol (default): the batched calls and the bench.py comparison; bulk: msm and base_mul; "
+                         "all: both")
     args = ap.parse_args()
     import torch
 
@@ -180,6 +244,16 @@ def main():
     out = Tee(args.out)
     print(f"# tools/multi_device.py  (host cores: {os.cpu_count()}, GPUs: {n})", file=out)
     print(f"# nvidia-smi index, name, power.limit, clocks.max.sm:\n# " + card().replace("\n", "\n# "), file=out)
+    lists = [list(range(D)) for D in range(1, Dmax + 1)] + [[0, 0]]
+    if args.rows != "protocol":
+        print(f"# in-process, bulk rows: median wall time of {args.reps} calls after one warm-up call; [0, 0] = two "
+              "slots on GPU 0 (the split's cost on one GPU, not a speedup)", file=out)
+        inputs = bulk_inputs(pkg)
+        for devs in lists:
+            measure_bulk(pkg, devs, args.reps, inputs, out)
+        del inputs
+    if args.rows == "bulk":
+        return
     print("# in-process: one context over the device list", file=out)
     inproc = {}
     for D in range(1, Dmax + 1):
