@@ -98,6 +98,7 @@ def load_library():
     lib.cdl_whisk_is_valid_shuffle_proof_batch.argtypes = [vp, vp, sz, vp, vp, vp, sz, C.POINTER(vp), i32p, i32p]
     lib.cdl_whisk_generate_tracker_proof_batch.argtypes = [vp, sz, vp, vp, C.POINTER(vp), vp, i32p]
     lib.cdl_whisk_is_valid_tracker_proof_batch.argtypes = [vp, sz, vp, vp, vp, i32p, i32p]
+    lib.cdl_whisk_generate_registration_batch.argtypes = [vp, sz, vp, C.POINTER(vp), vp, vp, vp, i32p]
     lib.cdl_whisk_match_trackers.argtypes = [vp, sz, vp, sz, vp, i32p, i32p]
     lib.cdl_host_selftest.argtypes = [vp, vp, vp, vp]
     lib.cdl_host_selftest_fibers.argtypes = [C.c_uint32, C.c_uint32, vp, C.POINTER(C.c_int32)]
@@ -632,6 +633,22 @@ def _ctx_whisk_is_valid_tracker_proof_batch(self, trackers: bytes, k_comms: byte
     return list(ok), list(status)
 
 
+def _ctx_whisk_generate_registration_batch(self, ks: bytes, rands):
+    """Whisk registration for B = len(rands) validators with secrets ks (B x 32 bytes, gnark fr.Element): r is
+    drawn from each Rand, then one blinder -> (B x 96 tracker bytes {rG, krG}, B x 48 k-commitment bytes kG,
+    B x 128 opening-proof bytes, status list).  A validator whose status is not 0 (r = 0 or 1) has zero bytes.
+    rands must be distinct Rand objects, one per validator: the validators draw concurrently."""
+    B = len(rands)
+    trackers = C.create_string_buffer(max(1, B) * 96)
+    k_comms = C.create_string_buffer(max(1, B) * 48)
+    proofs = C.create_string_buffer(max(1, B) * 128)
+    status = (C.c_int32 * max(1, B))()
+    rh = (C.c_void_p * max(1, B))(*[r.h for r in rands])
+    self._chk(self.lib.cdl_whisk_generate_registration_batch(self.h, B, _inbuf(ks), rh, trackers, k_comms, proofs,
+                                                             status))
+    return trackers.raw[:96 * B], k_comms.raw[:48 * B], proofs.raw[:128 * B], list(status)[:B]
+
+
 def _ctx_whisk_match_trackers(self, trackers: bytes, ks: bytes):
     """Which of the V secrets in ks (V x 32 bytes, gnark fr.Element) own which of the T trackers
     (T x 96 bytes) -> (owner list, status list); owner[t] is the smallest owning key index or -1."""
@@ -713,6 +730,7 @@ Context.whisk_generate_shuffle_proof_batch = _ctx_whisk_generate_batch
 Context.whisk_is_valid_shuffle_proof_batch = _ctx_whisk_is_valid_batch
 Context.whisk_generate_tracker_proof_batch = _ctx_whisk_generate_tracker_proof_batch
 Context.whisk_is_valid_tracker_proof_batch = _ctx_whisk_is_valid_tracker_proof_batch
+Context.whisk_generate_registration_batch = _ctx_whisk_generate_registration_batch
 Context.whisk_match_trackers = _ctx_whisk_match_trackers
 Context.launch_count = _ctx_launch_count
 Context.engine_busy_ms = _ctx_engine_busy_ms

@@ -32,7 +32,7 @@ static bool msm_tasks(const uint32_t* offsets, size_t k, std::vector<MsmTask>& t
 
 extern "C" {
 
-uint32_t cdl_abi_version(void) { return (1u << 16) | 10u; }
+uint32_t cdl_abi_version(void) { return (1u << 16) | 11u; }
 
 void cdl_destroy(cdl_ctx* c);
 

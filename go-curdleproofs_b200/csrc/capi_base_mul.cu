@@ -39,6 +39,8 @@ constexpr size_t kOffCopies = kOffWaff + cdl::kFbW * sizeof(cdl::G1Affine);
 
 }  // namespace
 
+size_t cdlh::base_mul_min_block(size_t per_unit) { return (kBaseSlotScalars + per_unit - 1) / per_unit; }
+
 int32_t Engine::base_mul(const cdl_g1_affine& base, const Fr* sc, size_t n, cdl_g1_affine* out, uint8_t* out48) {
   // the cached table of this base, if any
   BaseTable* hit = nullptr;

@@ -84,10 +84,15 @@ int32_t rand_points_to_pool(Engine* E, cdl_rand* r, uint32_t gen_slot, uint32_t 
   return E->run_elem(ops, sc);
 }
 
-int32_t put_generator(Engine* E, uint32_t slot) {
+cdl_g1_affine generator() {
   cdl_g1_affine g;
   memcpy(g.x.l, kGenX, 48);
   memcpy(g.y.l, kGenY, 48);
+  return g;
+}
+
+int32_t put_generator(Engine* E, uint32_t slot) {
+  const cdl_g1_affine g = generator();
   return E->upload_points(slot, &g, 1);
 }
 
@@ -890,6 +895,19 @@ cdlh::Fr tracker_challenge(const uint8_t* kG, const uint8_t* krG, const uint8_t*
   tr.append_points("tracker_opening_proof", B, 1);
   return tr.challenge("tracker_opening_proof_challenge");
 }
+
+// the end of whisk.GenerateWhiskTrackerProof (whisk/whisk.go:149-176) once kG, A = blinder*G and B = blinder*rG
+// are encoded: the challenge and the 128-byte proof A | B | s with s = blinder - challenge*k
+void write_tracker_proof(uint8_t* out, const uint8_t* tracker, const uint8_t* kG, const uint8_t* A, const uint8_t* B,
+                         const Fr& k, const Fr& blinder) {
+  const Fr ch = tracker_challenge(kG, tracker + 48, tracker, A, B);
+  memcpy(out, A, 48);
+  memcpy(out + 48, B, 48);
+  cdlh::fr_to_bytes_be(out + 96, cdlh::fr_sub(blinder, cdlh::fr_mul(ch, k)));
+}
+
+// scalars of one validator's registration, all multiples of G: r, k*r, k, blinder, blinder*r
+constexpr size_t kRegScalars = 5;
 }  // namespace
 
 int32_t cdl_whisk_generate_tracker_proof_batch(cdl_ctx* c, size_t B, const uint8_t* trackers, const cdl_fr* ks,
@@ -932,14 +950,62 @@ int32_t cdl_whisk_generate_tracker_proof_batch(cdl_ctx* c, size_t B, const uint8
     uint8_t* out = proofs + 128 * b;
     if (status_out[b] != CDL_OK) { memset(out, 0, 128); return; }
     const uint8_t* kG = enc.data() + 48 * (3 * b);
-    const uint8_t* A = kG + 48;
-    const uint8_t* Bp = kG + 96;
-    const uint8_t* rG = trackers + 96 * b;
-    Fr ch = tracker_challenge(kG, rG + 48, rG, A, Bp);
-    Fr s = cdlh::fr_sub(sc[2 * b + 1], cdlh::fr_mul(ch, sc[2 * b]));  // s = blinder - challenge*k
-    memcpy(out, A, 48);
-    memcpy(out + 48, Bp, 48);
-    cdlh::fr_to_bytes_be(out + 96, s);
+    write_tracker_proof(out, trackers + 96 * b, kG, kG + 48, kG + 96, sc[2 * b], sc[2 * b + 1]);
+  });
+  return CDL_OK;
+}
+
+// The composition "draw r; rG = r*G; krG = k*rG; kG = k*G; cdl_whisk_generate_tracker_proof_batch" with every point
+// written as a multiple of G: k*r and blinder*r are taken mod q on the host, so the five points of every validator
+// come from one Engine::base_mul of G (DESIGN §5e).
+int32_t cdl_whisk_generate_registration_batch(cdl_ctx* c, size_t B, const cdl_fr* ks, cdl_rand* const* rands,
+                                              uint8_t* trackers, uint8_t* k_comms, uint8_t* proofs, int32_t* status) {
+  if (!c || !ks || !rands || !trackers || !k_comms || !proofs || !status || B == 0) return CDL_ERR_INVALID_ARG;
+  if (B > CDL_WHISK_REGISTER_MAX) {
+    std::lock_guard<std::mutex> lk(c->mu);
+    return c->fail(CDL_ERR_TOO_LARGE, "whisk registration: %zu validators exceed 2^21", B);
+  }
+  if (!rands_present(rands, B)) return CDL_ERR_INVALID_ARG;
+  const size_t min_block = cdlh::base_mul_min_block(kRegScalars);
+  if (slots_for(c, B, min_block) > 1)
+    return run_split(c, B, [&](cdl_ctx* lane, size_t lo, size_t hi) {
+      return cdl_whisk_generate_registration_batch(lane, hi - lo, ks + lo, rands + lo, trackers + 96 * lo,
+                                                   k_comms + 48 * lo, proofs + 128 * lo, status + lo);
+    }, false, 1, min_block);
+  std::lock_guard<std::mutex> lk(c->mu);
+  CDL_CUDA(c, cudaSetDevice(c->device));
+  Engine* E = engine_of(c);
+  std::vector<Fr> sc(kRegScalars * B);
+  E->par(B, [&](size_t v) {
+    Fr* s = &sc[kRegScalars * v];
+    const Fr r = rands[v]->r.get_fr();
+    if (cdlh::fr_is_zero(r) || cdlh::fr_eq(r, cdlh::FR_ONE)) {  // refused: s stays zero, the blinder is not drawn
+      status[v] = CDL_ERR_PROTOCOL;
+      return;
+    }
+    Fr k;
+    memcpy(&k, ks + v, 32);
+    const Fr blinder = rands[v]->r.get_fr();
+    s[0] = r;
+    s[1] = cdlh::fr_mul(r, k);  // r < q first: k may have limbs >= q
+    s[2] = k;
+    s[3] = blinder;
+    s[4] = cdlh::fr_mul(blinder, r);
+    status[v] = CDL_OK;
+  });
+  for (size_t v = 0; v < B; v++)
+    if (status[v] != CDL_OK) c->fail(status[v], "whisk registration: validator %zu drew r = 0 or 1", v);
+  // rG krG kG A B of every validator
+  std::vector<uint8_t> enc(48 * sc.size());
+  int32_t rc = E->base_mul(generator(), sc.data(), sc.size(), nullptr, enc.data());
+  if (rc) return rc;
+  E->par(B, [&](size_t v) {
+    if (status[v] != CDL_OK) return;
+    const uint8_t* e = enc.data() + 48 * kRegScalars * v;
+    const Fr* s = &sc[kRegScalars * v];
+    memcpy(trackers + 96 * v, e, 96);
+    memcpy(k_comms + 48 * v, e + 96, 48);
+    write_tracker_proof(proofs + 128 * v, e, e + 96, e + 144, e + 192, s[2], s[3]);
   });
   return CDL_OK;
 }

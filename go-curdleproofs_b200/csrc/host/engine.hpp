@@ -280,6 +280,10 @@ size_t slots_for(cdl_ctx* c, size_t B, size_t min_block = kMinLaneBatch);
 // piece on the slot's lane 0.  Holds c's mutex while the pieces run.
 int32_t run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes = true,
                   size_t align = 1, size_t min_block = kMinLaneBatch);
+// Minimum block of a split call whose units are `per_unit` scalars each of one Engine::base_mul (capi_base_mul.cu):
+// ceil(kBaseSlotScalars / per_unit) units, so that every slot's base_mul takes the table path exactly when the
+// one-device call would.
+size_t base_mul_min_block(size_t per_unit);
 // run_split for a caller that already holds c's mutex (and keeps it for work after the pieces)
 int32_t run_split_locked(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn,
                          bool lanes, size_t align, size_t min_block);

@@ -71,8 +71,9 @@ int32_t cdl_create(int device, cdl_ctx** out);
  * cdl_g1_msm of more than 1 024 terms (and cdl_g1_sum_affine through it) over D' = max(1, min(n, terms /
  * 65 536)) slots, so from 131 072 terms on; slot s sums its contiguous block of the terms and the D' partial
  * sums are added on devices[0].  cdl_g1_batch_scalar_mul_base over D' = max(1, min(n, scalars / 32 768))
- * slots, so from 65 536 scalars on; slot s multiplies its contiguous block with its own cached tables.  Below
- * these sizes both run on slot 0 exactly as on a one-device context.
+ * slots, so from 65 536 scalars on; slot s multiplies its contiguous block with its own cached tables.
+ * cdl_whisk_generate_registration_batch likewise over D' = max(1, min(n, B / 6 554)) slots, in blocks of
+ * validators.  Below these sizes they run on slot 0 exactly as on a one-device context.
  *
  * Everything else runs on slot 0's device (devices[0]): the other cdl_g1_* primitives, cdl_g1_msm_batch,
  * the device and sharded MSMs, cdl_dev_* buffers (device memory of devices[0]), cdl_rand_get_g1_affines and
@@ -291,6 +292,26 @@ int32_t cdl_whisk_generate_tracker_proof_batch(cdl_ctx* ctx, size_t B, const uin
  * ok[b] is the reference's bool, status[b] its error (CDL_ERR_DECODE for malformed proof / points). */
 int32_t cdl_whisk_is_valid_tracker_proof_batch(cdl_ctx* ctx, size_t B, const uint8_t* trackers, const uint8_t* k_comms,
                                                const uint8_t* proofs, int32_t* ok, int32_t* status);
+/* Whisk registration material for B validators (first-proposal registration, checked by
+ * process_whisk_registration): for validator b with secret ks[b] (gnark fr.Element, read as
+ * cdl_whisk_generate_tracker_proof_batch reads it, limbs >= r included), r = the next Fr drawn from rands[b];
+ * trackers + 96 b = {r*G, k*r*G} compressed, k_comms + 48 b = k*G, proofs + 128 b = the opening proof that
+ * cdl_whisk_generate_tracker_proof_batch gives for that tracker and k with rands[b] as left after drawing r
+ * (it draws one blinder).  The bytes and the Rand positions are those of that composition (draw r,
+ * cdl_g1_batch_scalar_mul_base, cdl_g1_scalar_mul_affine, cdl_g1_batch_scalar_mul_base for k*G, then the proof
+ * call), but every point is a multiple of G (k*r and blinder*r are formed on the host), so the call is one
+ * fixed-base multiplication of 5 B scalars by G, from G's cached table as cdl_g1_batch_scalar_mul_base runs it.
+ * rands[b] must be a distinct Rand per validator (the validators draw concurrently; a Rand listed twice races).
+ * status[b] = CDL_ERR_PROTOCOL when r is 0 or 1 (rG at infinity or rG == G); such a validator draws no blinder
+ * and its outputs are left as they were.
+ * On a context of several device slots a call of at least 2 * 6 554 validators is split (cdl_create_devices),
+ * each slot multiplying the 5 * 6 554 or more scalars of its block; the results do not depend on the device list.
+ * Returns CDL_OK when the arguments are valid, whatever the statuses; CDL_ERR_INVALID_ARG for a null pointer
+ * or B == 0; CDL_ERR_TOO_LARGE for B > CDL_WHISK_REGISTER_MAX, before any Rand is drawn. */
+#define CDL_WHISK_REGISTER_MAX (1u << 21)
+int32_t cdl_whisk_generate_registration_batch(cdl_ctx* ctx, size_t B, const cdl_fr* ks, cdl_rand* const* rands,
+                                              uint8_t* trackers, uint8_t* k_comms, uint8_t* proofs,
+                                              int32_t* status);
 /* Which of the caller's Whisk secrets own which trackers.  trackers: T x 96 bytes {rG, krG} as in
  * cdl_whisk_generate_tracker_proof_batch; ks: V secrets (gnark fr.Element, Montgomery).
  * owner[t] = the smallest v with ks[v] * rG_t == krG_t (equal as group elements), else -1.
@@ -322,7 +343,8 @@ int32_t cdl_host_selftest_fibers(uint32_t n, uint32_t rounds, uint8_t* digest32,
  * multiplication, 2 decompress, 3 compress / normalise): launches, CUDA-event milliseconds on the
  * launching stream, algorithmic modmul (SURVEY.md §8d conventions; 3 193 per matched (key, tracker)
  * pair and per scalar of cdl_g1_batch_scalar_mul_base, which counts one class-1 launch per chunk of
- * up to 2^20 scalars) and algorithmic bytes.  Each output array has 4 entries. */
+ * up to 2^20 scalars; cdl_whisk_generate_registration_batch counts as that call on its 5 B scalars) and
+ * algorithmic bytes.  Each output array has 4 entries. */
 int32_t cdl_engine_stats(cdl_ctx* ctx, uint64_t* launches, double* ms, double* modmul, double* bytes, int reset);
 /* Device busy time since the last cdl_engine_stats(.., reset = 1): the length of
  * the union of all timed kernel intervals over every lane's stream (lanes overlap,
@@ -338,8 +360,9 @@ int32_t cdl_engine_busy_ms_device(cdl_ctx* ctx, size_t slot, double* busy_ms);
  * lanes' kernels.  Results do not depend on it.  Also environment CDL_LANES.
  * With several device slots this is the number of lanes per slot. */
 int32_t cdl_set_lanes(cdl_ctx* ctx, int32_t lanes);
-/* Number of GPU kernels launched by protocol-level calls, batched MSMs, tracker matching and
- * cdl_g1_batch_scalar_mul_base on this context so far, summed over its device slots. */
+/* Number of GPU kernels launched by protocol-level calls, batched MSMs, tracker matching,
+ * cdl_g1_batch_scalar_mul_base and cdl_whisk_generate_registration_batch on this context so far, summed over
+ * its device slots. */
 uint64_t cdl_launch_count(cdl_ctx* ctx);
 
 /* ---- large MSM, device-resident vectors, multi-GPU ----------------------

@@ -192,6 +192,32 @@ func (c *Context) MatchWhiskTrackers(trackers []byte, ks []fr.Element) (owner, s
 	return owner, status, nil
 }
 
+// GenerateWhiskRegistrationBatch prepares the first-proposal Whisk registration of len(ks) validators: validator b
+// draws r from rands[b] and gets the fresh tracker {r·G, k·r·G} (96 bytes), its k-commitment k·G (48 bytes) and
+// the opening proof GenerateWhiskTrackerProof gives for them (128 bytes, one blinder drawn from rands[b] after
+// r).  status[b] == CDL_ERR_PROTOCOL when r is 0 or 1 (rG at infinity or rG == G, which
+// process_whisk_registration refuses); that validator draws no blinder and its bytes stay zero.  rands must hold
+// one distinct *Rand per validator: the validators draw concurrently, so a Rand passed for two validators is a
+// data race (a tool with one RNG for all validators draws into separate Rands, or seeds one per validator).
+func (c *Context) GenerateWhiskRegistrationBatch(ks []fr.Element, rands []*Rand) (trackers, kComms, proofs []byte,
+	status []int32, err error) {
+	B := len(ks)
+	if B == 0 || len(rands) != B {
+		return nil, nil, nil, nil, errStatus(C.int32_t(C.CDL_ERR_INVALID_ARG))
+	}
+	trackers = make([]byte, B*TrackerSize)
+	kComms = make([]byte, B*48)
+	proofs = make([]byte, B*C.CDL_WHISK_TRACKER_PROOF_SIZE)
+	status = make([]int32, B)
+	rc := C.cdl_whisk_generate_registration_batch(c.h, C.size_t(B), frPtr(ks), randHandles(rands),
+		(*C.uint8_t)(unsafe.Pointer(&trackers[0])), (*C.uint8_t)(unsafe.Pointer(&kComms[0])),
+		(*C.uint8_t)(unsafe.Pointer(&proofs[0])), (*C.int32_t)(unsafe.Pointer(&status[0])))
+	if rc != 0 {
+		return nil, nil, nil, nil, c.err(rc)
+	}
+	return trackers, kComms, proofs, status, nil
+}
+
 func randHandles(rands []*Rand) **C.cdl_rand {
 	hs := make([]*C.cdl_rand, len(rands))
 	for i, r := range rands {
