@@ -1,5 +1,6 @@
 // C ABI of libcurdle_b200.so (include/curdle_b200.h): context, device buffers,
 // host-pointer entry points that mirror the gnark-crypto calls of the reference.
+#include <algorithm>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -28,6 +29,34 @@ static bool msm_tasks(const uint32_t* offsets, size_t k, std::vector<MsmTask>& t
     tasks[j] = MsmTask{offsets[j], offsets[j + 1] - offsets[j], (uint32_t)j, 0};
   }
   return true;
+}
+
+// Terms per device slot from which cdl_g1_msm_batch is split over the slots of a multi-device context: the value
+// of kMsmSlotTerms (capi_msm.cu), not measured for this call.
+constexpr size_t kMsmBatchSlotTerms = 65536;
+
+// The MSM blocks of cdl_g1_msm_batch on c (offsets monotone): slot s of the D' = slots_for(c, terms,
+// kMsmBatchSlotTerms) slots takes MSMs [cut[s], cut[s + 1]), cut at the MSM boundary nearest to the term at which
+// shard_bounds(terms, D', s) starts, so the blocks balance terms, not MSMs.  Equal offsets cut before the first
+// of them, and trailing empty MSMs join the last block, so every non-empty block holds terms.  Empty when fewer
+// than two blocks hold terms (one MSM holding every term, a lane, a small call): the call does not split.
+static std::vector<size_t> msm_batch_cuts(cdl_ctx* c, const uint32_t* offsets, size_t k) {
+  const size_t first = offsets[0], terms = offsets[k] - first;
+  const size_t D = cdlh::slots_for(c, terms, kMsmBatchSlotTerms);
+  std::vector<size_t> cut(D + 1, k);
+  cut[0] = 0;
+  size_t busy = 0;
+  for (size_t s = 1; s <= D; s++) {
+    if (s < D) {
+      const size_t t = first + cdlh::shard_lo(terms, D, s);
+      const uint32_t* hi = std::lower_bound(offsets, offsets + k + 1, t);  // offsets[k] >= t
+      const uint32_t v = hi > offsets && t - hi[-1] < hi[0] - t ? hi[-1] : hi[0];
+      cut[s] = v == offsets[k] ? k : (size_t)(std::lower_bound(offsets, offsets + k + 1, v) - offsets);
+    }
+    busy += offsets[cut[s]] > offsets[cut[s - 1]];
+  }
+  if (busy < 2) cut.clear();
+  return cut;
 }
 
 extern "C" {
@@ -170,6 +199,14 @@ int32_t cdl_g1_msm_batch(cdl_ctx* c, const cdl_g1_affine* points, const cdl_fr* 
   // the bases go to pool slots [k, k + total); pool indices are 30 bits (bit 31 negates, bit 30 is the kernels' flag)
   if (k + total >= (1u << 30))
     return c->fail(CDL_ERR_INVALID_ARG, "msm_batch: %zu MSMs of %zu terms exceed the 2^30-point pool", k, total);
+  // on several slots, whole MSMs per slot with rebased offsets (the checks above ran on the whole call)
+  const std::vector<size_t> cut = msm_batch_cuts(c, offsets, k);
+  if (!cut.empty())
+    return cdlh::run_blocks_locked(c, cut, [&](cdl_ctx* l, size_t j0, size_t j1) {
+      std::vector<uint32_t> offs(j1 - j0 + 1);
+      for (size_t j = j0; j <= j1; j++) offs[j - j0] = offsets[j] - offsets[j0];
+      return cdl_g1_msm_batch(l, points + offsets[j0], scalars + offsets[j0], offs.data(), j1 - j0, out + j0);
+    }, false);
   CDL_CUDA(c, cudaSetDevice(c->device));
   c->spin_wait = true;  // latency regime, as for small protocol batches: see cdl_ctx::sync_stream
   cdlh::Engine* E = cdlh::engine_of(c);
@@ -274,20 +311,47 @@ static int32_t scalar_mul_impl(cdl_ctx* c, const cdl_g1_affine* in, const cdl_fr
   return CDL_OK;
 }
 
+// Points per device slot from which cdl_g1_scalar_mul_affine is split over the slots of a multi-device context,
+// every slot running its block on its lane 0.  Measured on one B200 (tools/primitive_sweep.py,
+// profiles/r10_primitive_slot_sweep.txt): from blocks of 4 096 points, halving a call takes more kernel time off
+// it than a call's fixed cost (uploads, launch, wait and download: 0.11 ms); below, the GLV kernel is latency-bound.
+constexpr size_t kScalarMulSlotPoints = 4096;
+
 int32_t cdl_g1_scalar_mul_affine(cdl_ctx* c, const cdl_g1_affine* in, const cdl_fr* s, size_t n,
                                  size_t scalar_stride, cdl_g1_affine* out) {
   if (!c || (n && (!in || !s || !out)) || scalar_stride > 1) return CDL_ERR_INVALID_ARG;
+  if (cdlh::slots_for(c, n, kScalarMulSlotPoints) > 1)  // a broadcast scalar goes to every block
+    return cdlh::run_split(c, n, [&](cdl_ctx* l, size_t lo, size_t hi) {
+      return cdl_g1_scalar_mul_affine(l, in + lo, s + scalar_stride * lo, hi - lo, scalar_stride, out + lo);
+    }, false, 1, kScalarMulSlotPoints);
   return scalar_mul_impl(c, in, s, n, scalar_stride, nullptr, out);
 }
 
+// Points per device slot from which cdl_g1_fold is split, measured as for kScalarMulSlotPoints (the same kernel
+// with an addend): halving a call saves 0.004 ms of kernel time at blocks of 2 048 points and 0.29 ms at 4 096,
+// against a fixed cost of 0.03 ms
+constexpr size_t kFoldSlotPoints = 4096;
+
 int32_t cdl_g1_fold(cdl_ctx* c, cdl_g1_affine* L, const cdl_g1_affine* R, const cdl_fr* x, size_t n) {
   if (!c || (n && (!L || !R || !x))) return CDL_ERR_INVALID_ARG;
+  if (cdlh::slots_for(c, n, kFoldSlotPoints) > 1)
+    return cdlh::run_split(c, n, [&](cdl_ctx* l, size_t lo, size_t hi) {
+      return cdl_g1_fold(l, L + lo, R + lo, x, hi - lo);
+    }, false, 1, kFoldSlotPoints);
   return scalar_mul_impl(c, R, x, n, 0, L, L);
 }
+
+// Points per device slot from which cdl_g1_batch_to_affine is split, measured as for kScalarMulSlotPoints: the
+// kernel time halving a call saves reaches the fixed cost (0.027 ms) from blocks of 32 768 points
+constexpr size_t kToAffineSlotPoints = 32768;
 
 int32_t cdl_g1_batch_to_affine(cdl_ctx* c, const cdl_g1_jac* in, size_t n, cdl_g1_affine* out) {
   if (!c || (n && (!in || !out))) return CDL_ERR_INVALID_ARG;
   if (n == 0) return CDL_OK;
+  if (cdlh::slots_for(c, n, kToAffineSlotPoints) > 1)
+    return cdlh::run_split(c, n, [&](cdl_ctx* l, size_t lo, size_t hi) {
+      return cdl_g1_batch_to_affine(l, in + lo, hi - lo, out + lo);
+    }, false, 1, kToAffineSlotPoints);
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   if (!c->in.grow(n * sizeof(G1Jac), c->stream) || !c->out.grow(n * sizeof(G1Affine), c->stream))
@@ -303,9 +367,17 @@ int32_t cdl_g1_batch_to_affine(cdl_ctx* c, const cdl_g1_jac* in, size_t n, cdl_g
 }
 
 // --------------------------------------------------------------------- codecs
+// Points per device slot from which cdl_g1_compress is split, measured as for kScalarMulSlotPoints: the kernel
+// time halving a call saves reaches the fixed cost (0.019 ms) from blocks of 131 072 points
+constexpr size_t kCompressSlotPoints = 131072;
+
 int32_t cdl_g1_compress(cdl_ctx* c, const cdl_g1_affine* in, size_t n, uint8_t* out48) {
   if (!c || (n && (!in || !out48))) return CDL_ERR_INVALID_ARG;
   if (n == 0) return CDL_OK;
+  if (cdlh::slots_for(c, n, kCompressSlotPoints) > 1)
+    return cdlh::run_split(c, n, [&](cdl_ctx* l, size_t lo, size_t hi) {
+      return cdl_g1_compress(l, in + lo, hi - lo, out48 + 48 * lo);
+    }, false, 1, kCompressSlotPoints);
   std::lock_guard<std::mutex> lk(c->mu);
   CDL_CUDA(c, cudaSetDevice(c->device));
   if (!c->in.grow(n * sizeof(G1Affine), c->stream) || !c->out.grow(n * 48, c->stream))
@@ -320,10 +392,30 @@ int32_t cdl_g1_compress(cdl_ctx* c, const cdl_g1_affine* in, size_t n, uint8_t* 
   return CDL_OK;
 }
 
+// CDL_ERR_DECODE naming the first rejected point of status[0 .. n), else CDL_OK
+static int32_t decode_verdict(cdl_ctx* c, const uint8_t* status, size_t n) {
+  for (size_t i = 0; i < n; i++)
+    if (status[i]) return c->fail(CDL_ERR_DECODE, "g1 decompress: point %zu rejected (reason %u)", i, (unsigned)status[i]);
+  return CDL_OK;
+}
+
+// Points per device slot from which cdl_g1_decompress is split, measured as for kScalarMulSlotPoints: the kernel
+// time halving a call saves reaches the fixed cost (0.034 ms) from blocks of 16 384 points
+constexpr size_t kDecompressSlotPoints = 16384;
+
 int32_t cdl_g1_decompress(cdl_ctx* c, const uint8_t* in48, size_t n, cdl_g1_affine* out, uint8_t* status) {
   if (!c || (n && (!in48 || !out || !status))) return CDL_ERR_INVALID_ARG;
   if (n == 0) return CDL_OK;
   std::lock_guard<std::mutex> lk(c->mu);
+  if (cdlh::slots_for(c, n, kDecompressSlotPoints) > 1) {
+    // every block writes all of its points and statuses; the verdict is then taken over the whole call, so that
+    // it names the call's first rejected point as the one-device call does
+    const int32_t rc = cdlh::run_split_locked(c, n, [&](cdl_ctx* l, size_t lo, size_t hi) {
+      const int32_t r = cdl_g1_decompress(l, in48 + 48 * lo, hi - lo, out + lo, status + lo);
+      return r == CDL_ERR_DECODE ? CDL_OK : r;
+    }, false, 1, kDecompressSlotPoints);
+    return rc ? rc : decode_verdict(c, status, n);
+  }
   CDL_CUDA(c, cudaSetDevice(c->device));
   if (!c->in.grow(n * 48, c->stream) || !c->out.grow(n * sizeof(G1Affine), c->stream) || !c->status.grow(n, c->stream))
     return c->fail(CDL_ERR_CUDA, "device allocation failed");
@@ -336,9 +428,7 @@ int32_t cdl_g1_decompress(cdl_ctx* c, const uint8_t* in48, size_t n, cdl_g1_affi
   CDL_CUDA(c, cudaMemcpyAsync(out, d_out, n * sizeof(G1Affine), cudaMemcpyDeviceToHost, c->stream));
   CDL_CUDA(c, cudaMemcpyAsync(status, d_st, n, cudaMemcpyDeviceToHost, c->stream));
   CDL_CUDA(c, cudaStreamSynchronize(c->stream));
-  for (size_t i = 0; i < n; i++)
-    if (status[i]) return c->fail(CDL_ERR_DECODE, "g1 decompress: point %zu rejected (reason %u)", i, (unsigned)status[i]);
-  return CDL_OK;
+  return decode_verdict(c, status, n);
 }
 
 // --------------------------------------------------------------------- diagnostics

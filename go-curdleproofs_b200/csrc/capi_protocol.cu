@@ -152,8 +152,7 @@ size_t cdlh::slots_for(cdl_ctx* c, size_t B, size_t min_block) {
   return std::max<size_t>(1, std::min<size_t>(c->slots.size(), B / min_block));
 }
 
-// first unit of block s when B units are dealt to D slots in contiguous blocks (sharding.shard_bounds)
-static size_t shard_lo(size_t B, size_t D, size_t s) { return s * (B / D) + std::min(s, B % D); }
+size_t cdlh::shard_lo(size_t B, size_t D, size_t s) { return s * (B / D) + std::min(s, B % D); }
 
 int32_t cdlh::run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes,
                         size_t align, size_t min_block) {
@@ -163,15 +162,18 @@ int32_t cdlh::run_split(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ct
 
 int32_t cdlh::run_split_locked(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn,
                                bool lanes, size_t align, size_t min_block) {
+  const size_t D = slots_for(c, B, min_block);
+  std::vector<size_t> bounds(D + 1, B);
+  for (size_t s = 0; s < D; s++) bounds[s] = std::min(B, (shard_lo(B, D, s) + align / 2) / align * align);
+  return run_blocks_locked(c, bounds, fn, lanes);
+}
+
+int32_t cdlh::run_blocks_locked(cdl_ctx* c, const std::vector<size_t>& bounds,
+                                const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes) {
   struct Piece { cdl_ctx* ctx; size_t lo, hi; };
   std::vector<Piece> pieces;
-  const size_t D = slots_for(c, B, min_block);
-  auto bound = [&](size_t s) {
-    if (s == D) return B;
-    return std::min(B, (shard_lo(B, D, s) + align / 2) / align * align);
-  };
-  for (size_t s = 0; s < D; s++) {
-    const size_t lo = bound(s), n = bound(s + 1) - lo;
+  for (size_t s = 0; s + 1 < bounds.size(); s++) {
+    const size_t lo = bounds[s], n = bounds[s + 1] - lo;
     if (!n) continue;
     const size_t G = lanes ? lanes_for(c, n) : 1;
     for (size_t g = 0; g < G; g++) {

@@ -287,5 +287,11 @@ size_t base_mul_min_block(size_t per_unit);
 // run_split for a caller that already holds c's mutex (and keeps it for work after the pieces)
 int32_t run_split_locked(cdl_ctx* c, size_t B, const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn,
                          bool lanes, size_t align, size_t min_block);
+// run_split_locked with the caller's blocks: slot s takes [bounds[s], bounds[s + 1]) (bounds non-decreasing, at
+// most one block per slot; empty blocks are skipped)
+int32_t run_blocks_locked(cdl_ctx* c, const std::vector<size_t>& bounds,
+                          const std::function<int32_t(cdl_ctx*, size_t, size_t)>& fn, bool lanes);
+// first unit of block s when B units are dealt to D slots in contiguous blocks (sharding.shard_bounds)
+size_t shard_lo(size_t B, size_t D, size_t s);
 
 }  // namespace cdlh

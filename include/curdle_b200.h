@@ -67,17 +67,25 @@ int32_t cdl_create(int device, cdl_ctx** out);
  * as a one-device context cuts a batch.  A call of fewer than 64 instances, and every single
  * (non-batched) protocol call, runs on slot 0.
  *
- * Two single calls split by size, each slot running its block on its lane 0 (one piece per slot):
+ * Single calls split by size, each slot running its block on its lane 0 (one piece per slot):
  * cdl_g1_msm of more than 1 024 terms (and cdl_g1_sum_affine through it) over D' = max(1, min(n, terms /
  * 65 536)) slots, so from 131 072 terms on; slot s sums its contiguous block of the terms and the D' partial
  * sums are added on devices[0].  cdl_g1_batch_scalar_mul_base over D' = max(1, min(n, scalars / 32 768))
  * slots, so from 65 536 scalars on; slot s multiplies its contiguous block with its own cached tables.
  * cdl_whisk_generate_registration_batch likewise over D' = max(1, min(n, B / 6 554)) slots, in blocks of
- * validators.  Below these sizes they run on slot 0 exactly as on a one-device context.
+ * validators.  The elementwise calls split by points the same way, each with its own minimum block kMin
+ * over D' = max(1, min(n, points / kMin)) slots: cdl_g1_decompress (16 384), cdl_g1_compress (131 072),
+ * cdl_g1_batch_to_affine (32 768), cdl_g1_scalar_mul_affine (4 096) and cdl_g1_fold (4 096); slot s writes
+ * its contiguous range of the outputs.  cdl_g1_msm_batch splits at MSM boundaries over D' = max(1, min(n,
+ * terms / 65 536)) slots: slot s takes whole, contiguous MSMs, the blocks balanced by terms, and a call whose
+ * terms all sit in one MSM does not split.  Below 2 * kMin units every one of these calls runs on slot 0
+ * exactly as on a one-device context.  A split call returns what the one-device call returns: the same
+ * bytes, status, return code and cdl_last_error text.  Its blocks read their inputs and write their outputs
+ * concurrently, so outputs may be the inputs themselves (in place) but must not overlap them otherwise.
  *
- * Everything else runs on slot 0's device (devices[0]): the other cdl_g1_* primitives, cdl_g1_msm_batch,
- * the device and sharded MSMs, cdl_dev_* buffers (device memory of devices[0]), cdl_rand_get_g1_affines and
- * CRS generation.
+ * Everything else runs on slot 0's device (devices[0]): cdl_g1_msm and cdl_g1_sum_affine of at most 1 024
+ * terms, the entry points on device vectors (*_device, including cdl_g1_msm_batch_device), the sharded MSMs,
+ * cdl_dev_* buffers (device memory of devices[0]), cdl_fp_mul, cdl_rand_get_g1_affines and CRS generation.
  * cdl_comm_init refuses a context of more than one slot: the NCCL-sharded MSM runs one process (and
  * one single-device context) per GPU.
  * CDL_ERR_INVALID_ARG for n == 0, n > 16 or a device id out of range; CDL_ERR_NO_DEVICE without a
@@ -113,7 +121,10 @@ int32_t cdl_g1_msm(cdl_ctx* ctx, const cdl_g1_affine* points, const cdl_fr* scal
  * [offsets[j], offsets[j+1]).  Affine results.  Covers the 4 / 6 MSMs of one
  * IPA / SameMSM round (innerproductargument.go:108-138,
  * samemultiscalarargument.go:93-111) and the verifier's tiny MSMs
- * (innerproductargument.go:238,250,275,281). */
+ * (innerproductargument.go:238,250,275,281).
+ * CDL_ERR_INVALID_ARG for offsets that decrease or when k + offsets[k] >= 2^30 (the point pool), before any
+ * input is read.  On a context of several device slots, from 2 * 65 536 terms held by at least two MSMs, the
+ * MSMs are dealt to the slots in contiguous groups of whole MSMs balanced by terms (cdl_create_devices). */
 int32_t cdl_g1_msm_batch(cdl_ctx* ctx, const cdl_g1_affine* points, const cdl_fr* scalars,
                          const uint32_t* offsets, size_t k, cdl_g1_affine* out);
 
@@ -122,13 +133,15 @@ int32_t cdl_g1_msm_batch(cdl_ctx* ctx, const cdl_g1_affine* points, const cdl_fr
  * (common/util.go:55-63); scalar_stride == 1 gives per-element scalars:
  * Gs'[i] = beta^-(i+1) * Gs[i] (grandproductargument.go:94-103).  The scalar is
  * the fr.Element itself (the reference converts it with common.FrToBigInt,
- * common/util.go:16-20). */
+ * common/util.go:16-20).  Split by points from 2 * 4 096 points on a context of several device slots; a
+ * broadcast scalar goes to every block. */
 int32_t cdl_g1_scalar_mul_affine(cdl_ctx* ctx, const cdl_g1_affine* in, const cdl_fr* s, size_t n,
                                  size_t scalar_stride, cdl_g1_affine* out);
 
 /* Base folding L[i] += x * R[i], i < n, result affine in place.
  * Replaces the serial loops innerproductargument.go:155-166 (called with x =
- * gamma for G and gamma^-1 for G') and samemultiscalarargument.go:129-135. */
+ * gamma for G and gamma^-1 for G') and samemultiscalarargument.go:129-135.
+ * Split by points from 2 * 4 096 points on a context of several device slots. */
 int32_t cdl_g1_fold(cdl_ctx* ctx, cdl_g1_affine* L, const cdl_g1_affine* R, const cdl_fr* x, size_t n);
 
 /* bls12381.BatchScalarMultiplicationG1: out[i] = scalars[i] * base, i < n, for one base and many scalars: the
@@ -156,21 +169,25 @@ int32_t cdl_g1_fold(cdl_ctx* ctx, cdl_g1_affine* L, const cdl_g1_affine* R, cons
 int32_t cdl_g1_batch_scalar_mul_base(cdl_ctx* ctx, const cdl_g1_affine* base, const cdl_fr* scalars, size_t n,
                                      cdl_g1_affine* out, uint8_t* out48);
 
-/* bls12381.BatchJacobianToAffineG1 (transcript/transcript.go:26 and every Serialize). */
+/* bls12381.BatchJacobianToAffineG1 (transcript/transcript.go:26 and every Serialize).  Split by points from
+ * 2 * 32 768 points on a context of several device slots. */
 int32_t cdl_g1_batch_to_affine(cdl_ctx* ctx, const cdl_g1_jac* in, size_t n, cdl_g1_affine* out);
 
 /* sum of n affine points (crs.go:41-48 Gsum / Hsum). */
 int32_t cdl_g1_sum_affine(cdl_ctx* ctx, const cdl_g1_affine* in, size_t n, cdl_g1_affine* out);
 
 /* G1Affine.Bytes() for n points -> n * 48 compressed bytes
- * (transcript/transcript.go:35, whisk/types.go:79-84). */
+ * (transcript/transcript.go:35, whisk/types.go:79-84).  Split by points from 2 * 131 072 points on a
+ * context of several device slots. */
 int32_t cdl_g1_compress(cdl_ctx* ctx, const cdl_g1_affine* in, size_t n, uint8_t* out48);
 
 /* G1Affine.SetBytes on n 48-byte compressed encodings, with curve and
  * subgroup checks (whisk/types.go:86-95; Decoder in curdleproof.go:320-356).
  * status[i] == 0 on success, else a positive reason code (1 bad flags /
  * uncompressed, 2 non-canonical x, 3 no square root, 4 not in subgroup,
- * 5 bad infinity padding).  Returns CDL_ERR_DECODE if any point failed. */
+ * 5 bad infinity padding).  Returns CDL_ERR_DECODE if any point failed; cdl_last_error then names the
+ * first rejected point.  Every point and status is written either way.  Split by points from 2 * 16 384
+ * points on a context of several device slots, with the same statuses, return code and message. */
 int32_t cdl_g1_decompress(cdl_ctx* ctx, const uint8_t* in48, size_t n, cdl_g1_affine* out, uint8_t* status);
 
 /* ---- protocol level: the reference's public API, batched on the GPU ------

@@ -9,13 +9,16 @@ warm-up call per row:
   whisk_validate    the validation call alone;
   prove_batch       cdl_prove_batch at ell = 124, B = 1 024 * D caller-supplied instances;
   match             cdl_whisk_match_trackers, 8 192 trackers x 16 384 keys;
-and, with --rows bulk (those rows alone) or --rows all (before the others), the two single calls that split by
+and, with --rows bulk (those rows alone) or --rows all (before the others), the single calls that split by
 size; the base_mul rows at 2^24 hold a 512 MB scalar vector and up to 1.6 GB of results per call:
   msm               cdl_g1_msm on host vectors at n = 2^16, 2^17, 2^18, 2^20 and 2^22 (a 2^20 set of points
                     repeated, its scalars rotated per repetition), wall time only (large MSMs are not in the
                     engine's accounting);
   base_mul          cdl_g1_batch_scalar_mul_base with a warm table at n = 2^16, 2^20, 2^22 and 2^24, affine and
-                    compressed results.
+                    compressed results;
+  decompress, compress, batch_to_affine (Z = 1), scalar_mul_affine (per-point scalars), fold
+                    the elementwise calls on n = 2^20 and 2^22 points, wall time only;
+  msm_batch         cdl_g1_msm_batch of 64 equal MSMs of n / 64 terms, n = 2^20 and 2^22.
 Every row gives the median of --reps timed calls and the busy time of every device slot
 (cdl_engine_busy_ms_device, union of that slot's kernel intervals) summed over the timed calls of the row.
 Rows marked [0, 0] run two slots on GPU 0: what the split costs on one GPU (one PCIe link, one device), not a
@@ -146,6 +149,7 @@ def measure(pkg, devices, reps, out):
 
 MSM_SIZES = [1 << 16, 1 << 17, 1 << 18, 1 << 20, 1 << 22]
 BASE_SIZES = [1 << 16, 1 << 20, 1 << 22, 1 << 24]
+PRIM_SIZES = [1 << 20, 1 << 22]
 SET = 1 << 20
 
 
@@ -159,8 +163,11 @@ def bulk_inputs(pkg):
     raw2 = rng.integers(0, 256, size=(SET, 32), dtype=np.uint8)
     raw2[:, 31] &= 0x3F
     base = aff_enc(b.g1_mul(b.G1_GEN, 0x1234567890ABCDEF))
+    enc = ctx.g1_compress(pts)
+    one = np.frombuffer(pow(2, 384, b.P).to_bytes(48, "little"), dtype=np.uint8)
+    jac = np.concatenate([np.frombuffer(pts, dtype=np.uint8).reshape(SET, 96), np.tile(one, (SET, 1))], axis=1)
     ctx.close()
-    return pts, raw2.tobytes(), base
+    return pts, raw2.tobytes(), base, enc, jac.tobytes()
 
 
 def scalars(inputs, n):
@@ -169,9 +176,9 @@ def scalars(inputs, n):
     return b"".join(sc[32 * r:] + sc[:32 * r] for r in range(-(-n // SET)))[:32 * n]
 
 
-def points(inputs, n):
-    """n points: the 2^20 set repeated"""
-    return (inputs[0] * -(-n // SET))[:96 * n]
+def points(inputs, n, which=0, unit=96):
+    """n points: the 2^20 set repeated (which = 3: encodings, 4: Jacobian forms)"""
+    return (inputs[which] * -(-n // SET))[:unit * n]
 
 
 def measure_bulk(pkg, devices, reps, inputs, out):
@@ -191,6 +198,23 @@ def measure_bulk(pkg, devices, reps, inputs, out):
             t, busy = timed(ctx, D, reps, lambda i: ctx.g1_batch_scalar_mul_base(base, S, **kw))
             rows.append(f"  {str(devices):14s} base_mul {kind:10s} n={n:>10d}  {n / t / 1e6:10.2f} M/s        median "
                         f"{t * 1e3:9.2f} ms   busy per slot ms: {' / '.join(f'{x:.1f}' for x in busy)}")
+    for n in PRIM_SIZES:
+        P, S = points(inputs, n), scalars(inputs, n)
+        E, J = points(inputs, n, 3, 48), points(inputs, n, 4, 144)
+        Rf = P[96:] + P[:96]
+        offs = [n * j // 64 for j in range(65)]
+        calls = [("decompress", lambda i: ctx.g1_decompress(E)),
+                 ("compress", lambda i: ctx.g1_compress(P)),
+                 ("batch_to_affine", lambda i: ctx.g1_batch_to_affine(J)),
+                 ("scalar_mul_affine", lambda i: ctx.g1_scalar_mul_affine(P, S, broadcast=False)),
+                 ("fold", lambda i: ctx.g1_fold(P, Rf, S[:32])),
+                 ("msm_batch", lambda i: ctx.g1_msm_batch(P, S, offs))]
+        for name, fn in calls:
+            t, busy = timed(ctx, D, reps, fn)
+            line = f"  {str(devices):14s} {name:17s} n={n:>10d}  {n / t / 1e6:10.2f} M/s        median {t * 1e3:9.2f} ms"
+            if name == "msm_batch":
+                line += f"   busy per slot ms: {' / '.join(f'{x:.1f}' for x in busy)}"
+            rows.append(line)
     ctx.close()
     for line in rows:
         print(line, file=out, flush=True)
@@ -216,8 +240,8 @@ def main():
     ap.add_argument("--bench-warmup", type=int, default=2)
     ap.add_argument("--out", default="", help="also write the report to this file")
     ap.add_argument("--rows", choices=["protocol", "bulk", "all"], default="protocol",
-                    help="protocol (default): the batched calls and the bench.py comparison; bulk: msm and base_mul; "
-                         "all: both")
+                    help="protocol (default): the batched calls and the bench.py comparison; bulk: the single calls "
+                         "that split by size; all: both")
     args = ap.parse_args()
     import torch
 
