@@ -56,9 +56,7 @@ using FrM = Mont<FrParams>;
 using Fp = FpM::El;  // 48 bytes == gnark fp.Element
 using Fr = FrM::El;  // 32 bytes == gnark fr.Element
 
-// public exponents, little-endian 32-bit words
-// (p+1)/4
-#define CDL_FP_SQRT  {0xffffeaabu, 0xee7fbfffu, 0xac54ffffu, 0x07aaffffu, 0x3dac3d89u, 0xd9cc34a8u, 0x3ce144afu, 0xd91dd2e1u, 0x90d2eb35u, 0x92c6e9edu, 0x8e5ff9a6u, 0x0680447au}
+// public constants, little-endian 32-bit words
 // (p-1)/2
 #define CDL_FP_HALF  {0xffffd555u, 0xdcff7fffu, 0x58a9ffffu, 0x0f55ffffu, 0x7b587b12u, 0xb3986950u, 0x79c2895fu, 0xb23ba5c2u, 0x21a5d66bu, 0x258dd3dbu, 0x1cbff34du, 0x0d0088f5u}
 // Montgomery form of curve constant b = 4 and of beta (cube root of unity with
@@ -66,12 +64,10 @@ using Fr = FrM::El;  // 32 bytes == gnark fr.Element
 #define CDL_FP_B     {0x000cfff3u, 0xaa270000u, 0xfc34000au, 0x53cc0032u, 0x6b0a807fu, 0x478fe97au, 0xe6ba24d7u, 0xb1d37ebeu, 0xbf78ab2fu, 0x8ec9733bu, 0x3d83de7eu, 0x09d64551u}
 #define CDL_FP_BETA  {0x8671f071u, 0xcd03c9e4u, 0x1fcda5d2u, 0x5dab2246u, 0xd3851b95u, 0x587042afu, 0x01bacb9eu, 0x8eb60ebeu, 0x83d050d2u, 0x03f97d6eu, 0x54638741u, 0x18f02065u}
 
-static const uint32_t FP_SQRT_H[12] = CDL_FP_SQRT;
 static const uint32_t FP_HALF_H[12] = CDL_FP_HALF;
 static const uint32_t FP_B_H[12] = CDL_FP_B;
 static const uint32_t FP_BETA_H[12] = CDL_FP_BETA;
 #if defined(__CUDACC__)
-static __device__ __constant__ uint32_t FP_SQRT_D[12] = CDL_FP_SQRT;
 static __device__ __constant__ uint32_t FP_HALF_D[12] = CDL_FP_HALF;
 static __device__ __constant__ uint32_t FP_B_D[12] = CDL_FP_B;
 static __device__ __constant__ uint32_t FP_BETA_D[12] = CDL_FP_BETA;
@@ -366,10 +362,18 @@ CDL_FN void fp_inv(Fp& r, const Fp& x) {
   FpM::mul(r, raw, r3);
 }
 
+// r = r^(2^n): a loop, so that a squaring run costs one squaring's code (inlined or the shared body)
+CDL_FN void fp_sqr_n(Fp& r, int n) {
+#pragma unroll 1
+  for (int i = 0; i < n; i++) FpM::sqr(r, r);
+}
+
+#include "fp_sqrt_chain.cuh"  // fp_pow_sqrt_exp(r, a): r = a^((p+1)/4) by a fixed addition chain
+
 // candidate square root a^((p+1)/4) (p = 3 mod 4); returns whether it squares to a
 CDL_FN bool fp_sqrt(Fp& r, const Fp& a) {
   Fp s, t;
-  FpM::pow_words<12>(s, a, CDL_SEL(FP_SQRT_D, FP_SQRT_H));
+  fp_pow_sqrt_exp(s, a);
   FpM::sqr(t, s);
   r = s;
   return FpM::eq(t, a);

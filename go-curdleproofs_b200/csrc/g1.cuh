@@ -447,36 +447,51 @@ CDL_FN void jac_scalar_mul_glv(G1Jac& r, const G1Affine& p, const uint32_t* k) {
   FpM::mul(r.z, r.z, zc);  // back from the isomorphic curve (infinity stays Z = 0)
 }
 
-// r = e * p for a public 64-bit e (MSB-first double-and-add on a Jacobian base)
-CDL_FN void jac_mul_u64(G1Jac& r, const G1Jac& p, uint64_t e) {
-  jac_set_inf(r);
-  bool started = false;
+CDL_FN void jac_dbl_n(G1Jac& r, int n) {
 #pragma unroll 1
-  for (int i = 63; i >= 0; i--) {
-    if (started) jac_dbl(r, r);
-    if ((e >> i) & 1) {
-      if (started) jac_add(r, r, p); else { r = p; started = true; }
-    }
-  }
+  for (int i = 0; i < n; i++) jac_dbl(r, r);
 }
 
-// Subgroup membership by the endomorphism: P is in G1 iff P + [z^2] phi(P) = 0
-// (z^2 * lambda + 1 = r).  This is gnark-crypto's own G1 IsInSubGroup test
-// (126 doublings + 11 additions instead of a 255-bit multiplication by r).
+// Subgroup membership by the endomorphism: P is in G1 iff P + [z^2] phi(P) = 0, i.e. [z^2] phi(P) = -P
+// (z^2 * lambda + 1 = r).  This is gnark-crypto's own G1 IsInSubGroup test (126 doublings + 10 additions
+// instead of a 255-bit multiplication by r).  z^2 phi(P) is computed as |z| (|z| phi(P)).  |z| =
+// 0xd201000000010000 has bits 63, 62, 60, 57, 48 and 16 set: from the top bit, the doubling runs 1, 2, 3, 9, 32
+// each end in an addition of the base, then 16 doublings follow.  The first base, phi(P) = (beta x, y), is
+// affine, so its additions are mixed; the second, |z| phi(P), stays Jacobian (normalising it would cost an
+// inversion).  Every addition keeps the complete exceptional-case handling: P need not have prime order here.
 CDL_FN bool g1_in_subgroup_endo(const G1Affine& p) {
   if (aff_is_inf(p)) return true;
-  const uint64_t kZ = 0xd201000000010000ull;  // |z|
-  G1Jac q, t;
+  constexpr uint32_t kRuns = 1u | 2u << 6 | 3u << 12 | 9u << 18 | 32u << 24;  // 6 bits per run
+  G1Affine q;
   Fp beta;
   fp_set_beta(beta);
   FpM::mul(q.x, p.x, beta);
   q.y = p.y;
-  FpM::set_one(q.z);
-  jac_mul_u64(t, q, kZ);
-  q = t;
-  jac_mul_u64(t, q, kZ);
-  jac_add_mixed(t, t, p);
-  return jac_is_inf(t);
+  G1Jac t, u;
+  jac_from_affine(t, q);
+#pragma unroll 1
+  for (int s = 0; s < 30; s += 6) {
+    jac_dbl_n(t, (kRuns >> s) & 63u);
+    jac_add_mixed(t, t, q);
+  }
+  jac_dbl_n(t, 16);
+  u = t;
+#pragma unroll 1
+  for (int s = 0; s < 30; s += 6) {
+    jac_dbl_n(t, (kRuns >> s) & 63u);
+    jac_add(t, t, u);
+  }
+  jac_dbl_n(t, 16);
+  // t == -P without normalising t: X = x Z^2 and Y = -y Z^3.  t = infinity is never -P (P is finite).
+  if (jac_is_inf(t)) return false;
+  Fp zz, w;
+  FpM::sqr(zz, t.z);
+  FpM::mul(w, p.x, zz);
+  if (!FpM::eq(w, t.x)) return false;
+  FpM::mul(zz, zz, t.z);
+  FpM::mul(w, p.y, zz);
+  FpM::add(w, w, t.y);
+  return FpM::is_zero(w);
 }
 
 }  // namespace cdl

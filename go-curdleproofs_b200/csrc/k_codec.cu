@@ -1,5 +1,6 @@
 // Batched point (de)compression kernels — replaces G1Affine.Bytes()/SetBytes()
 // (whisk/types.go:79-95, transcript/transcript.go:35, curdleproof.go:320-387).
+#define CDL_FP_MUL_CALL 1  // one shared product body, as in k_elem.cu: inlined, decompression is ~84 k instructions
 #include "codec.cuh"
 #include "launch.h"
 
@@ -12,8 +13,12 @@ __global__ void k_compress(const G1Affine* __restrict__ in, uint8_t* __restrict_
   g1_compress_dev(out + 48 * (size_t)i, p);
 }
 
-__global__ void k_decompress(const uint8_t* __restrict__ in, G1Affine* __restrict__ out,
-                             uint8_t* __restrict__ status, int n) {
+// Decompression: 64 threads per block, six blocks (12 warps) per SM.  ptxas then fits the kernel in 168 registers with
+// 312 bytes of stack (540 B of spill stores); without the bound it needs 252
+// registers and no stack, but only 8 warps fit per SM, and that measured slower on a B200 at 1 000 W
+// from 2^17 points on (4 % at 2^19 .. 2^22; 2 % faster at 2^16; profiles/r11_decompress_chain.txt).
+__global__ void __launch_bounds__(64, 6) k_decompress(const uint8_t* __restrict__ in,
+                                                     G1Affine* __restrict__ out, uint8_t* __restrict__ status, int n) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   G1Affine p;
@@ -33,7 +38,7 @@ __global__ void k_compress_idx(const G1Affine* __restrict__ pool, const uint32_t
   g1_compress_dev(out + 48 * (size_t)i, p);
 }
 
-__global__ void k_decompress_idx(const uint8_t* __restrict__ in, G1Affine* __restrict__ pool,
+__global__ void __launch_bounds__(64, 6) k_decompress_idx(const uint8_t* __restrict__ in, G1Affine* __restrict__ pool,
                                  const uint32_t* __restrict__ dst, uint8_t* __restrict__ status, int n) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;

@@ -389,25 +389,6 @@ struct Mont {
     for (int i = 0; i < N; i++) r2.v[i] = F::r2(i);
     mul(r, a, r2);
   }
-
-  // r = a^e, e given as NE little-endian 32-bit words (public exponent).
-  // 4-bit fixed window; a == 0 gives 0 for e != 0.
-  template <int NE>
-  static CDL_HD void pow_words(El& r, const El& a, const uint32_t* e) {
-    El tab[16];
-    set_one(tab[0]);
-    tab[1] = a;
-#pragma unroll 1
-    for (int i = 2; i < 16; i++) mul(tab[i], tab[i - 1], a);
-    set_one(r);
-#pragma unroll 1
-    for (int w = NE * 8 - 1; w >= 0; w--) {
-#pragma unroll 1
-      for (int j = 0; j < 4; j++) sqr(r, r);
-      uint32_t d = (e[w >> 3] >> ((w & 7) * 4)) & 15;
-      mul(r, r, tab[d]);  // public exponent: data-independent index (local memory on device)
-    }
-  }
 };
 
 }  // namespace cdl
