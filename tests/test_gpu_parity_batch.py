@@ -140,12 +140,14 @@ def test_whisk_n128_batch64_five_mutation_kinds_match_oracle(ctx, pkg):
 
 
 def test_fixed_base_tables_give_the_same_bytes_and_verdicts(ctx, pkg):
-    """CRS fixed-base tables (cdl_set_fixed_base_min_batch; csrc/fixed_base.cuh) forced on for every call —
-    table look-ups for the commitments, B_c / B_a, the first round of both folding arguments, Gs' and the
-    verifier's merged CRS terms, and with them the lazy schedule of Engine::prove (second-round MSMs on pairs of
-    CRS points, the twice-folded G, G', Gm built straight from the CRS) — against the oracle's proofs and verdicts with all five mutation kinds, at
+    """CRS fixed-base tables (cdl_set_fixed_base_min_batch; csrc/fixed_base.cuh) forced on for every call, with
+    them the lazy schedule of Engine::prove (second-round MSMs on pairs of CRS points, the twice-folded G, G', Gm
+    built straight from the CRS), against the oracle's proofs and verdicts with all five mutation kinds, at
     n = 128 and (small, so that short windows, tiny tasks and the Gt / Gu slots of the first fold are hit) n = 16;
-    then the same batch with the tables off: identical bytes."""
+    then the same batch with the tables off: identical bytes.  These batches of at most 32 instances per lane
+    read the tables in the MSMs only (k_msm_fixed, the commitments, B_c / B_a and the verifier's merged CRS
+    terms): their elementwise stages stay within kQuadMaxOps ops, and the quad kernel that runs them has no
+    tables.  The folds and Gs' on the tables are checked in test_gpu_crossovers.py."""
     try:
         ctx.set_fixed_base_min_batch(1)
         run_batch(ctx, pkg, 124, 64, 4576, 4, 2)

@@ -58,7 +58,7 @@ def test_fold(ctx, pts):
     assert want[-2] is None
 
 
-@pytest.mark.parametrize("n", [1, 2, 7, 8, 9, 64, 128, 300, 628])
+@pytest.mark.parametrize("n", [1, 2, 7, 8, 9, 64, 128, 300, 628, 1024])
 def test_msm_sizes(ctx, n):
     r = Rand(1000 + n)
     base = r.get_g1_affines(min(n, 48))
@@ -211,9 +211,10 @@ def test_public_known_answers(ctx):
 
 
 def test_msm_batch_multi_chunk_tasks(ctx, pts):
-    """Throughput path with tasks longer than one bucket-warp chunk (128 terms): the chunk partials
-    are summed per (task, window) before the Horner combine; also a single long MSM (> 384 terms,
-    chunked chain with 32-term chunks) next to short ones."""
+    """Throughput path with tasks longer than one bucket-warp chunk: both launches hold fewer than
+    2 * sm_count * kMsmChunk terms, so msm_tp_pick_chunk cuts them into 32-term chunks, and the chunk
+    partials are summed per (task, window) before the Horner combine; also a single long MSM (> 384
+    terms) next to short ones.  128-term chunks are checked in test_gpu_crossovers.py."""
     import random
     random.seed(12)
     r = Rand(79)
