@@ -115,6 +115,17 @@ int32_t crs_finish(cdl_ctx* c, Engine* E, const Layout& L, cdl_crs** out) {
   return CDL_OK;
 }
 
+// sum Gs to pool[gs_out] and sum Hs to pool[hs_out] from the image at the start of the pool   (crs.go:41-48);
+// st.out48 receives their encodings
+int32_t crs_sums(Engine* E, const Layout& L, uint32_t gs_out, uint32_t hs_out, cdlh::MsmStage& st) {
+  st.idx.resize(L.ell + 4);
+  st.sc.assign(L.ell + 4, cdlh::FR_ONE);
+  for (uint32_t i = 0; i < L.ell + 4; i++) st.idx[i] = L.Gs + i;  // Gs and Hs are contiguous in the image
+  st.tasks.push_back(cdl::MsmTask{0, L.ell, gs_out, 0});
+  st.tasks.push_back(cdl::MsmTask{L.ell, 4, hs_out, 0});
+  return E->run_msm(st);
+}
+
 struct Prep {
   Engine* E;
   Layout L;
@@ -372,14 +383,8 @@ int32_t cdl_crs_generate(cdl_ctx* c, size_t ell, cdl_rand* r, cdl_crs** out) {
   if ((rc = put_generator(E, gen))) return rc;
   // draw order: Gs (ell), Hs (4), H, Gt, Gu   (crs.go:21-40); these are contiguous in the image
   if ((rc = rand_points_to_pool(E, r, gen, L.Gs, ell + 7))) return rc;
-  // Gsum = sum Gs, Hsum = sum Hs   (crs.go:41-48)
   cdlh::MsmStage st;
-  st.idx.resize(ell + 4);
-  st.sc.assign(ell + 4, cdlh::FR_ONE);
-  for (uint32_t i = 0; i < ell + 4; i++) st.idx[i] = i;
-  st.tasks.push_back(cdl::MsmTask{0, (uint32_t)ell, L.Gsum, 0});
-  st.tasks.push_back(cdl::MsmTask{(uint32_t)ell, 4, L.Hsum, 0});
-  if ((rc = E->run_msm(st))) return rc;
+  if ((rc = crs_sums(E, L, L.Gsum, L.Hsum, st))) return rc;
   return crs_finish(c, E, L, out);
 }
 
@@ -390,7 +395,17 @@ int32_t cdl_crs_from_points(cdl_ctx* c, size_t ell, const cdl_g1_affine* points,
   Engine* E = engine_of(c);
   Layout L((uint32_t)ell);
   int32_t rc;
-  if ((rc = E->ensure_pool(L.crs_size + 1)) || (rc = E->upload_points(0, points, ell + 9))) return rc;
+  if ((rc = E->ensure_pool(L.crs_size + 2)) || (rc = E->upload_points(0, points, ell + 9))) return rc;
+  // Every cdl_crs has Gsum = sum Gs and Hsum = sum Hs: the prover and the verifier use the two sums in place
+  // of the vectors they stand for (Engine::prove's B and D).  The caller's sums are checked against sums of the
+  // caller's points (scratch slots after the image), compared as encodings.
+  cdlh::MsmStage st;
+  std::vector<uint8_t> given;
+  if ((rc = crs_sums(E, L, L.crs_size, L.crs_size + 1, st)) || (rc = E->compress({L.Gsum, L.Hsum}, given))) return rc;
+  if (memcmp(st.out48.data(), given.data(), 48) != 0)
+    return c->fail(CDL_ERR_INVALID_ARG, "crs: Gsum is not the sum of the %zu Gs points", ell);
+  if (memcmp(st.out48.data() + 48, given.data() + 48, 48) != 0)
+    return c->fail(CDL_ERR_INVALID_ARG, "crs: Hsum is not the sum of the 4 Hs points");
   return crs_finish(c, E, L, out);
 }
 

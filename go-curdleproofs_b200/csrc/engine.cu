@@ -613,7 +613,8 @@ int32_t Engine::prove(const Layout& L, uint32_t B, const cdl_crs* crs, const std
       s.rs_b[i] = fr_add(fr_mul(s.alpha, rs_m_in[b][i]), ra);
     }
   });
-  // B = A + alpha*M + beta*sum(Gs)   (:62-73; sum(Gs) is crs.Gsum)
+  // B = A + alpha*M + beta*sum(Gs)   (:62-73; sum(Gs) is crs.Gsum: every cdl_crs has Gsum = sum Gs and
+  // Hsum = sum Hs, which cdl_crs_from_points checks)
   {
     StageBuilder sb(st, B, 3, 1);
     for (uint32_t b = 0; b < B; b++) {
@@ -716,7 +717,8 @@ int32_t Engine::prove(const Layout& L, uint32_t B, const cdl_crs* crs, const std
   // D, the self-check on D, B_c, B_d  (:105-177, innerproductargument.go:59-72).
   // D = B - <beta^i, Gs'> + <alpha*beta^(ell+1), Hs'> (:132-138) with Gs'[i] = beta^-(i+1) Gs[i] and
   // Hs'[j] = beta^-(ell+1) Hs[j] is B - beta^-1 * Gsum + alpha * Hsum term by term - the very formula
-  // the verifier uses (:243-246) - so it is computed as that three-term MSM (same point, same bytes).
+  // the verifier uses (:243-246) - so it is computed as that three-term MSM (same point, same bytes).  Term by
+  // term only because every cdl_crs has Gsum = sum Gs and Hsum = sum Hs (checked by cdl_crs_from_points).
   // The reference's self-check msm(Gs||Hs, cs||r_cs) == C (:164-170) recomputes C = <cs, Gs> + <r_cs, Hs>
   // (:66-73) from the very same operands: it cannot fail, so it is not launched.  msm(G', d) == D
   // (:171-177) depends on the caller's M and rs_m and is the reference's error path for a witness that

@@ -214,7 +214,11 @@ int32_t cdl_rand_generate_permutation(cdl_rand* r, size_t n, uint32_t* out);
 
 /* curdleproof.GenerateCRS (crs.go:20-59): draws ell Gs, 4 Hs, H, Gt, Gu and forms Gsum, Hsum. */
 int32_t cdl_crs_generate(cdl_ctx* ctx, size_t ell, cdl_rand* r, cdl_crs** out);
-/* Wrap an existing Go-side CRS: points[] = Gs[ell] | Hs[4] | H | Gt | Gu | Gsum | Hsum, all affine. */
+/* Wrap an existing Go-side CRS: points[] = Gs[ell] | Hs[4] | H | Gt | Gu | Gsum | Hsum, all affine.
+ * Gsum must be the sum of the Gs and Hsum the sum of the Hs (one MSM of ell + 4 terms checks both):
+ * the prover and verifier use the sums in place of the vectors, so a CRS whose sums disagree would give
+ * proofs that differ from the reference's and that its verifier rejects.  CDL_ERR_INVALID_ARG otherwise,
+ * with cdl_last_error naming the wrong sum.  The points are not checked to be on the curve or in G1. */
 int32_t cdl_crs_from_points(cdl_ctx* ctx, size_t ell, const cdl_g1_affine* points, cdl_crs** out);
 /* Same order as cdl_crs_from_points, ell + 9 points. */
 int32_t cdl_crs_export(cdl_ctx* ctx, const cdl_crs* crs, cdl_g1_affine* points);

@@ -1,6 +1,7 @@
 """The launch-size crossovers of the kernel launchers, read from the CUDA sources, and a restatement of the MSM
-window-combine schedules on discrete logarithms, so that a test can show that a crafted MSM task makes a combine
-step add two equal or two opposite points.  Shared by test_crossovers_cpu.py (no GPU) and test_gpu_crossovers.py.
+window-combine schedules and of the Pippenger bucket fill on discrete logarithms, so that a test can show that a
+crafted MSM task makes a combine step add two equal or two opposite points, or fills a bucket with a known multiset.
+Shared by test_crossovers_cpu.py (no GPU), test_gpu_crossovers.py and test_gpu_msm_repeated_bases.py.
 
 Every point of a crafted task is a multiple a * G of the generator, so a point is its discrete log a mod r (0 is
 the point at infinity) and phi(P) = lambda * P is lambda * a."""
@@ -27,6 +28,8 @@ SOURCES = {
     "kBigMsmThreshold": ("launch.h", r"constexpr size_t kBigMsmThreshold\s*=\s*(\d+);"),
     "kBigQuadMaxOutputs": ("k_msm_big.cu", r"constexpr int kBigQuadMaxOutputs\s*=\s*(\d+);"),
     "kMsmC": ("k_msm.cu", r"constexpr int kMsmC\s*=\s*(\d+);"),
+    "kBigLargeBucket": ("k_msm_big.cu", r"constexpr uint32_t kBigLargeBucket\s*=\s*(\d+);"),
+    "kBigMaxBaRounds": ("launch.h", r"constexpr int kBigMaxBaRounds\s*=\s*(\d+);"),
 }
 
 
@@ -90,6 +93,13 @@ def big_reduce1_outputs(n):
     c = big_pick_c(n)
     W, M = (128 + c - 1) // c, 1 << (c - 1)
     return W * (M // min(M, 8))
+
+
+def big_large(n, c, rounds):
+    """restatement of BigMsmDims::large (big_msm_dims): a bucket of more entries than this after the batch-affine
+    rounds is summed by k_big_slice / k_big_large_finish instead of one k_big_accum thread"""
+    mean = 2 * n // (1 << (c - 1)) + 1
+    return min(max(8 * ((mean >> rounds) + 1), 64), const("kBigLargeBucket"))
 
 
 def pick_chunk(nterm, sm_count):
@@ -222,3 +232,41 @@ def big_collision_task(n, kind):
     e = 1 << big_pick_c(n)
     task = [(1, e), (e if kind == "equal" else R - e, 1)]
     return task + [(2 + i, 0) for i in range(n - 2)]
+
+
+# ------------------------------------------------------------------------------------------------- bucket contents
+def big_buckets(hc, task, c):
+    """restatement of k_big_digits' bucket fill for a one-device Pippenger MSM: {(window, |digit|): sorted discrete
+    logs of the bucket's entries}.  Entry = the half's base (P or phi(P)), negated when the digit's sign and the
+    half's GLV sign differ; the order the scatter leaves inside a bucket is not modelled (it varies)."""
+    out = {}
+    for k, a in halves(hc, task):
+        for w, d in enumerate(signed_digits(k, c)):
+            if d:
+                out.setdefault((w, abs(d)), []).append(a if d > 0 else (R - a) % R)
+    return {key: sorted(v) for key, v in out.items()}
+
+
+KNOWN_WINDOWS = 3  # windows 0 .. 2 carry the digit of a known-bucket scalar, the others are zero
+
+
+def known_bucket_task(c, rounds):
+    """Terms (discrete log, scalar) on the bases P = G (log 1) and -P whose Pippenger buckets hold known multisets
+    at window width c: a scalar d * (1 + 2^c + 2^(2c)) with d in [1, 2^(c-1)] is far below lambda / 2, so the GLV
+    split leaves it whole (k2 = 0, no negation), and its c-bit digits are d, d, d and zeros: no carry, so it puts
+    exactly one +P into bucket (w, d) of windows 0 .. 2.  For every count m in {1, 2, 3, 2^R - 1, 2^R, 2^R + 1}
+    (R = rounds) m terms share a digit d_m (d = 2^(c-1), the largest digit, first), and one more digit holds one
+    term on P and one on -P.  Returns (task, {bucket: intended sorted multiset}).  Whatever order the scatter
+    leaves, the first batch-affine round then adds (P, P), (P, inf), (inf, inf) and (P, -P) pairs, and round j
+    adds (2^(j-1) P, 2^(j-1) P) in the buckets of 2^R entries."""
+    M = 1 << (c - 1)
+    spread = sum(1 << (c * w) for w in range(KNOWN_WINDOWS))
+    counts = sorted({1, 2, 3, (1 << rounds) - 1, 1 << rounds, (1 << rounds) + 1} - {0})
+    task, want, d = [], {}, M
+    for m in counts:
+        task += [(1, d * spread)] * m
+        want.update({(w, d): [1] * m for w in range(KNOWN_WINDOWS)})
+        d -= 1
+    task += [(1, d * spread), (R - 1, d * spread)]
+    want.update({(w, d): [1, R - 1] for w in range(KNOWN_WINDOWS)})
+    return task, want

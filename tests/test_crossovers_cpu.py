@@ -1,6 +1,7 @@
 """No GPU: the thresholds test_gpu_crossovers.py derives its sizes from are still found in the CUDA sources, and
 the MSM tasks it crafts to hit the exceptional cases of the window-combine additions really do so under a
-restatement of the kernels' digit schedules (digits from the product's own glv_decompose, built for the host)."""
+restatement of the kernels' digit schedules (digits from the product's own glv_decompose, built for the host), and
+the tasks test_gpu_msm_repeated_bases crafts fill the Pippenger buckets with the multisets it intends."""
 import ctypes
 import os
 import subprocess
@@ -93,3 +94,35 @@ def test_a_changed_task_no_longer_collides(hc):
     task = X.big_collision_task(n, "equal")
     task[0] = (1, task[0][1] * 2)
     assert X.big_schedule(hc, task, X.big_pick_c(n))[1] == []
+
+
+def test_slice_path_sizes():
+    """test_gpu_msm_repeated_bases' slice case: 8192 copies of one base with one scalar put 8192 entries into one
+    bucket per window and GLV half, above BigMsmDims::large at 0 and 3 batch-affine rounds"""
+    n = 8192
+    c = X.big_pick_c(n)
+    for rounds in (0, 3):
+        assert n >> rounds > X.big_large(n, c, rounds), rounds
+    assert X.big_large(1 << 22, 16, 0) <= X.const("kBigLargeBucket")
+
+
+@pytest.mark.parametrize("c", [8, 11, 16])
+def test_known_buckets_hold_their_multisets(hc, c):
+    """For every forced round count the crafted task fills each targeted bucket with exactly the intended multiset
+    (counts 1, 2, 3, 2^R - 1, 2^R, 2^R + 1 of +P, and {P, -P}) and no other bucket, its scalars take no GLV split or
+    negation, and a task with one scalar changed no longer does."""
+    assert X.const("kBigMaxBaRounds") == 8
+    for rounds in range(X.const("kBigMaxBaRounds") + 1):
+        task, want = X.known_bucket_task(c, rounds)
+        scalars = sorted({s for _, s in task})
+        assert all(k2 == 0 and not n1 and not n2 for _, k2, n1, n2 in X.glv_split(hc, scalars))
+        got = X.big_buckets(hc, task, c)
+        for key, v in want.items():
+            assert got.get(key) == v, (c, rounds, key, got.get(key), v)
+        assert set(got) == set(want)  # no bucket outside the targeted ones
+        assert {len(v) for v in want.values()} == {1, 2, 3, (1 << rounds) - 1, 1 << rounds, (1 << rounds) + 1} - {0}
+        for i in (0, len(task) - 1):
+            changed = list(task)
+            changed[i] = (changed[i][0], changed[i][1] + 1)
+            got = X.big_buckets(hc, changed, c)
+            assert any(got.get(key) != v for key, v in want.items()), (c, rounds, i)
